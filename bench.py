@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MPPI rollout state-steps/s (samples x horizon per MPPI iteration) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one MPPI iteration of the hot path (propagate + get_cost + shift_policy_means; sampling the
 policy noise is excluded, SURVEY.md 8(d)) over one batch of synthetic input.  Default workload =
@@ -15,6 +15,12 @@ timed, max over ranks; `e2e` = the same through the C ABI host-buffer entry poin
 `cpu_baseline` = the reference's own classes (oracle/_ref, staged by oracle/make_ref.sh; torch CPU, all host
 threads) on a bounded sample -- the oracle port only when that tree is absent.
 `--impl reference` times that CPU arm alone with the same --steps / --warmup.
+`--dump-outputs DIR` writes what the last timed step returned (trajectories, distances, kernel values, dot products,
+activations, qdot, cost, the updated policy means, n_updated) as DIR/<name>.npy, at most 64 MB (a fixed, seeded
+subset of samples beyond that); the inputs are seeded, so two builds run with the same arguments compare array for
+array.  On N > 1 GPUs only rank 0's shard of the samples is written (the policy means are the same on every rank).
+`--steps K` is the number of timed iterations of `value` and of `e2e`; on the latency workload `integrator` a step is
+one control tick (30 untimed warm-up ticks; a few hundred timed ticks give a stable rate).
 On N > 1 GPUs the run first proves the NCCL path (`multi_gpu_check`: ranks bit-identical, sharded == single-rank
 update; exit 3 otherwise) and adds `c5`, the BASELINE configs[4] shard shape (125 000 samples x 50 steps per GPU).
 """
@@ -308,13 +314,42 @@ def policy_vector(mppi):
     return torch.cat((P.mu_c.flatten(), P.sigma_c.flatten(), P.alpha_c.flatten())).float()
 
 
+DUMP_BYTES = 63_000_000     # array data of one --dump-outputs directory; the .npy headers stay well inside 64 MB
+
+
+def dump_outputs(out_dir, per_sample, other, seed=0):
+    """Writes every array as <out_dir>/<name>.npy: float32 stays float32, anything else becomes float64.
+    `per_sample` arrays have the sample axis first; when all arrays together would pass DUMP_BYTES, the same fixed,
+    seeded subset of samples is kept of each of them and its indices are written as sample_index.npy."""
+    import numpy as np
+
+    def host(t):
+        t = torch.as_tensor(t).detach().cpu()
+        return (t if t.dtype == torch.float32 else t.double()).numpy()
+
+    per_sample = {k: host(v) for k, v in per_sample.items()}
+    other = {k: host(v) for k, v in other.items()}
+    n = next(iter(per_sample.values())).shape[0]
+    row_bytes = sum(a.nbytes for a in per_sample.values()) // n
+    budget = DUMP_BYTES - sum(a.nbytes for a in other.values())
+    if row_bytes * n > budget:
+        keep = np.sort(np.random.default_rng(seed).choice(n, budget // (row_bytes + 8), replace=False))
+        per_sample = {k: a[keep] for k, a in per_sample.items()}
+        other["sample_index"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in {**per_sample, **other}.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def measure_control_tick(dev_index, ticks=400, n_obs=28):
     """The integrator process's loop (frankaIntegrator.py:101-121): ONE sample, TWO steps per control tick, CPU tensors
     in and out as that script uses them -- update_obstacles, sample_policy, propagate, q += qdot * dt, clamp.  Wall
     clock per tick, everything included (this is a latency figure, the reference logs ~500 Hz for it).  The drop-in
-    replays one CUDA graph per propagate() at this size (MPPI._propagate_tick)."""
+    replays one CUDA graph per propagate() at this size (MPPI._propagate_tick).  Returns the timing and what the last
+    tick computed."""
     from optimalmodulationds_b200 import MPPI, LinDS
     from optimalmodulationds_b200.sdf.robot_sdf import RobotSdfCollisionNet
+    torch.manual_seed(0)                                   # sample_policy draws from the global generator
     p = problem("franka_shelf_294")
     obs = p["obs"][:n_obs].clone()
     W, b, _ = load_net_arrays("franka")
@@ -333,21 +368,25 @@ def measure_control_tick(dev_index, ticks=400, n_obs=28):
     def tick():
         m.update_obstacles(obs)
         P.sample_policy()
-        m.propagate()
+        out = m.propagate()
         m.q_cur = torch.clamp(m.q_cur + m.qdot[0, :] * 0.01, m.Cost.q_min, m.Cost.q_max)
+        return out
 
     for _ in range(30):
         tick()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     for _ in range(ticks):
-        tick()
+        out = tick()
     torch.cuda.synchronize()
     dt = (time.perf_counter() - t0) / ticks
+    traj, dist_all, kval, dots, acts = out
+    outputs = dict(all_traj=traj, closest_dist_all=dist_all, kernel_val_all=kval, dot_products=dots,
+                   kernel_activations=acts, qdot=m.qdot), dict(q_cur=m.q_cur)
     return dict(hz=1.0 / dt, ms_per_tick=dt * 1e3, ticks=ticks, graphed="_tick" in m.__dict__,
                 config=f"Franka net, {n_obs} spheres, N=1, H=2, K={p['K']}, 5 kernels, CPU caller tensors, "
                        "loop of frankaIntegrator.py:101-121 (update_obstacles, sample_policy, propagate, q += qdot dt)",
-                timing="wall clock per tick incl. host wrapper, H2D, launch, D2H")
+                timing="wall clock per tick incl. host wrapper, H2D, launch, D2H"), outputs
 
 
 def check_sharding(p, dev, args, rank, world, mppi_main):
@@ -406,7 +445,13 @@ def main():
     ap.add_argument("--per-step", action="store_true", help="disable the whole-horizon single-launch path")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c5", action="store_true", help="skip the configs[4]-shaped record of multi-GPU runs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (rank 0's samples)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -453,9 +498,11 @@ def main():
             return
         sampler = ClockSampler(local_rank)
         sampler.start()
-        tick = measure_control_tick(local_rank, ticks=max(200, 100 * args.steps))
+        tick, outputs = measure_control_tick(local_rank, ticks=args.steps)
         sampler.stop_flag = True
         sampler.join()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *outputs)
         line = dict(metric="mppi_rollout_state_steps_per_sec", value=2 * tick["hz"], unit="state-steps/s", n_gpus=1,
                     steps=tick["ticks"], warmup=30, ms_per_step=tick["ms_per_tick"], higher_is_better=True,
                     scaling="weak", vs_baseline=None, dtype="f32 (scoring: split-fp16 tcgen05, fp32-accurate)",
@@ -481,9 +528,10 @@ def main():
     flush = torch.empty(256 * 1024 * 1024 // 4, device=dev)
 
     def step(m=mppi):
-        m.propagate()
-        m.get_cost()
-        m.shift_policy_means()
+        out = m.propagate()
+        cost = m.get_cost()
+        _, n_updated = m.shift_policy_means()
+        return out, cost, n_updated
 
     def sync_all():
         torch.cuda.synchronize(dev)
@@ -495,10 +543,11 @@ def main():
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(n_steps)]
         kt_ms, kt_n, name = 0.0, 0, "exact_mlp_kernel"
         sync_all()
+        last = None
         for a, bq in evs:
             flush.fill_(1.0)
             a.record()
-            step(m)
+            last = step(m)
             bq.record()
             bq.synchronize()
             if with_kernel_timing:
@@ -510,7 +559,7 @@ def main():
         ms = torch.tensor([sum(a.elapsed_time(bq) for a, bq in evs) / n_steps], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms), kt_ms, kt_n, name
+        return float(ms), kt_ms, kt_n, name, last
 
     for _ in range(warm):
         step()
@@ -519,10 +568,17 @@ def main():
     sampler = ClockSampler(local_rank)
     sampler.start()
     launches0 = mppi.launch_count()
-    ms_per_step, kt_ms, kt_n, kern_name = timed_steps(mppi, args.steps, True)
+    ms_per_step, kt_ms, kt_n, kern_name, last = timed_steps(mppi, args.steps, True)
     launches = mppi.launch_count() - launches0
     sampler.stop_flag = True
     sampler.join()
+    if args.dump_outputs and rank == 0:
+        (traj, dist_all, kval, dots, acts), cost, n_updated = last
+        P = mppi.Policy
+        dump_outputs(args.dump_outputs,
+                     dict(all_traj=traj, closest_dist_all=dist_all, kernel_val_all=kval, dot_products=dots,
+                          kernel_activations=acts, qdot=mppi.qdot, cost=cost),
+                     dict(mu_c=P.mu_c, sigma_c=P.sigma_c, alpha_c=P.alpha_c, n_updated=n_updated))
     value = world * N * H / (ms_per_step * 1e-3)
     stats = mppi.pass1_stats()
     xstats = mppi.exactness_stats()
@@ -552,12 +608,11 @@ def main():
     for _ in range(2):
         h2d, d2h = mppi.iteration_host(host)
     sync_all()
-    e_steps = max(2, min(args.steps, 5))
     t0 = time.perf_counter()
-    for _ in range(e_steps):
+    for _ in range(args.steps):
         h2d, d2h = mppi.iteration_host(host)
     torch.cuda.synchronize(dev)
-    e_ms = torch.tensor([(time.perf_counter() - t0) * 1e3 / e_steps], device=dev)
+    e_ms = torch.tensor([(time.perf_counter() - t0) * 1e3 / args.steps], device=dev)
     if world > 1:
         dist.all_reduce(e_ms, op=dist.ReduceOp.MAX)
         hp = torch.cat((host["mu_c"].flatten(), host["sigma_c"], host["alpha_c"].flatten())).to(dev)
@@ -578,7 +633,7 @@ def main():
         torch.cuda.empty_cache()
         m5, _, _ = build_mppi(p, C5_SAMPLES_PER_GPU, H, dev, args, 500 + rank, world)
         step(m5)
-        ms5, _, _, _ = timed_steps(m5, 2, False)
+        ms5, _, _, _, _ = timed_steps(m5, 2, False)
         c5 = dict(samples_per_gpu=C5_SAMPLES_PER_GPU, samples_total=world * C5_SAMPLES_PER_GPU, horizon=H,
                   n_obstacles=M, ms_per_iteration=ms5, timed_iterations=2, warmup=1,
                   value=world * C5_SAMPLES_PER_GPU * H / (ms5 * 1e-3), unit="state-steps/s",
@@ -675,7 +730,7 @@ def main():
     if world == 1:
         del mppi
         torch.cuda.empty_cache()
-        line["control_tick"] = measure_control_tick(local_rank)
+        line["control_tick"] = measure_control_tick(local_rank)[0]
     if world == 1 and not args.no_cpu_baseline:
         r = cpu_reference_rate(p, target_seconds=15.0)
         line["cpu_baseline"] = dict(value=r["value"], unit="state-steps/s", cores=r["cores"], kind=r["kind"],

@@ -25,7 +25,8 @@ REF = os.path.join(ROOT, "oracle", "_ref")
 DS_MPPI = os.path.join(REF, "python_scripts", "ds_mppi")
 
 needs_ref = pytest.mark.skipif(not os.path.isdir(DS_MPPI),
-                               reason="oracle/_ref is not staged (run oracle/make_ref.sh in the build container)")
+                               reason="oracle/_ref is not staged (DSMPPI_REFERENCE_SRC=<checkout of the original "
+                                      "project> oracle/make_ref.sh)")
 
 # sitecustomize-free way to learn, from inside the unmodified script's process, which MPPI module it imported: a
 # PYTHONSTARTUP-like hook is not available for scripts, so the check runs as a separate probe with the same environment

@@ -1,5 +1,5 @@
-import cProfile, pstats, sys, time, torch
-sys.path.insert(0, "/root/repo")
+import cProfile, os, pstats, sys, time, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from tests.golden_util import load_npz
 from tests.mppi_factory import make_mppi
 for dev in ("cuda", "cpu"):

@@ -1,5 +1,5 @@
 import os, sys, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from tests.golden_util import load_npz
 from tests import mppi_factory as F
 for tag in ("planar7", "planar7_near", "planar2_near", "franka_shelf"):
