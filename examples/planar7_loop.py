@@ -5,7 +5,10 @@ names (`from MPPI import *`, `from LinDS import *`, `from sdf.robot_sdf import R
 optimalmodulationds_b200/dropin, CPU tensors go in and come out, attributes are poked after construction, and a
 second 1-sample x 1-step MPPI object moves the robot.  Headless (the drop-in `plots` module draws nothing).
 
-    python examples/planar7_loop.py [--iters 200] [--checkpoint path/to/7dof_sdf_256x5_mesh.pt]
+    python examples/planar7_loop.py [--iters 200] [--checkpoint path/to/7dof_sdf_256x5_mesh.pt] [--layers 128x3]
+
+--layers WxL builds a seeded random-init network of L hidden layers of width W instead of the shipped 256 x 4 weights
+(any 1 <= L <= 4, W <= 256 runs; a checkpoint of that shape can be loaded with --checkpoint as well).
 """
 import argparse
 import copy
@@ -24,12 +27,17 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--iters", type=int, default=200)
     ap.add_argument("--checkpoint", default=None)
+    ap.add_argument("--layers", default=None, help="WxL: L hidden layers of width W (default: the shipped 256x4)")
     args = ap.parse_args()
     params = {'device': 'cpu', 'dtype': torch.float32}                       # noqa: F405
     DOF, L = 7, 1
-    nn_model = RobotSdfCollisionNet(in_channels=DOF + 3, out_channels=DOF, layers=[256] * 4, skips=[])
+    width, depth = (int(x) for x in (args.layers or "256x4").split("x"))
+    torch.manual_seed(0)                                                     # noqa: F405
+    nn_model = RobotSdfCollisionNet(in_channels=DOF + 3, out_channels=DOF, layers=[width] * depth, skips=[])
     if args.checkpoint:
         nn_model.load_weights(args.checkpoint, params)
+    elif args.layers:
+        print(f"seeded random-init {width}x{depth} distance network")
     else:
         z = np.load(os.path.join(ROOT, "tests", "golden", "weights", "planar7.npz"))   # noqa: F405
         nn_model.load_arrays([z[f"W{i}"] for i in range(5)], [z[f"b{i}"] for i in range(5)])

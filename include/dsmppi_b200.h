@@ -31,18 +31,22 @@ extern "C" {
 #define DSMPPI_MAX_DOF 8
 #define DSMPPI_MAX_LINKS 16      /* network output channels O (<= 16) */
 #define DSMPPI_MAX_CLOSEST 8     /* n_closest_obs K (<= 8) */
-#define DSMPPI_HIDDEN 256        /* width of the shipped distance MLP */
+#define DSMPPI_HIDDEN 256        /* width of the shipped distance MLP, and the largest supported */
+#define DSMPPI_MAX_HIDDEN_LAYERS 4  /* hidden layers of the shipped distance MLP, and the most supported */
 
 typedef struct dsmppi_ctx dsmppi_ctx;
 
 /* Network weights as torch stores them: W[l] is (out, in) row-major (mlp_learn/sdf/network_macros_mod.py
- * 137-146 with skips=[]: 3(d+3) -> 256 -> 256 -> 256 -> 256 -> O, ReLU between).  HOST pointers. */
+ * 137-146 with skips=[]: 3(d+P) -> W -> ... -> W -> O with L hidden layers of one width W, ReLU between; the shipped
+ * networks are 256 x 4).  W_host[0..L-1] / b_host[0..L-1] are the hidden layers ((W, 3(d+P)), then (W, W)) and
+ * W_host[L] / b_host[L] the output layer (O, W); entries past L are ignored.  HOST pointers. */
 typedef struct {
   int32_t n_dof;                 /* d  */
   int32_t n_out;                 /* O  */
   int32_t n_point_dim;           /* P: obstacle coordinates fed to the network (in_channels = d + P); 3 for every
                                   * robot net, 2 for the planar "toy" net (standaloneToy2d.py:30); 0 means 3      */
-  int32_t reserved;
+  int16_t n_hidden;              /* L: hidden layers, 1..4; 0 means 4                                            */
+  int16_t hidden_width;          /* W: width of every hidden layer, 1..256; 0 means 256                          */
   const float* W_host[5];
   const float* b_host[5];
 } dsmppi_net;
@@ -172,7 +176,10 @@ void dsmppi_modulation_toy(dsmppi_modulation* out);       /* MPPI_toy.py constan
 
 /* MPPI.__init__ (MPPI.py:22-73): packs the network (fp32 both orientations + fp16/bf16 UMMA smem images),
  * the DH table (dh_params (d+1, 4) = [d, theta, a, alpha], HOST) and sizes the workspace for
- * `capacity` samples.  `device` is the CUDA ordinal. */
+ * `capacity` samples.  `device` is the CUDA ordinal.  A network narrower or shallower than 256 x 4 is embedded in
+ * that shape (zero rows / columns for the missing features, identity layers for the missing depth), which changes no
+ * result: the FFMA scoring kernels run the network's own width and depth, the tensor-core kernels the embedded one.
+ * A shape outside 1 <= L <= 4, 1 <= W <= 256 returns 2. */
 int dsmppi_ctx_create(dsmppi_ctx** out, const dsmppi_net* net, const float* dh_params_host,
                       int32_t capacity, int32_t device);
 int dsmppi_ctx_destroy(dsmppi_ctx* ctx);

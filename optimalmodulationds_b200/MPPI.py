@@ -54,16 +54,26 @@ def _stage_tags(names):
         yield
 
 
+_NET_FAMILY = ("the supported distance networks are 3(d+P) -> W -> ... -> W -> O MLPs without skips: 1 to 4 hidden "
+               "layers of one width W <= 256, O <= 16 outputs")
+
+
 def _network_arrays(nn_model):
-    """The five (out, in) weight matrices and biases of nn_model.model as contiguous fp32 CPU tensors."""
+    """The (out, in) weight matrices and biases of nn_model.model as contiguous fp32 CPU tensors: L hidden layers, then
+    the output layer.  Raises NotImplementedError for a network outside the family the library runs."""
+    if len(getattr(nn_model.model, 'skips', ()) or ()) > 0:
+        raise NotImplementedError(f"skip connections are not supported; {_NET_FAMILY}")
     lin = [m for m in nn_model.model.modules() if isinstance(m, torch.nn.Linear)]
-    if len(lin) != 5:
-        raise NotImplementedError(f"expected the 5-layer distance MLP (4 hidden + output), found {len(lin)} layers")
     W = [m.weight.detach().to('cpu', torch.float32).contiguous() for m in lin]
     b = [m.bias.detach().to('cpu', torch.float32).contiguous() for m in lin]
-    if W[0].shape != (256, 3 * nn_model.in_channels) or any(w.shape != (256, 256) for w in W[1:4]) \
-            or W[4].shape != (nn_model.out_channels, 256):
-        raise NotImplementedError("only the shipped 3(d+P)-256-256-256-256-O layout (skips=[]) is supported")
+    L = len(W) - 1
+    if not 1 <= L <= _capi.MAX_HIDDEN_LAYERS:
+        raise NotImplementedError(f"found {max(L, 0)} hidden layers; {_NET_FAMILY}")
+    width = W[0].shape[0]
+    shapes = [(width, 3 * nn_model.in_channels)] + [(width, width)] * (L - 1) + [(nn_model.out_channels, width)]
+    if [tuple(w.shape) for w in W] != shapes or not 1 <= width <= _capi.MAX_HIDDEN \
+            or not 1 <= nn_model.out_channels <= _capi.MAX_LINKS:
+        raise NotImplementedError(f"layer shapes {[tuple(w.shape) for w in W]}; {_NET_FAMILY}")
     return W, b
 
 
@@ -146,7 +156,8 @@ class MPPI:
                              "expected n_dof + 3 (or n_dof + 2 for the planar toy net)")
         net = _capi.Net()
         net.n_dof, net.n_out, net.n_point_dim = self.n_dof, self.nn_model.out_channels, self._point_dim
-        for i in range(5):
+        net.n_hidden, net.hidden_width = len(W) - 1, W[0].shape[0]
+        for i in range(len(W)):
             net.W_host[i] = W[i].data_ptr()
             net.b_host[i] = b[i].data_ptr()
         dh = self.dh_params.detach().to('cpu', torch.float32).contiguous()

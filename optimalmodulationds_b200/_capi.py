@@ -15,6 +15,8 @@ N_KERNEL_MAX = 50
 MAX_DOF = 8
 MAX_LINKS = 16
 MAX_CLOSEST = 8
+MAX_HIDDEN = 256          # widest hidden layer of the distance network
+MAX_HIDDEN_LAYERS = 4
 
 PASS1_EXACT_FP32, PASS1_TC_F16, PASS1_TC_BF16, PASS1_AUTO = 0, 1, 2, 3
 SCORE_FFMA, SCORE_TC_SPLIT, SCORE_AUTO = 0, 1, 2
@@ -29,7 +31,8 @@ COST_JOINT_LIMITS, COST_TERMINAL_FK, COST_ALL = 1, 2, 3
 
 
 class Net(C.Structure):
-    _fields_ = [("n_dof", C.c_int32), ("n_out", C.c_int32), ("n_point_dim", C.c_int32), ("reserved", C.c_int32),
+    _fields_ = [("n_dof", C.c_int32), ("n_out", C.c_int32), ("n_point_dim", C.c_int32),
+                ("n_hidden", C.c_int16), ("hidden_width", C.c_int16),
                 ("W_host", _fp * 5), ("b_host", _fp * 5)]
 
 

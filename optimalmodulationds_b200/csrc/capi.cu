@@ -111,12 +111,55 @@ int ensure_workspace(dsmppi_ctx* c, int n, int M) {
   return 0;
 }
 
-namespace { void tick_free(dsmppi_ctx* c); }
+namespace {
+
+// The caller's network (L hidden layers of width W) in the shipped 256 x 4 shape, the one storage format of every
+// weight image.  Missing features get zero weights and biases: their pre-activation is 0, ReLU keeps it 0, and they
+// add exact zeros downstream.  Missing layers L+1..4 are the identity on the first W features with zero bias: their
+// input is already >= 0, so relu(I h) = h exactly, and their ReLU mask equals layer L's, which leaves the VJP unchanged.
+struct Frame {
+  std::vector<float> W[5], b[5];
+  dsmppi_net net{};
+};
+
+Frame embed_net(const dsmppi_net* src, int nenc, int L, int W) {
+  Frame f;
+  const int O = src->n_out;
+  for (int l = 0; l < 4; ++l) {
+    const int in = l == 0 ? nenc : HID, in_src = l == 0 ? nenc : W;
+    f.W[l].assign((size_t)HID * in, 0.f);
+    f.b[l].assign(HID, 0.f);
+    for (int o = 0; o < W; ++o) {
+      if (l < L) {
+        for (int k = 0; k < in_src; ++k) f.W[l][(size_t)o * in + k] = src->W_host[l][(size_t)o * in_src + k];
+        f.b[l][o] = src->b_host[l][o];
+      } else {
+        f.W[l][(size_t)o * in + o] = 1.f;
+      }
+    }
+  }
+  f.W[4].assign((size_t)O * HID, 0.f);
+  for (int o = 0; o < O; ++o)
+    for (int k = 0; k < W; ++k) f.W[4][(size_t)o * HID + k] = src->W_host[L][(size_t)o * W + k];
+  f.b[4].assign(src->b_host[L], src->b_host[L] + O);
+  f.net = *src;
+  f.net.n_hidden = MAXL;
+  f.net.hidden_width = HID;
+  for (int l = 0; l < 5; ++l) {
+    f.net.W_host[l] = f.W[l].data();
+    f.net.b_host[l] = f.b[l].data();
+  }
+  return f;
+}
+
+void tick_free(dsmppi_ctx* c);
+
+}  // namespace
 
 extern "C" {
 
 const char* dsmppi_last_error(void) { return g_last_error.c_str(); }
-int dsmppi_version(void) { return 101; }
+int dsmppi_version(void) { return 102; }   // 102: dsmppi_net.n_hidden / hidden_width
 
 void dsmppi_modulation_default(dsmppi_modulation* m) {
   if (!m) return;
@@ -150,6 +193,11 @@ int dsmppi_ctx_create(dsmppi_ctx** out, const dsmppi_net* net, const float* dh_p
   REQUIRE(capacity >= 1, "capacity must be positive");
   const int P = net->n_point_dim == 0 ? 3 : net->n_point_dim;
   REQUIRE(P == 2 || P == 3, "n_point_dim must be 2 or 3");
+  const int L = net->n_hidden == 0 ? MAXL : net->n_hidden;
+  const int W = net->hidden_width == 0 ? HID : net->hidden_width;
+  REQUIRE(L >= 1 && L <= MAXL && W >= 1 && W <= HID,
+          "unsupported network shape: the supported family is 1..4 hidden layers of one width 1..256 (n_hidden, "
+          "hidden_width)");
   int ndev = 0;
   CUDA_TRY(cudaGetDeviceCount(&ndev));
   REQUIRE(ndev > 0 && device < ndev, "no such CUDA device (this library has no CPU fallback)");
@@ -168,6 +216,9 @@ int dsmppi_ctx_create(dsmppi_ctx** out, const dsmppi_net* net, const float* dh_p
   c->capacity = capacity;
   for (int i = 0; i <= c->d; ++i)
     for (int j = 0; j < 4; ++j) c->dh.v[i][j] = dh_params_host[i * 4 + j];
+  // Every image below is built from the 256 x 4 frame, never from the caller's arrays
+  const Frame fr = embed_net(net, c->nenc, L, W);
+  const dsmppi_net* fnet = &fr.net;
   // fp32 weight blob: Wf[l] = W_l^T ([in][256]) and Wb[l] = W_l ([256][in]) for the hidden layers, W4, biases
   const int in_dim[5] = {c->nenc, HID, HID, HID, HID};
   auto pad = [](size_t x) { return (x + 63) / 64 * 64; };
@@ -178,16 +229,16 @@ int dsmppi_ctx_create(dsmppi_ctx** out, const dsmppi_net* net, const float* dh_p
   for (int l = 0; l < 5; ++l) { off_bias[l] = total; total += pad(HID); }
   std::vector<float> blob(total, 0.f);
   for (int l = 0; l < 4; ++l) {
-    const float* W = net->W_host[l];
+    const float* Wl = fnet->W_host[l];
     for (int o = 0; o < HID; ++o)
       for (int k = 0; k < in_dim[l]; ++k) {
-        blob[off_f[l] + (size_t)k * HID + o] = W[(size_t)o * in_dim[l] + k];
-        blob[off_b[l] + (size_t)o * in_dim[l] + k] = W[(size_t)o * in_dim[l] + k];
+        blob[off_f[l] + (size_t)k * HID + o] = Wl[(size_t)o * in_dim[l] + k];
+        blob[off_b[l] + (size_t)o * in_dim[l] + k] = Wl[(size_t)o * in_dim[l] + k];
       }
-    std::memcpy(&blob[off_bias[l]], net->b_host[l], HID * sizeof(float));
+    std::memcpy(&blob[off_bias[l]], fnet->b_host[l], HID * sizeof(float));
   }
-  std::memcpy(&blob[off_w4], net->W_host[4], (size_t)c->O * HID * sizeof(float));
-  std::memcpy(&blob[off_bias[4]], net->b_host[4], (size_t)c->O * sizeof(float));
+  std::memcpy(&blob[off_w4], fnet->W_host[4], (size_t)c->O * HID * sizeof(float));
+  std::memcpy(&blob[off_bias[4]], fnet->b_host[4], (size_t)c->O * sizeof(float));
   if (cudaMalloc(reinterpret_cast<void**>(&c->weights_blob), total * sizeof(float)) != cudaSuccess) {
     delete c;
     dsmppi_set_error("cudaMalloc(weights) failed");
@@ -196,6 +247,8 @@ int dsmppi_ctx_create(dsmppi_ctx** out, const dsmppi_net* net, const float* dh_p
   CUDA_TRY(cudaMemcpy(c->weights_blob, blob.data(), total * sizeof(float), cudaMemcpyHostToDevice));
   c->net.d = c->d; c->net.nin = c->nin; c->net.nenc = c->nenc; c->net.O = c->O;
   c->net.scale = (c->O == 9) ? 0.01f : 1.f;            // MPPI.py:236-237
+  c->net.nh = L;
+  c->net.width = W;
   for (int l = 0; l < 4; ++l) {
     c->net.Wf[l] = c->weights_blob + off_f[l];
     c->net.Wb[l] = c->weights_blob + off_b[l];
@@ -203,8 +256,8 @@ int dsmppi_ctx_create(dsmppi_ctx** out, const dsmppi_net* net, const float* dh_p
   c->net.W4 = c->weights_blob + off_w4;
   for (int l = 0; l < 5; ++l) c->net.b[l] = c->weights_blob + off_bias[l];
   if (exact_set_attributes()) { delete c; return 1; }
-  if (tc_build_images(c, net)) { delete c; return 1; }
-  if (tcx_build_images(c, net)) { delete c; return 1; }
+  if (tc_build_images(c, fnet)) { delete c; return 1; }
+  if (tcx_build_images(c, fnet)) { delete c; return 1; }
   if (const char* e = std::getenv("DSMPPI_HALF_TILES")) c->half_tiles = std::atoi(e) != 0;
   if (const char* e = std::getenv("DSMPPI_PASS1_ACC")) c->pass1_hacc = std::strcmp(e, "f32") != 0;
   c->upd_blocks = c->sm_count * 4;       // update_partial_kernel: four 256-thread CTAs per SM (56 registers per thread)

@@ -18,6 +18,11 @@
 // registers as bit masks (the forward and backward tilings coincide), so the backward pass needs no extra memory.
 // The host picks RPT per launch from the (estimated) row count: big tiles amortise the weight stream, small tiles
 // fill the 148 SMs when there are few rows and shorten the tail of the last wave (pick_rpt below).
+// A network narrower or shallower than 256 x 4 costs what it computes: the kernels are instantiated for WID = 64, 128
+// and 256 features per hidden layer (the smallest that covers the network's width is launched: fewer warps, stages and
+// k-steps) and run net.nh hidden layers, i.e. nh forward GEMMs and nh - 1 backward ones plus W_1^T.  The features past
+// the network's width are zero in the weights, so every WID >= width gives the same bits (ReLU keeps them at 0 and a
+// zero product leaves an fp32 FMA chain unchanged).
 // All arithmetic is IEEE fp32 (no fast-math): this is the path that has to agree with the reference's torch-CPU
 // numbers to ~1e-6.
 #include <cstdlib>
@@ -29,12 +34,15 @@
 namespace {
 using namespace exact_tile;
 
-// resident CTAs per SM the register budget is sized for: the 4-warp shape packs 4 (32-row) or 6 (16-row) tiles on
-// an SM, the 8-warp shape 2, the 16-warp shape 1
-__host__ __device__ constexpr int min_ctas(int RPT, int FT) { return FT == 8 ? (RPT == 8 ? 4 : 6) : (FT == 4 ? (RPT == 8 ? 2 : 3) : 1); }
+// resident CTAs per SM the register budget is sized for: at WID = 256 the 4-warp shape packs 4 (32-row) or 6 (16-row)
+// tiles on an SM, the 8-warp shape 2, the 16-warp shape 1; a narrower tile has proportionally fewer warps, so the same
+// register budget per thread packs proportionally more of them
+__host__ __device__ constexpr int min_ctas(int RPT, int FT, int WID) {
+  return (FT == 8 ? (RPT == 8 ? 4 : 6) : (FT == 4 ? (RPT == 8 ? 2 : 3) : 1)) * (HID / WID);
+}
 
-template <bool BWD, int RPT, int FT>
-__global__ void __launch_bounds__(nthreads(FT), min_ctas(RPT, FT))
+template <bool BWD, int RPT, int FT, int WID>
+__global__ void __launch_bounds__(nthreads(FT, WID), min_ctas(RPT, FT, WID))
 exact_mlp_kernel(NetDev net, RowSrc src, const float* __restrict__ q, int q_stride, const float* __restrict__ obs,
                  uint32_t ignore_mask, float* __restrict__ out_m, float* __restrict__ out_dist,
                  float* __restrict__ out_grad) {
@@ -43,13 +51,14 @@ exact_mlp_kernel(NetDev net, RowSrc src, const float* __restrict__ q, int q_stri
   const int n_rows = src.n_rows_dev ? min(*src.n_rows_dev, src.n_rows) : src.n_rows;
   const int tiles = (n_rows + R - 1) / R;
   if ((int)blockIdx.x >= tiles) return;
-  TileSmem<RPT> sm(smem);
-  WeightStream ws;
+  TileSmem<RPT, WID> sm(smem);
+  WeightStream<WID> ws;
   // one tile per CTA in the regular launches; the re-scoring launch (launch_exact_fixup) strides a bounded grid
-  stream_begin<BWD, nthreads(FT)>(ws, &net, sm.ring, (tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x);
+  stream_begin<BWD, nthreads(FT, WID)>(ws, &net, sm.ring,
+                                       (tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x);
   int stage = 0;
   for (int tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-    mlp_tile<BWD, RPT, FT>(net, src, tile * R, n_rows, q, q_stride, obs, ignore_mask, out_m, out_dist, out_grad, sm, ws,
+    mlp_tile<BWD, RPT, FT, WID>(net, src, tile * R, n_rows, q, q_stride, obs, ignore_mask, out_m, out_dist, out_grad, sm, ws,
                            stage);
     __syncthreads();
   }
@@ -64,8 +73,8 @@ exact_mlp_kernel(NetDev net, RowSrc src, const float* __restrict__ q, int q_stri
 // problems (planar scripts: M = 2..4; Franka integrator tick: N = 1, H = 2) where launch latency, not FLOPs,
 // set the pace of the per-step launch sequence.
 // ------------------------------------------------------------------------------------------------
-template <int RPT, int FT>
-__global__ void __launch_bounds__(nthreads(FT), FT == 8 ? 3 : 2)
+template <int RPT, int FT, int WID>
+__global__ void __launch_bounds__(nthreads(FT, WID), (FT == 8 ? 3 : 2) * (HID / WID))
 rollout_fused_kernel(NetDev net, StepArgs sa, const float* __restrict__ obs, int M, uint32_t ignore_mask,
                      float* m_rows, float* row_dist, float* row_grad, int* sel_rows) {
   constexpr int R = 4 * RPT;
@@ -76,9 +85,9 @@ rollout_fused_kernel(NetDev net, StepArgs sa, const float* __restrict__ obs, int
   const int ns = min(S, sa.N - i0);
   const int row0 = i0 * M;                              // dense rows: row = i * M + j
   const int n_rows = row0 + ns * M;
-  TileSmem<RPT> sm(smem);
-  WeightStream ws;
-  stream_begin<true, nthreads(FT)>(ws, &net, sm.ring, sa.H);
+  TileSmem<RPT, WID> sm(smem);
+  WeightStream<WID> ws;
+  stream_begin<true, nthreads(FT, WID)>(ws, &net, sm.ring, sa.H);
   int stage = 0;
   RowSrc src{};
   src.mode = ROWS_DENSE;
@@ -87,7 +96,7 @@ rollout_fused_kernel(NetDev net, StepArgs sa, const float* __restrict__ obs, int
   const int tid = threadIdx.x;
   for (int t = 1; t <= sa.H; ++t) {
     const float* q = sa.traj + (size_t)(t - 1) * d;     // q_prev = all_traj[:, t-1, :]
-    mlp_tile<true, RPT, FT>(net, src, row0, n_rows, q, sa.H * d, obs, ignore_mask, m_rows, row_dist, row_grad, sm,
+    mlp_tile<true, RPT, FT, WID>(net, src, row0, n_rows, q, sa.H * d, obs, ignore_mask, m_rows, row_dist, row_grad, sm,
                             ws, stage);
     __syncthreads();                                    // the tile's rows are visible to the whole CTA
     if (tid < ns) {
@@ -141,23 +150,33 @@ Shape pick_shape(const dsmppi_ctx* c, long long rows, int min_rows_per_tile) {
   return s;
 }
 
-template <bool BWD, int RPT, int FT>
+template <bool BWD, int RPT, int FT, int WID>
 int launch_variant(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask, float* out_m,
                    float* out_dist, float* out_grad, cudaStream_t st) {
   constexpr int R = 4 * RPT;
   const long long grid = ((long long)src.n_rows + R - 1) / R;
-  exact_mlp_kernel<BWD, RPT, FT><<<(unsigned)grid, nthreads(FT), smem_bytes(R), st>>>(
+  exact_mlp_kernel<BWD, RPT, FT, WID><<<(unsigned)grid, nthreads(FT, WID), smem_bytes(R, WID), st>>>(
       c->net, src, q, q_stride, c->obs, ignore_mask, out_m, out_dist, out_grad);
   CUDA_TRY(cudaGetLastError());
   c->launches++;
   return 0;
 }
 
-#define SHAPE_DISPATCH(sh, CALL)                                  \
+// the smallest instantiated width that covers the network's hidden width
+int tile_width(const dsmppi_ctx* c) { return c->net.width <= 64 ? 64 : (c->net.width <= 128 ? 128 : HID); }
+
+#define SHAPE_DISPATCH_W(sh, W, CALL)                             \
   do {                                                            \
-    if (sh.ft == 8) return CALL(8, 8);                            \
-    if (sh.rpt == 8) return CALL(8, 4);                           \
-    return CALL(4, 4);                                            \
+    if (sh.ft == 8) return CALL(8, 8, W);                         \
+    if (sh.rpt == 8) return CALL(8, 4, W);                        \
+    return CALL(4, 4, W);                                         \
+  } while (0)
+#define SHAPE_DISPATCH(c, sh, CALL)                               \
+  do {                                                            \
+    const int w_ = tile_width(c);                                 \
+    if (w_ == 64) SHAPE_DISPATCH_W(sh, 64, CALL);                 \
+    if (w_ == 128) SHAPE_DISPATCH_W(sh, 128, CALL);               \
+    SHAPE_DISPATCH_W(sh, HID, CALL);                              \
   } while (0)
 
 template <bool BWD>
@@ -166,34 +185,42 @@ int launch(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint3
   if (src.n_rows <= 0) return 0;
   if (rows_estimate <= 0 || rows_estimate > src.n_rows) rows_estimate = src.n_rows;
   const Shape sh = pick_shape(c, rows_estimate, 1);
-#define CALL(RPT, FT) launch_variant<BWD, RPT, FT>(c, q, q_stride, src, ignore_mask, out_m, out_dist, out_grad, st)
-  SHAPE_DISPATCH(sh, CALL);
+#define CALL(RPT, FT, WID) \
+  launch_variant<BWD, RPT, FT, WID>(c, q, q_stride, src, ignore_mask, out_m, out_dist, out_grad, st)
+  SHAPE_DISPATCH(c, sh, CALL);
 #undef CALL
 }
 
-template <int RPT, int FT>
+template <int RPT, int FT, int WID>
 int launch_fused_variant(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream_t st) {
   constexpr int R = 4 * RPT;
   const int S = R / c->M;
   const long long grid = ((long long)a->N + S - 1) / S;
   const StepArgs sa = make_step_args(c, a, 0);
-  rollout_fused_kernel<RPT, FT><<<(unsigned)grid, nthreads(FT), smem_bytes(R), st>>>(
+  rollout_fused_kernel<RPT, FT, WID><<<(unsigned)grid, nthreads(FT, WID), smem_bytes(R, WID), st>>>(
       c->net, sa, c->obs, c->M, a->ignored_link_mask, c->m_rows, c->row_dist, c->row_grad, c->sel_rows);
   CUDA_TRY(cudaGetLastError());
   c->launches++;
   return 0;
 }
 
-template <int RPT, int FT>
+template <int RPT, int FT, int WID>
 int set_attributes_variant() {
   constexpr int R = 4 * RPT;
-  CUDA_TRY(cudaFuncSetAttribute(exact_mlp_kernel<true, RPT, FT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)smem_bytes(R)));
-  CUDA_TRY(cudaFuncSetAttribute(exact_mlp_kernel<false, RPT, FT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)smem_bytes(R)));
-  CUDA_TRY(cudaFuncSetAttribute(rollout_fused_kernel<RPT, FT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)smem_bytes(R)));
+  CUDA_TRY(cudaFuncSetAttribute(exact_mlp_kernel<true, RPT, FT, WID>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)smem_bytes(R, WID)));
+  CUDA_TRY(cudaFuncSetAttribute(exact_mlp_kernel<false, RPT, FT, WID>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)smem_bytes(R, WID)));
+  CUDA_TRY(cudaFuncSetAttribute(rollout_fused_kernel<RPT, FT, WID>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)smem_bytes(R, WID)));
   return 0;
+}
+
+template <int WID>
+int set_attributes_width() {
+  if (set_attributes_variant<8, 8, WID>()) return 1;
+  if (set_attributes_variant<8, 4, WID>()) return 1;
+  return set_attributes_variant<4, 4, WID>();
 }
 
 }  // namespace
@@ -202,9 +229,9 @@ int set_attributes_variant() {
 // cudaSetDevice, so a second context on another GPU of the same process gets it too (a process-wide "done" flag
 // would leave that device without it).
 int exact_set_attributes() {
-  if (set_attributes_variant<8, 8>()) return 1;
-  if (set_attributes_variant<8, 4>()) return 1;
-  return set_attributes_variant<4, 4>();
+  if (set_attributes_width<64>()) return 1;
+  if (set_attributes_width<128>()) return 1;
+  return set_attributes_width<HID>();
 }
 
 // whole-horizon single launch; the caller has checked M <= 32 and initialised all_traj[:, 0]
@@ -212,25 +239,36 @@ int launch_rollout_fused(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream
   const int M = c->M;
   // a CTA holds whole samples: S = R / M of them, so the row count that matters is N * (R / S) ~ N * M
   const Shape sh = pick_shape(c, (long long)a->N * M, M);
-#define CALL(RPT, FT) launch_fused_variant<RPT, FT>(c, a, st)
-  SHAPE_DISPATCH(sh, CALL);
+#define CALL(RPT, FT, WID) launch_fused_variant<RPT, FT, WID>(c, a, st)
+  SHAPE_DISPATCH(c, sh, CALL);
 #undef CALL
 }
 
-int launch_exact_fixup(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
+namespace {
+template <int WID>
+int launch_fixup_width(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
                        float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st) {
   constexpr int RPT = 8, FT = 8, R = 4 * RPT;
   long long grid = ((long long)src.n_rows + R - 1) / R;
   if (grid > 4LL * c->sm_count) grid = 4LL * c->sm_count;       // usually no row is flagged: keep the launch tiny
   if (bwd)
-    exact_mlp_kernel<true, RPT, FT><<<(unsigned)grid, nthreads(FT), smem_bytes(R), st>>>(
+    exact_mlp_kernel<true, RPT, FT, WID><<<(unsigned)grid, nthreads(FT, WID), smem_bytes(R, WID), st>>>(
         c->net, src, q, q_stride, c->obs, ignore_mask, m_rows, row_dist, row_grad);
   else
-    exact_mlp_kernel<false, RPT, FT><<<(unsigned)grid, nthreads(FT), smem_bytes(R), st>>>(
+    exact_mlp_kernel<false, RPT, FT, WID><<<(unsigned)grid, nthreads(FT, WID), smem_bytes(R, WID), st>>>(
         c->net, src, q, q_stride, c->obs, ignore_mask, m_rows, nullptr, nullptr);
   CUDA_TRY(cudaGetLastError());
   c->launches++;
   return 0;
+}
+}  // namespace
+
+int launch_exact_fixup(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
+                       float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st) {
+  const int w = tile_width(c);
+  if (w == 64) return launch_fixup_width<64>(c, q, q_stride, src, ignore_mask, m_rows, row_dist, row_grad, bwd, st);
+  if (w == 128) return launch_fixup_width<128>(c, q, q_stride, src, ignore_mask, m_rows, row_dist, row_grad, bwd, st);
+  return launch_fixup_width<HID>(c, q, q_stride, src, ignore_mask, m_rows, row_dist, row_grad, bwd, st);
 }
 
 int launch_exact_forward(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,

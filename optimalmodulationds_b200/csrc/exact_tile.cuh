@@ -1,8 +1,10 @@
 // The fp32 (IEEE FFMA) network tile shared by exact_mlp.cu (its kernels) and tc_exact.cu (which re-scores, inside its
-// whole-horizon kernel, the rows that left the fp16 range): rows -> encoded inputs -> 4 hidden layers -> output layer
-// -> analytic VJP, on R = 4 * RPT rows held feature-major in shared memory.  See exact_mlp.cu for the design notes.
-// Every barrier is the named barrier 2 over the NT = nthreads(FT) threads that run the tile, so a kernel may hand the
-// tile to a subset of its warps (threadIdx.x < NT) while the others do something else.
+// whole-horizon kernel, the rows that left the fp16 range): rows -> encoded inputs -> net.nh hidden layers -> output
+// layer -> analytic VJP, on R = 4 * RPT rows held feature-major in shared memory.  See exact_mlp.cu for the design notes.
+// WID is the number of features the tile computes per hidden layer (64, 128 or 256, at least the network's width; the
+// weights are read from the 256 x 4 frame, whose features past the network's width are zero).
+// Every barrier is the named barrier 2 over the NT = nthreads(FT, WID) threads that run the tile, so a kernel may hand
+// the tile to a subset of its warps (threadIdx.x < NT) while the others do something else.
 #pragma once
 #include "internal.cuh"
 
@@ -11,9 +13,10 @@ namespace exact_tile {
 template <int NT>
 __device__ __forceinline__ void tile_sync() { asm volatile("bar.sync 2, %0;" ::"n"(NT) : "memory"); }
 
-__host__ __device__ constexpr int nthreads(int FT) { return 32 * (HID / (8 * FT)); }   // 128 / 256 / 512 threads for FT = 8 / 4 / 2
+// a warp computes 8 * FT features: 128 / 256 / 512 threads for FT = 8 / 4 / 2 at WID = 256
+__host__ __device__ constexpr int nthreads(int FT, int WID = HID) { return 32 * (WID / (8 * FT)); }
 constexpr int XS = 12;    // padded row stride of the raw-input scratch (nin <= 11)
-constexpr int WS = 8;     // k-rows of weights per pipeline stage (8 KB)
+constexpr int WS = 8;     // k-rows of weights per pipeline stage (8 KB at WID = 256)
 constexpr int NSTAGE = 4; // ring depth
 
 __device__ __forceinline__ bool row_lookup(const RowSrc& s, int r, int n_rows, int& i, int& j) {
@@ -43,7 +46,7 @@ struct Tile {
   __device__ __forceinline__ int feat(int j) const { return FT == 8 ? fa + (j & 3) + ((j >> 2) << 5) : fa + j; }
 };
 
-// FT consecutive-group values of a 256-wide row (weights of one k, or a bias vector) for this thread's tile
+// FT consecutive-group values of a feature row (weights of one k, or a bias vector) for this thread's tile
 template <int FT>
 __device__ __forceinline__ void load_feats(const float* p, float (&w)[FT]) {
   if constexpr (FT == 8) {
@@ -97,11 +100,13 @@ __device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
   return d;
 }
 
-// The weight stream: GEMM g = 0..3 are the forward layers (Wf[g], K = nenc or 256), g = 4..6 the backward ones
-// (Wb[3], Wb[2], Wb[1]); stage indices run through all of them.
+// The weight stream: GEMM g = 0..L-1 are the forward layers (Wf[g], K = nenc or WID), g = L..2L-2 the backward ones
+// (Wb[L-1], .., Wb[1]), L = net->nh; stage indices run through all of them.  A stage is WS k-rows of WID features,
+// taken from the 256-wide rows of the frame.
+template <int WID = HID>
 struct WeightStream {
   const NetDev* net;
-  float* ring;            // [NSTAGE][WS][HID]
+  float* ring;            // [NSTAGE][WS][WID]
   int n0;                 // stages of GEMM 0 = ceil(nenc / WS)
   int per_pass;           // stages of one pass over a row tile (forward, or forward + backward)
   int total;              // stages in the whole stream: per_pass x number of passes this CTA makes
@@ -111,9 +116,10 @@ struct WeightStream {
     int g, st;
     stage %= per_pass;
     if (stage < n0) { g = 0; st = stage; }
-    else { g = 1 + (stage - n0) / (HID / WS); st = (stage - n0) % (HID / WS); }
-    const int K = g == 0 ? net->nenc : HID;
-    const float* W = g < 4 ? net->Wf[g] : net->Wb[7 - g];
+    else { g = 1 + (stage - n0) / (WID / WS); st = (stage - n0) % (WID / WS); }
+    const int K = g == 0 ? net->nenc : WID;
+    const int L = net->nh;
+    const float* W = g < L ? net->Wf[g] : net->Wb[2 * L - 1 - g];
     src = W + (size_t)st * WS * HID;
     rows = min(WS, K - st * WS);
   }
@@ -124,20 +130,23 @@ struct WeightStream {
       const float* src;
       int rows;
       locate(issued, src, rows);
-      float* dst = ring + (size_t)(issued % NSTAGE) * WS * HID;
-      for (int c = threadIdx.x; c < rows * (HID / 4); c += NT) cp_async16(dst + c * 4, src + c * 4);
+      float* dst = ring + (size_t)(issued % NSTAGE) * WS * WID;
+      for (int c = threadIdx.x; c < rows * (WID / 4); c += NT) {
+        const int kk = c / (WID / 4), f = c - kk * (WID / 4);
+        cp_async16(dst + kk * WID + f * 4, src + (size_t)kk * HID + f * 4);
+      }
     }
     ++issued;
     cp_async_commit();
   }
 };
 
-// acc[i][j] = sum_k act[k][r0+i] * W[k*256 + feat(j)], W arriving through the ring; `stage` is the stream position
+// acc[i][j] = sum_k act[k][r0+i] * W[k*WID + feat(j)], W arriving through the ring; `stage` is the stream position
 // of this GEMM's first stage and is advanced past its last one
-template <int RPT, int FT>
-__device__ __forceinline__ void gemm_tile(WeightStream& ws, int& stage, int K, const float (*act)[4 * RPT],
+template <int RPT, int FT, int WID>
+__device__ __forceinline__ void gemm_tile(WeightStream<WID>& ws, int& stage, int K, const float (*act)[4 * RPT],
                                           const Tile<FT>& t, float (&acc)[RPT][FT]) {
-  constexpr int NT = nthreads(FT);
+  constexpr int NT = nthreads(FT, WID);
   uint64_t acc2[RPT][FT / 2];             // acc2[i][p] = (acc[i][2p], acc[i][2p+1])
 #pragma unroll
   for (int i = 0; i < RPT; ++i)
@@ -147,14 +156,14 @@ __device__ __forceinline__ void gemm_tile(WeightStream& ws, int& stage, int K, c
     cp_async_wait<NSTAGE - 2>();          // this thread's share of `stage` has landed ...
     tile_sync<NT>();                      // ... and everybody's; the buffer of stage-1 is free again
     ws.template request_next<NT>();       // refill it with stage + NSTAGE - 1
-    const float* wb = ws.ring + (size_t)(stage % NSTAGE) * WS * HID + t.fa;
+    const float* wb = ws.ring + (size_t)(stage % NSTAGE) * WS * WID + t.fa;
     const int rows = min(WS, K - k0);
     if (rows == WS) {
 #pragma unroll
       for (int kk = 0; kk < WS; ++kk) {
         float a[RPT], w[FT];
         load_rows<RPT>(&act[k0 + kk][t.r0], a);
-        load_feats<FT>(wb + kk * HID, w);
+        load_feats<FT>(wb + kk * WID, w);
         uint64_t wp[FT / 2];
 #pragma unroll
         for (int p = 0; p < FT / 2; ++p) wp[p] = pack2f(w[2 * p], w[2 * p + 1]);
@@ -169,7 +178,7 @@ __device__ __forceinline__ void gemm_tile(WeightStream& ws, int& stage, int K, c
       for (int kk = 0; kk < rows; ++kk) {
         float a[RPT], w[FT];
         load_rows<RPT>(&act[k0 + kk][t.r0], a);
-        load_feats<FT>(wb + kk * HID, w);
+        load_feats<FT>(wb + kk * WID, w);
         uint64_t wp[FT / 2];
 #pragma unroll
         for (int p = 0; p < FT / 2; ++p) wp[p] = pack2f(w[2 * p], w[2 * p + 1]);
@@ -204,19 +213,20 @@ __device__ __forceinline__ void store_tile(float (*act)[4 * RPT], const Tile<FT>
   }
 }
 
-template <int RPT>
+template <int RPT, int WID = HID>
 struct TileSmem {
   static constexpr int R = 4 * RPT;
-  float (*act)[R];   // [256][R]
-  float* ring;       // [NSTAGE][WS][256] weight stages
+  static_assert(WID >= 3 * (MAXD + 3), "the encoded inputs share the activation rows");
+  float (*act)[R];   // [WID][R]
+  float* ring;       // [NSTAGE][WS][WID] weight stages
   float* xs;         // [R][XS]  raw inputs x = [q, p]
   float* zs;         // [R][MAXO] raw outputs
   float* rad;        // [R]
   int* lst;          // [R] argmin link
   __device__ __forceinline__ explicit TileSmem(float* smem) {
     act = reinterpret_cast<float (*)[R]>(smem);
-    ring = smem + HID * R;
-    xs = ring + NSTAGE * WS * HID;
+    ring = smem + WID * R;
+    xs = ring + NSTAGE * WS * WID;
     zs = xs + R * XS;
     rad = zs + R * MAXO;
     lst = reinterpret_cast<int*>(rad + R);
@@ -225,12 +235,12 @@ struct TileSmem {
 
 // starts the weight stream of a CTA that will make `passes` passes over row tiles: the first three stages fly
 // while the inputs are encoded
-template <bool BWD, int NT>
-__device__ __forceinline__ void stream_begin(WeightStream& ws, const NetDev* net, float* ring, int passes) {
+template <bool BWD, int NT, int WID>
+__device__ __forceinline__ void stream_begin(WeightStream<WID>& ws, const NetDev* net, float* ring, int passes) {
   ws.net = net;
   ws.ring = ring;
   ws.n0 = (net->nenc + WS - 1) / WS;
-  ws.per_pass = ws.n0 + (BWD ? 6 : 3) * (HID / WS);
+  ws.per_pass = ws.n0 + (BWD ? 2 : 1) * (net->nh - 1) * (WID / WS);
   ws.total = ws.per_pass * passes;
   ws.issued = 0;
 #pragma unroll
@@ -239,13 +249,13 @@ __device__ __forceinline__ void stream_begin(WeightStream& ws, const NetDev* net
 
 // One pass of the network over the R rows [row0, row0 + R) of `src` (rows >= n_rows are padding): forward, and with
 // BWD the analytic VJP.  Called by all NT threads of the CTA; `ws` / `stage` carry the weight stream across calls.
-template <bool BWD, int RPT, int FT>
+template <bool BWD, int RPT, int FT, int WID = HID>
 __device__ __forceinline__ void mlp_tile(const NetDev& net, const RowSrc& src, int row0, int n_rows,
                                          const float* q, int q_stride, const float* __restrict__ obs,
                                          uint32_t ignore_mask, float* out_m, float* out_dist, float* out_grad,
-                                         const TileSmem<RPT>& sm, WeightStream& ws, int& stage) {
+                                         const TileSmem<RPT, WID>& sm, WeightStream<WID>& ws, int& stage) {
   constexpr int R = 4 * RPT;
-  constexpr int NT = nthreads(FT);
+  constexpr int NT = nthreads(FT, WID);
   float (*act)[R] = sm.act;
   float* xs = sm.xs;
   float* zs = sm.zs;
@@ -254,7 +264,7 @@ __device__ __forceinline__ void mlp_tile(const NetDev& net, const RowSrc& src, i
   const int tid = threadIdx.x;
   Tile<FT> t;
   t.init(tid, RPT);
-  const int d = net.d, nin = net.nin, nenc = net.nenc, O = net.O;
+  const int d = net.d, nin = net.nin, nenc = net.nenc, O = net.O, L = net.nh;
 
   // ---- rows -> encoded inputs [x, sin x, cos x]  (network_macros_mod.py:139-140)
   for (int idx = tid; idx < R * nin; idx += NT) {
@@ -271,12 +281,12 @@ __device__ __forceinline__ void mlp_tile(const NetDev& net, const RowSrc& src, i
   }
   tile_sync<NT>();
 
-  uint64_t mk[4];          // ReLU masks of this thread's tile, bit i*FT+j
+  uint64_t mk[MAXL];       // ReLU masks of this thread's tile, bit i*FT+j
   float acc[RPT][FT];
   // ---- hidden layers: h = relu(W h + b)
 #pragma unroll 1
-  for (int l = 0; l < 4; ++l) {
-    gemm_tile<RPT, FT>(ws, stage, l == 0 ? nenc : HID, act, t, acc);
+  for (int l = 0; l < L; ++l) {
+    gemm_tile<RPT, FT, WID>(ws, stage, l == 0 ? nenc : WID, act, t, acc);
     tile_sync<NT>();
     float bb[FT];
     load_feats<FT>(net.b[l] + t.fa, bb);
@@ -301,7 +311,7 @@ __device__ __forceinline__ void mlp_tile(const NetDev& net, const RowSrc& src, i
     const float* w = net.W4 + o * HID;
     float s = 0.f;
 #pragma unroll 8
-    for (int k = 0; k < HID; ++k) s = fmaf(act[k][r], __ldg(w + k), s);
+    for (int k = 0; k < WID; ++k) s = fmaf(act[k][r], __ldg(w + k), s);
     zs[r * MAXO + o] = s + __ldg(net.b[4] + o);
   }
   tile_sync<NT>();
@@ -350,17 +360,17 @@ __device__ __forceinline__ void mlp_tile(const NetDev& net, const RowSrc& src, i
 #pragma unroll
   for (int i = 0; i < RPT; ++i) {
     const float* w = net.W4 + lst[t.r0 + i] * HID;
-    const uint32_t bits = (uint32_t)(mk[3] >> (i * FT)) & 0xffu;
+    const uint32_t bits = (uint32_t)(mk[L - 1] >> (i * FT)) & 0xffu;
 #pragma unroll
     for (int j = 0; j < FT; ++j) acc[i][j] = ((bits >> j) & 1u) ? __ldg(w + t.feat(j)) : 0.f;
   }
   store_tile<RPT, FT>(act, t, acc);
   tile_sync<NT>();
 
-  // g_{l-1} = (W_l^T g_l) * s_{l-1},  l = 3, 2, 1   (Wb[l] is torch's [out][in]: out = k, in = n)
+  // g_{l-1} = (W_l^T g_l) * s_{l-1},  l = L-1, .., 1   (Wb[l] is torch's [out][in]: out = k, in = n)
 #pragma unroll 1
-  for (int l = 3; l >= 1; --l) {
-    gemm_tile<RPT, FT>(ws, stage, HID, act, t, acc);
+  for (int l = L - 1; l >= 1; --l) {
+    gemm_tile<RPT, FT, WID>(ws, stage, WID, act, t, acc);
     tile_sync<NT>();
     const uint64_t m = mk[l - 1];
 #pragma unroll
@@ -380,7 +390,7 @@ __device__ __forceinline__ void mlp_tile(const NetDev& net, const RowSrc& src, i
     const float* w = net.Wb[0];
     float a0 = 0.f, a1 = 0.f, a2 = 0.f;
 #pragma unroll 4
-    for (int k = 0; k < HID; ++k) {
+    for (int k = 0; k < WID; ++k) {
       const float g = act[k][r];
       a0 = fmaf(g, __ldg(w + k * nenc + c), a0);
       a1 = fmaf(g, __ldg(w + k * nenc + nin + c), a1);
@@ -396,8 +406,8 @@ __device__ __forceinline__ void mlp_tile(const NetDev& net, const RowSrc& src, i
 }
 
 
-constexpr size_t smem_bytes(int R) {
-  return (size_t)(HID * R + NSTAGE * WS * HID + R * XS + R * MAXO + R + R) * sizeof(float);
+constexpr size_t smem_bytes(int R, int WID = HID) {
+  return (size_t)(WID * R + NSTAGE * WS * WID + R * XS + R * MAXO + R + R) * sizeof(float);
 }
 
 }  // namespace exact_tile

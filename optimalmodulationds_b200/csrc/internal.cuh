@@ -8,6 +8,7 @@
 #include "dsmppi_b200.h"
 
 #define HID DSMPPI_HIDDEN
+#define MAXL DSMPPI_MAX_HIDDEN_LAYERS
 #define MAXD DSMPPI_MAX_DOF
 #define MAXO DSMPPI_MAX_LINKS
 #define MAXK DSMPPI_MAX_CLOSEST
@@ -44,6 +45,8 @@ struct NetDev {
   int nenc;     // 3 * nin
   int O;        // links
   float scale;  // 0.01 when O == 9 (centimetres -> metres, MPPI.py:236-237), else 1
+  int nh;       // hidden layers of the caller's network (1..4); the arrays below hold it embedded in 256 x 4
+  int width;    // width of its hidden layers (1..256)
   const float* Wf[4];   // layers 0..3, forward orientation [in][256]
   const float* Wb[4];   // layers 0..3, torch orientation  [256][in]
   const float* W4;      // output layer, torch orientation [O][256]
@@ -170,14 +173,15 @@ int launch_rollout_fused(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream
 int launch_exact_fixup(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
                        float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st);
 // tc_exact.cu: the same rows / outputs as the two launches above, on the tensor cores (split-fp16 operands)
-int tcx_build_images(dsmppi_ctx* c, const dsmppi_net* net);
+// (both image builders take the network embedded in the 256 x 4 frame by dsmppi_ctx_create, never the caller's)
+int tcx_build_images(dsmppi_ctx* c, const dsmppi_net* frame);
 void tcx_free_images(dsmppi_ctx* c);
 int launch_tc_exact(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask, float* m_rows,
                     float* row_dist, float* row_grad, bool bwd, cudaStream_t st);
 int launch_tc_rollout(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream_t st);
 inline bool use_tc_scoring(const dsmppi_ctx* c) { return c->tcx_blob && c->score_mode != DSMPPI_SCORE_FFMA; }
 // tc_pass1.cu
-int tc_build_images(dsmppi_ctx* c, const dsmppi_net* net);
+int tc_build_images(dsmppi_ctx* c, const dsmppi_net* frame);
 void tc_free_images(dsmppi_ctx* c);
 int tc_set_obstacles(dsmppi_ctx* c, cudaStream_t st);
 // table_ready: the per-sample layer-1 table (c->enc_q) of these n states has already been written

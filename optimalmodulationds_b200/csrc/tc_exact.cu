@@ -83,8 +83,21 @@ constexpr int NSLOT = 3;
 constexpr int SLOT_BYTES = 32768;
 constexpr uint32_t A_LBO = TROWS * 16;     // bytes between consecutive 8-element K chunks of the A images
 constexpr float SPLIT = 2048.f, INV_SPLIT = 1.f / 2048.f;
-// accumulator-truncation compensation of a D1 chain of n MMA steps: 1.65e-8 n + 2.1e-8 (see the header)
-constexpr float COMP_K256 = 1.65e-8f * 16 + 2.1e-8f, COMP_K32 = 1.65e-8f * 2 + 2.1e-8f;
+// accumulator-truncation compensation of a D1 chain of n MMA steps: 1.65e-8 n + 2.1e-8 (see the header).  Only steps
+// with a non-zero product truncate: a GEMM over the hidden features of a W-wide network (embedded in the 256 x 4 frame)
+// needs comp_steps(ceil(W / 16)), and an identity layer of the frame, one non-zero product per sum, needs 0.
+__host__ __device__ constexpr float comp_steps(int n) { return n > 0 ? 1.65e-8f * n + 2.1e-8f : 0.f; }
+constexpr float COMP_K256 = comp_steps(16), COMP_K32 = comp_steps(2);
+static_assert(COMP_K256 == 1.65e-8f * 16 + 2.1e-8f && COMP_K32 == 1.65e-8f * 2 + 2.1e-8f, "shipped constants");
+// per-GEMM compensation of a pass: [0..3] forward layers, [4] output layer, [5..7] backward W_l^T for l = 3, 2, 1,
+// [8] the final W_1^T
+constexpr int N_GEMM = 9;
+__device__ __forceinline__ float comp_of(const float (&comp)[N_GEMM], int g) {
+  float v = comp[0];
+#pragma unroll
+  for (int i = 1; i < N_GEMM; ++i) v = g == i ? comp[i] : v;
+  return v;
+}
 __device__ __forceinline__ float combine(uint32_t d1, uint32_t d2, float comp) {
   const float a = __uint_as_float(d1);
   return fmaf(a, comp, fmaf(__uint_as_float(d2), INV_SPLIT, a));
@@ -205,6 +218,7 @@ struct TxArgs {
   int fix_cap;
   // whole-horizon mode (MODE 2): a CTA owns S = 128 / M samples and all of their (sample, obstacle) rows for all H steps
   StepArgs sa; int M; int S; float* m_rows; float* row_dist; float* row_grad; int* sel_rows;
+  float comp[N_GEMM];                        // accumulator-truncation compensation per GEMM (set_compensation)
   int dbg;                                   // DSMPPI_TCX_DEBUG=4: no accumulator-truncation compensation (precision tools)
   long long* prof;                           // -DDSMPPI_TCX_PROF builds: (event id, clock64) pairs of CTA 0's warps
 };
@@ -541,7 +555,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
 #pragma unroll 1
       for (int l = 0; l < 4; ++l) {
         const float* bl = net.b[l] + cb;
-        const float comp = (a.dbg & 4) ? 0.f : (l == 0 ? COMP_K32 : COMP_K256);
+        const float comp = (a.dbg & 4) ? 0.f : comp_of(a.comp, l);
         if constexpr (HM) {
           // one 32-column chunk per N half: features 128 x + 64 fb + 32 h + [0, 32) -> K quarter 2 x + fb
           wait_d0();
@@ -628,7 +642,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
         if (q4 == 0) TCX_PROF(h, 64);
         // straight-line; the links the network does not have (o >= O, a launch-wide constant: uniform branches) are
         // skipped -- their IEEE divisions were half of this epilogue for the 7- and 9-link networks
-        const float comp_o = (a.dbg & 4) ? 0.f : COMP_K256;
+        const float comp_o = (a.dbg & 4) ? 0.f : a.comp[4];
         const float* b4s = reinterpret_cast<const float*>(smem + OFF_B4);
         const bool scaled = net.scale != 1.f;
         float v[16];
@@ -746,7 +760,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
         // ---- g_{l-1} = (W_l^T g_l) * s_{l-1},  l = 3, 2, 1 (same half-by-half schedule as the forward layers)
 #pragma unroll 1
         for (int l = 3; l >= 1; --l) {
-          const float comp = (a.dbg & 4) ? 0.f : COMP_K256;
+          const float comp = (a.dbg & 4) ? 0.f : comp_of(a.comp, 8 - l);
           if constexpr (HM) {
             wait_d0();
             {
@@ -831,7 +845,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
             tc_wait_ld();
             float* scr = reinterpret_cast<float*>(smem + OFF_SCRATCH) + row;
 #pragma unroll
-            for (int e = 0; e < 16; ++e) scr[(16 * fb + e) * TROWS] = combine(r1[e], r2[e], (a.dbg & 4) ? 0.f : COMP_K256);
+            for (int e = 0; e < 16; ++e) scr[(16 * fb + e) * TROWS] = combine(r1[e], r2[e], (a.dbg & 4) ? 0.f : a.comp[8]);
           }
           asm volatile("bar.sync 1, 256;" ::: "memory");
           if (h == 0 && fb == 0) {
@@ -847,7 +861,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
           tc_wait_ld();
           float* scr = reinterpret_cast<float*>(smem + OFF_SCRATCH) + row;     // a[e] at scr[e * 128]
 #pragma unroll
-          for (int e = 0; e < 32; ++e) scr[e * TROWS] = combine(r1[e], r2[e], (a.dbg & 4) ? 0.f : COMP_K256);
+          for (int e = 0; e < 32; ++e) scr[e * TROWS] = combine(r1[e], r2[e], (a.dbg & 4) ? 0.f : a.comp[8]);
 #pragma unroll
           for (int c = 0; c < MAXD; ++c)
             if (c < d) o_g[c] = scr[c * TROWS] + cs[c] * scr[(nin + c) * TROWS] - sn[c] * scr[(2 * nin + c) * TROWS];
@@ -881,7 +895,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
         if (nfix > 0) {
           if (tid < exact_tile::nthreads(8)) {
             exact_tile::TileSmem<8> ts(reinterpret_cast<float*>(smem + OFF_AHI));
-            exact_tile::WeightStream ws;
+            exact_tile::WeightStream<> ws;
             const int passes = (nfix + 31) / 32;
             exact_tile::stream_begin<true, exact_tile::nthreads(8)>(ws, &a.net, ts.ring, passes);
             RowSrc fs{};
@@ -952,7 +966,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
         if (nfix > 0 && tid < exact_tile::nthreads(8)) {
           // the FFMA tile of exact_mlp.cu on warps 0-3, its shared memory carved out of the (idle) A operand images
           exact_tile::TileSmem<8> ts(reinterpret_cast<float*>(smem + OFF_AHI));
-          exact_tile::WeightStream ws;
+          exact_tile::WeightStream<> ws;
           const int passes = (nfix + 31) / 32;
           exact_tile::stream_begin<true, exact_tile::nthreads(8)>(ws, &a.net, ts.ring, passes);
           RowSrc fs{};
@@ -1261,6 +1275,18 @@ inline size_t canon(int n, int k, int rows) {
   return (size_t)(k / 8) * rows * 16 + (size_t)n * 16 + (size_t)(k % 8) * 2;
 }
 
+// Per-GEMM compensation of the network in hand.  Layer 1 keeps c(2) (K = 3(d+P) <= 32 whatever the width); for the
+// 256 x 4 network every other GEMM gets c(16), the constants the kernel had before networks of other shapes existed.
+void set_compensation(const dsmppi_ctx* c, float (&comp)[N_GEMM]) {
+  const int L = c->net.nh;
+  const float hid = comp_steps((c->net.width + 15) / 16);    // a GEMM over the hidden features
+  comp[0] = COMP_K32;
+  for (int l = 1; l < 4; ++l) comp[l] = l < L ? hid : 0.f;   // forward layer l + 1: hidden, or identity
+  comp[4] = hid;
+  for (int l = 3; l >= 1; --l) comp[8 - l] = l < L ? hid : 0.f;
+  comp[8] = hid;
+}
+
 }  // namespace
 
 int tcx_build_images(dsmppi_ctx* c, const dsmppi_net* net) {
@@ -1378,6 +1404,7 @@ int launch_tc_exact(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& s
   a.fix_list = c->fix_list;
   a.fix_cap = (int)c->fix_cap;
   c->fix_parity ^= 1;
+  set_compensation(c, a.comp);
   const char* dbg = std::getenv("DSMPPI_TCX_DEBUG");
   a.dbg = dbg ? std::atoi(dbg) : 0;
   a.prof = nullptr;
@@ -1454,6 +1481,7 @@ int launch_tc_rollout(dsmppi_ctx* c, const dsmppi_rollout_args* ra, cudaStream_t
   a.fix_dropped = c->counters + 7;
   a.fix_list = nullptr;
   a.fix_cap = 0;
+  set_compensation(c, a.comp);
   const char* dbg = std::getenv("DSMPPI_TCX_DEBUG");
   a.dbg = dbg ? std::atoi(dbg) : 0;
 #ifdef DSMPPI_TCX_PROF
