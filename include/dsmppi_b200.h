@@ -232,7 +232,8 @@ int dsmppi_distance_grad_fk(dsmppi_ctx* ctx, const float* q_dev, int32_t n, int3
                             float* distance_dev, float* grad_dev, int32_t* closest_idx_dev, void* stream);
 
 /* Test hook: the per-pair masked minimum link distance of pass 1 (MPPI.py:235-243), (n, M) row-major, from
- * the fp32 path (mode = DSMPPI_PASS1_EXACT_FP32) or the tensor-core prefilter (TC_F16 / TC_BF16). */
+ * the fp32 path (mode = DSMPPI_PASS1_EXACT_FP32) or the tensor-core prefilter (TC_F16 / TC_BF16).  Any other mode,
+ * AUTO included, returns 2. */
 int dsmppi_debug_pass1(dsmppi_ctx* ctx, const float* q_dev, int32_t n, uint32_t ignored_link_mask, int32_t mode,
                        float* out_dev, void* stream);
 

@@ -33,11 +33,43 @@ int alloc(T*& p, size_t n) {
 }
 
 constexpr int FUSE_M_MAX = 16;   // up to this many obstacles the fp32 path differentiates every pair in one launch
-int resolved_mode(const dsmppi_ctx* c) {
-  int m = c->pass1_mode;
-  if (m == DSMPPI_PASS1_AUTO) m = (c->M >= 64 && c->tc_blob) ? DSMPPI_PASS1_TC_F16 : DSMPPI_PASS1_EXACT_FP32;
+
+// The pass-1 mode that runs when `requested` is asked for with M obstacles: AUTO takes the fp16 prefilter from 64
+// obstacles on, and every tensor-core mode needs the prefilter's weight images.  Each entry point resolves once and
+// passes the result down; the context's own mode and obstacle count are only written by their setters.
+int resolve_mode(const dsmppi_ctx* c, int requested, int M) {
+  int m = requested;
+  if (m == DSMPPI_PASS1_AUTO) m = (M >= 64 && c->tc_blob) ? DSMPPI_PASS1_TC_F16 : DSMPPI_PASS1_EXACT_FP32;
   if (m != DSMPPI_PASS1_EXACT_FP32 && !c->tc_blob) m = DSMPPI_PASS1_EXACT_FP32;
   return m;
+}
+
+// which of band_cal / band_cal_M / band_cal_err holds the guard band of a prefilter mode
+int band_slot(int mode) { return mode == DSMPPI_PASS1_TC_BF16 ? 1 : 0; }
+
+// Samples never interact, so a very large batch is processed in blocks of samples: it bounds the workspace
+// (the (n, M) prefilter matrix is the big one: <= 1 GiB) and keeps every row index inside 31 bits.
+long long sample_block(const dsmppi_ctx* c) {
+  const long long block = (1LL << 28) / c->M;
+  return block > (1 << 18) ? 1 << 18 : block < 1 ? 1 : block;
+}
+
+// the arguments of samples [off, off + n) of a batch
+dsmppi_rollout_args slice_samples(const dsmppi_rollout_args& a, int d, long long off, int n) {
+  dsmppi_rollout_args b = a;
+  b.N = n;
+  if (a.q_cur_is_batch) b.q_cur_dev = a.q_cur_dev + off * d;
+  if (a.mu_tmp_dev) b.mu_tmp_dev = a.mu_tmp_dev + off * NKMAX * d;
+  if (a.sigma_tmp_dev) b.sigma_tmp_dev = a.sigma_tmp_dev + off * NKMAX;
+  if (a.alpha_tmp_dev) b.alpha_tmp_dev = a.alpha_tmp_dev + off * NKMAX * d;
+  b.all_traj_dev = a.all_traj_dev + off * a.H * d;
+  b.closest_dist_all_dev = a.closest_dist_all_dev + off * a.H;
+  b.kernel_val_all_dev = a.kernel_val_all_dev + off * a.H * NKMAX;
+  b.dot_products_dev = a.dot_products_dev + off * a.H;
+  b.kernel_activations_dev = a.kernel_activations_dev + off * a.H;
+  b.qdot_dev = a.qdot_dev + off * d;
+  b.nn_grad_all_dev = a.nn_grad_all_dev + off * a.H * d;
+  return b;
 }
 
 constexpr int WHOLE_M_MAX = 32;  // largest obstacle set a row tile of the whole-horizon kernel can hold
@@ -45,8 +77,8 @@ constexpr int WHOLE_M_MAX = 32;  // largest obstacle set a row tile of the whole
 // Whole-horizon single launch: fp32 scoring with every (sample, obstacle) pair differentiated.  Always for
 // M <= 16 (same FLOPs as the per-step launches); for 17..32 obstacles only while the batch is latency-bound,
 // because differentiating all M pairs instead of the K closest costs up to 1.5x the FLOPs.
-bool use_whole_horizon(const dsmppi_ctx* c, int n) {
-  if (!c->fused_rollout || resolved_mode(c) != DSMPPI_PASS1_EXACT_FP32) return false;
+bool use_whole_horizon(const dsmppi_ctx* c, int n, int mode) {
+  if (!c->fused_rollout || mode != DSMPPI_PASS1_EXACT_FP32) return false;
   if (use_tc_scoring(c)) {
     // tensor-core scoring: a CTA pair holds 2 * (128 / M) samples for the whole horizon.  Worth it while one wave of
     // pairs covers the batch (the step then costs no launch); with more tiles per pair the per-step launches win,
@@ -72,12 +104,25 @@ int timing_mark(dsmppi_ctx* c, int kind, cudaStream_t st) {
   return 0;
 }
 
-}  // namespace
+// mean time of the start/stop event pairs the last call recorded
+int average_event_pairs(dsmppi_ctx* c, double* avg_ms, int* pairs) {
+  double tot = 0.0;
+  int n = 0;
+  for (int i = 0; i + 1 < c->ev_used; i += 2) {
+    CUDA_TRY(cudaEventSynchronize(c->ev[i + 1]));
+    float ms = 0.f;
+    CUDA_TRY(cudaEventElapsedTime(&ms, c->ev[i], c->ev[i + 1]));
+    tot += ms;
+    ++n;
+  }
+  *avg_ms = n ? tot / n : 0.0;
+  *pairs = n;
+  return 0;
+}
 
-int ensure_workspace(dsmppi_ctx* c, int n, int M) {
-  // The sizes below depend on the resolved pass-1 mode, and AUTO flips with the obstacle count (prefilter from 64
-  // obstacles on, dense fp32 scoring below): a workspace sized for one mode must not be taken for the other.
-  const int mode = resolved_mode(c);
+// The sizes below depend on the resolved pass-1 mode, and AUTO flips with the obstacle count (prefilter from 64
+// obstacles on, dense fp32 scoring below): a workspace sized for one mode must not be taken for the other.
+int ensure_workspace(dsmppi_ctx* c, int n, int M, int mode) {
   const size_t list_rows_now = cand_list_cap(c, n);
   if (n <= c->ws_n && M <= c->ws_M && mode == c->ws_mode && list_rows_now <= c->rowlist_cap) return 0;
   const int nn = n > c->ws_n ? n : c->ws_n;
@@ -110,8 +155,6 @@ int ensure_workspace(dsmppi_ctx* c, int n, int M) {
   c->ws_mode = mode;
   return 0;
 }
-
-namespace {
 
 // The caller's network (L hidden layers of width W) in the shipped 256 x 4 shape, the one storage format of every
 // weight image.  Missing features get zero weights and biases: their pre-activation is 0, ReLU keeps it 0, and they
@@ -382,6 +425,8 @@ int dsmppi_set_obstacles_host(dsmppi_ctx* c, const float* obs_host, int32_t M, v
   return dsmppi_set_obstacles(c, obs_host, M, stream);   // cudaMemcpyDefault handles host sources
 }
 
+}  // extern "C"
+
 // ---- guard band of the prefilter, calibrated per network ------------------------------------------------------
 // The tensor-core prefilter ranks obstacles on reduced-precision distances; every obstacle within `band` of the
 // K-th smallest is re-scored in fp32.  The band must exceed twice the prefilter's error, which depends on the
@@ -394,7 +439,7 @@ constexpr float CAL_SAFETY = 3.f;
 
 static int calibrate_band(dsmppi_ctx* c, const float* q, int q_stride, int n, uint32_t ignore_mask, int mode,
                           cudaStream_t st) {
-  const int slot = mode == DSMPPI_PASS1_TC_BF16 ? 1 : 0;
+  const int slot = band_slot(mode);
   const int d = c->d, M = c->M;
   const int n_act = n < CAL_Q ? n : CAL_Q;
   const int nq = CAL_Q + n_act;
@@ -411,7 +456,7 @@ static int calibrate_band(dsmppi_ctx* c, const float* q, int q_stride, int n, ui
   CUDA_TRY(cudaMemcpyAsync(dq, hq.data(), (size_t)CAL_Q * d * sizeof(float), cudaMemcpyHostToDevice, st));
   CUDA_TRY(cudaMemcpy2DAsync(dq + (size_t)CAL_Q * d, d * sizeof(float), q, (size_t)q_stride * sizeof(float),
                              d * sizeof(float), n_act, cudaMemcpyDeviceToDevice, st));
-  int rc = ensure_workspace(c, nq, M);
+  int rc = ensure_workspace(c, nq, M, mode);
   RowSrc src{};
   src.mode = ROWS_DENSE; src.M = M; src.n_rows = nq * M;
   if (!rc) rc = launch_exact_forward(c, dq, d, src, ignore_mask, ref, st);
@@ -433,24 +478,23 @@ static int calibrate_band(dsmppi_ctx* c, const float* q, int q_stride, int n, ui
   return 0;
 }
 
-// distance + gradient of n states q (row stride q_stride floats) against the current obstacles: fills
-// c->row_dist / c->row_grad and the ranked row indices c->sel_rows (n, K)
+// distance + gradient of n states q (row stride q_stride floats) against the current obstacles, scored in the
+// resolved pass-1 `mode`: fills c->row_dist / c->row_grad and the ranked row indices c->sel_rows (n, K)
 // table_ready / defer_rank: the rollout loop of the prefilter path hands the per-sample layer-1 table over from the
 // previous step and ranks inside its fused step launch (launch_rank_step)
-static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, int n, int K, uint32_t ignore_mask,
+static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, int n, int K, uint32_t ignore_mask, int mode,
                              cudaStream_t st, bool table_ready = false, bool defer_rank = false) {
   REQUIRE(c->M >= 1, "obstacles not set");
   REQUIRE(K >= 1 && K <= MAXK, "n_closest_obs out of range (1..8)");
   REQUIRE(K <= c->M, "n_closest_obs exceeds the number of obstacles");
-  const int mode = resolved_mode(c);
   if (mode != DSMPPI_PASS1_EXACT_FP32 && c->guard_band <= 0.f) {
-    const int slot = mode == DSMPPI_PASS1_TC_BF16 ? 1 : 0;
+    const int slot = band_slot(mode);
     if (c->band_cal[slot] <= 0.f || c->band_cal_M[slot] != c->M) {
       if (calibrate_band(c, q, q_stride, n, ignore_mask, mode, st)) return 1;
       table_ready = false;                 // the calibration wrote ITS states' table over the one handed in
     }
   }
-  if (ensure_workspace(c, n, c->M)) return 1;
+  if (ensure_workspace(c, n, c->M, mode)) return 1;
   RowSrc src{};
   src.M = c->M;
   src.K = K;
@@ -482,7 +526,7 @@ static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, int n,
   }
   // tensor-core prefilter -> candidate band -> one fp32 launch (ranking key + distance + gradient) -> rank
   c->prefilter_used = 1;
-  const float band = c->guard_band > 0.f ? c->guard_band : c->band_cal[mode == DSMPPI_PASS1_TC_BF16 ? 1 : 0];
+  const float band = c->guard_band > 0.f ? c->guard_band : c->band_cal[band_slot(mode)];
   const size_t cap_rows = cand_list_cap(c, n);
   if (timing_mark(c, 1, st)) return 1;
   if (tc_pass1(c, q, q_stride, n, ignore_mask, mode, st, table_ready)) return 1;
@@ -535,32 +579,35 @@ static int prefilter_verdict(dsmppi_ctx* c, int n_max, cudaStream_t st, int* ver
   return 0;
 }
 
-// one pass over the batch (in blocks of samples) with the context's current pass-1 mode and list budget
-static int rollout_once(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream_t st) {
+// The prefilter path is exact by construction: a call whose candidates did not all fit the row list is detected after
+// it ran (high-water mark, prefilter_verdict) and run again with a list that holds them -- or, past 2^27 rows or on
+// prefilter outputs beyond fp16, once more with every pair scored in fp32.  The repeat recomputes from the same inputs.
+// run(mode, attempt) does the work of one call in the resolved pass-1 `mode`; attempt is 0, 1, .. for the runs the
+// verdict checks and -1 for the fp32 fallback.
+template <typename Run>
+static int run_exact(dsmppi_ctx* c, int mode, int n_max, cudaStream_t st, Run&& run) {
+  for (int attempt = 0;; ++attempt) {
+    c->prefilter_used = 0;
+    CUDA_TRY(cudaMemsetAsync(c->counters + 8, 0, 2 * sizeof(int), st));
+    if (const int rc = run(mode, attempt)) return rc;
+    int verdict = 0, exact = 0;
+    if (const int rc = prefilter_verdict(c, n_max, st, &verdict, &exact)) return rc;
+    if (!verdict) return 0;
+    REQUIRE(attempt < 4, "candidate row list still too small after four attempts");
+    if (exact) return run(DSMPPI_PASS1_EXACT_FP32, -1);
+  }
+}
+
+// one pass over the batch (in blocks of samples) in the resolved pass-1 `mode` with the context's list budget
+static int rollout_once(dsmppi_ctx* c, const dsmppi_rollout_args* a, int mode, cudaStream_t st) {
   const int d = c->d;
-  // Samples never interact, so a very large batch is rolled out in blocks of samples: it bounds the workspace
-  // (the (n, M) prefilter matrix is the big one: <= 1 GiB) and keeps every row index inside 31 bits.
-  long long block = (1LL << 28) / c->M;
-  if (block > (1 << 18)) block = 1 << 18;
-  if (block < 1) block = 1;
+  const long long block = sample_block(c);
   for (long long off = 0; off < a->N; off += block) {
-    dsmppi_rollout_args b = *a;
-    b.N = (int)(a->N - off < block ? a->N - off : block);
-    if (a->q_cur_is_batch) b.q_cur_dev = a->q_cur_dev + off * d;
-    if (a->mu_tmp_dev) b.mu_tmp_dev = a->mu_tmp_dev + off * NKMAX * d;
-    if (a->sigma_tmp_dev) b.sigma_tmp_dev = a->sigma_tmp_dev + off * NKMAX;
-    if (a->alpha_tmp_dev) b.alpha_tmp_dev = a->alpha_tmp_dev + off * NKMAX * d;
-    b.all_traj_dev = a->all_traj_dev + off * a->H * d;
-    b.closest_dist_all_dev = a->closest_dist_all_dev + off * a->H;
-    b.kernel_val_all_dev = a->kernel_val_all_dev + off * a->H * NKMAX;
-    b.dot_products_dev = a->dot_products_dev + off * a->H;
-    b.kernel_activations_dev = a->kernel_activations_dev + off * a->H;
-    b.qdot_dev = a->qdot_dev + off * d;
-    b.nn_grad_all_dev = a->nn_grad_all_dev + off * a->H * d;
+    dsmppi_rollout_args b = slice_samples(*a, d, off, (int)(a->N - off < block ? a->N - off : block));
     if (launch_init_traj(c, &b, st)) return 1;
     if (a->distance_provider == DSMPPI_DISTANCE_FK) {
       // true-distance provider: FK + sphere distances write one (distance, gradient) row per sample, K = 1
-      if (ensure_workspace(c, b.N, c->M)) return 1;
+      if (ensure_workspace(c, b.N, c->M, mode)) return 1;
       if (launch_identity_rows(c, b.N, 1, st)) return 1;
       b.n_closest = 1;
       for (int t = 1; t <= b.H; ++t) {
@@ -571,17 +618,16 @@ static int rollout_once(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream_
       }
       continue;
     }
-    if (use_whole_horizon(c, b.N)) {
+    if (use_whole_horizon(c, b.N, mode)) {
       REQUIRE(b.n_closest >= 1 && b.n_closest <= MAXK, "n_closest_obs out of range (1..8)");
       REQUIRE(b.n_closest <= c->M, "n_closest_obs exceeds the number of obstacles");
-      if (ensure_workspace(c, b.N, c->M)) return 1;
+      if (ensure_workspace(c, b.N, c->M, mode)) return 1;
       const bool tcx = use_tc_scoring(c);
       if (timing_mark(c, tcx ? 4 : 2, st)) return 1;
       if (tcx ? launch_tc_rollout(c, &b, st) : launch_rollout_fused(c, &b, st)) return 1;
       if (timing_mark(c, tcx ? 4 : 2, st)) return 1;
       continue;
     }
-    const int mode = resolved_mode(c);
     if (mode != DSMPPI_PASS1_EXACT_FP32) {
       // prefilter path, four launches per step: tc_pass1 (all-pairs prefilter) -> select_candidates (guard band) ->
       // tc_exact / exact_mlp (fp32 scoring + VJP of the band; + its normally empty FFMA range fix-up) -> rank_step
@@ -589,19 +635,15 @@ static int rollout_once(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream_
       if (tc_reserve_sample_table(c, b.N)) return 1;
       for (int t = 1; t <= b.H; ++t) {
         const float* q = b.all_traj_dev + (size_t)(t - 1) * d;        // q_prev = all_traj[:, t-1, :]
-        // (the first call may calibrate the guard band, which runs the prefilter on other states: no table hand-over)
-        const bool handed = t > 1 && c->table_valid;
-        c->table_valid = 0;
-        if (distance_pipeline(c, q, b.H * d, b.N, b.n_closest, b.ignored_link_mask, st, handed, true)) return 1;
+        // from step 2 on, the previous step's rank_step launch wrote the layer-1 table of these states
+        if (distance_pipeline(c, q, b.H * d, b.N, b.n_closest, b.ignored_link_mask, mode, st, t > 1, true)) return 1;
         if (launch_rank_step(c, &b, t, mode, st)) return 1;
-        c->table_valid = 1;
       }
-      c->table_valid = 0;
       continue;
     }
     for (int t = 1; t <= b.H; ++t) {
       const float* q = b.all_traj_dev + (size_t)(t - 1) * d;          // q_prev = all_traj[:, t-1, :]
-      if (distance_pipeline(c, q, b.H * d, b.N, b.n_closest, b.ignored_link_mask, st)) return 1;
+      if (distance_pipeline(c, q, b.H * d, b.N, b.n_closest, b.ignored_link_mask, mode, st)) return 1;
       if (launch_step(c, &b, t, st)) return 1;
     }
   }
@@ -609,6 +651,8 @@ static int rollout_once(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream_
     if (launch_basis(c, a->nn_grad_all_dev, (int64_t)a->N * a->H, a->norm_basis_dev, st)) return 1;
   return 0;
 }
+
+extern "C" {
 
 int dsmppi_rollout(dsmppi_ctx* c, const dsmppi_rollout_args* a, void* stream) {
   REQUIRE(c && a, "null argument");
@@ -632,32 +676,17 @@ int dsmppi_rollout(dsmppi_ctx* c, const dsmppi_rollout_args* a, void* stream) {
   REQUIRE(c->M >= 1, "obstacles not set");
   if (!c->keep_counters) c->ev_used = 0;
   const int ev_start = c->ev_used;
-  long long block = (1LL << 28) / c->M;
-  if (block > (1 << 18)) block = 1 << 18;
-  const int n_max = (int)(a->N < block ? a->N : (block < 1 ? 1 : block));
-  // The prefilter path is exact by construction: a step whose candidates did not all fit the row list is detected
-  // after the rollout (high-water mark, prefilter_verdict) and the rollout is run again with a list that holds them
-  // -- or, past 2^27 rows, with every pair scored in fp32.  The repeat recomputes from the same inputs.
-  for (int attempt = 0;; ++attempt) {
+  const long long block = sample_block(c);
+  const int n_max = (int)(a->N < block ? a->N : block);
+  // The whole call is repeated.  Counters 1..3 restart with each run the verdict checks, except that the first run
+  // of a chunk of a chunked iteration adds to the earlier chunks' counts; the fp32 fallback keeps the counts of the
+  // run it replaces.
+  return run_exact(c, resolve_mode(c, c->pass1_mode, c->M), n_max, st, [&](int mode, int attempt) {
     c->ev_used = ev_start;
-    c->prefilter_used = 0;
-    if (!c->keep_counters || attempt > 0) CUDA_TRY(cudaMemsetAsync(c->counters + 1, 0, 3 * sizeof(int), st));
-    CUDA_TRY(cudaMemsetAsync(c->counters + 8, 0, 2 * sizeof(int), st));
-    if (rollout_once(c, a, st)) return 1;
-    int verdict = 0, exact = 0;
-    if (prefilter_verdict(c, n_max, st, &verdict, &exact)) return 1;
-    if (!verdict) break;
-    REQUIRE(attempt < 4, "candidate row list still too small after four attempts");
-    if (exact) {
-      const int saved = c->pass1_mode;
-      c->pass1_mode = DSMPPI_PASS1_EXACT_FP32;
-      c->ev_used = ev_start;
-      const int rc = rollout_once(c, a, st);
-      c->pass1_mode = saved;
-      return rc;
-    }
-  }
-  return 0;
+    if (attempt > 0 || (attempt == 0 && !c->keep_counters))
+      CUDA_TRY(cudaMemsetAsync(c->counters + 1, 0, 3 * sizeof(int), st));
+    return rollout_once(c, a, mode, st);
+  });
 }
 
 int dsmppi_distance_grad(dsmppi_ctx* c, const float* q_dev, int32_t n, int32_t n_closest, uint32_t ignored_link_mask,
@@ -667,25 +696,16 @@ int dsmppi_distance_grad(dsmppi_ctx* c, const float* q_dev, int32_t n, int32_t n
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_TRY(cudaSetDevice(c->device));
   REQUIRE(c->M >= 1, "obstacles not set");
-  long long block = (1LL << 28) / c->M;
-  if (block > (1 << 18)) block = 1 << 18;
-  if (block < 1) block = 1;
-  const int saved_mode = c->pass1_mode;
+  const long long block = sample_block(c);
+  const int mode = resolve_mode(c, c->pass1_mode, c->M);
   for (long long off = 0; off < n; off += block) {
     const int nb = (int)(n - off < block ? n - off : block);
-    for (int attempt = 0;; ++attempt) {                 // same exactness protocol as dsmppi_rollout, per block
-      c->prefilter_used = 0;
-      CUDA_TRY(cudaMemsetAsync(c->counters + 8, 0, 2 * sizeof(int), st));
-      int rc = distance_pipeline(c, q_dev + off * c->d, c->d, nb, n_closest, ignored_link_mask, st);
-      if (!rc) rc = launch_blend(c, nb, n_closest, distance_dev + off, nn_grad_dev + off * c->d, st);
-      int verdict = 0, exact = 0;
-      if (!rc) rc = prefilter_verdict(c, nb, st, &verdict, &exact);
-      if (rc) { c->pass1_mode = saved_mode; return rc; }
-      if (!verdict) break;
-      if (attempt >= 4) { c->pass1_mode = saved_mode; REQUIRE(false, "candidate row list still too small"); }
-      if (exact) c->pass1_mode = DSMPPI_PASS1_EXACT_FP32;
-    }
-    c->pass1_mode = saved_mode;
+    // each block is repeated on its own
+    const int rc = run_exact(c, mode, nb, st, [&](int m, int) {
+      const int r = distance_pipeline(c, q_dev + off * c->d, c->d, nb, n_closest, ignored_link_mask, m, st);
+      return r ? r : launch_blend(c, nb, n_closest, distance_dev + off, nn_grad_dev + off * c->d, st);
+    });
+    if (rc) return rc;
   }
   return 0;
 }
@@ -704,14 +724,12 @@ int dsmppi_distance_grad_fk(dsmppi_ctx* c, const float* q_dev, int32_t n, int32_
 int dsmppi_debug_pass1(dsmppi_ctx* c, const float* q_dev, int32_t n, uint32_t ignored_link_mask, int32_t mode,
                        float* out_dev, void* stream) {
   REQUIRE(c && q_dev && out_dev, "null argument");
+  REQUIRE(mode >= DSMPPI_PASS1_EXACT_FP32 && mode <= DSMPPI_PASS1_TC_BF16,
+          "bad pass-1 mode (EXACT_FP32, TC_F16 or TC_BF16; AUTO is not a kernel)");
   REQUIRE(c->M >= 1, "obstacles not set");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_TRY(cudaSetDevice(c->device));
-  const int saved = c->pass1_mode;
-  c->pass1_mode = mode;
-  const int rc = ensure_workspace(c, n, c->M);
-  c->pass1_mode = saved;
-  if (rc) return rc;
+  if (ensure_workspace(c, n, c->M, resolve_mode(c, mode, c->M))) return 1;
   const size_t bytes = (size_t)n * c->M * sizeof(float);
   if (mode == DSMPPI_PASS1_EXACT_FP32) {
     RowSrc src{};
@@ -871,15 +889,7 @@ int dsmppi_iteration_host(dsmppi_ctx* c, dsmppi_iteration_host_args* h, void* st
       }
       CUDA_TRY(cudaEventRecord(ev_in, c->s_in));
       CUDA_TRY(cudaStreamWaitEvent(st, ev_in, 0));
-      dsmppi_rollout_args b = a;
-      b.N = (int)n;
-      if (r.q_cur_is_batch) b.q_cur_dev = a.q_cur_dev + o * d;
-      b.mu_tmp_dev = a.mu_tmp_dev + o * NKMAX * d; b.sigma_tmp_dev = a.sigma_tmp_dev + o * NKMAX;
-      b.alpha_tmp_dev = a.alpha_tmp_dev + o * NKMAX * d;
-      b.all_traj_dev = a.all_traj_dev + o * H * d; b.closest_dist_all_dev = a.closest_dist_all_dev + o * H;
-      b.kernel_val_all_dev = a.kernel_val_all_dev + o * H * NKMAX; b.dot_products_dev = a.dot_products_dev + o * H;
-      b.kernel_activations_dev = a.kernel_activations_dev + o * H; b.qdot_dev = a.qdot_dev + o * d;
-      b.nn_grad_all_dev = a.nn_grad_all_dev + o * H * d;
+      const dsmppi_rollout_args b = slice_samples(a, c->d, (long long)o, (int)n);
       rc = dsmppi_rollout(c, &b, stream);
       if (rc) break;
       dsmppi_cost_args cb = ca;
@@ -969,15 +979,14 @@ int dsmppi_pass1_stats(dsmppi_ctx* c, int64_t* rescored_pairs, int64_t* band_ove
     std::memcpy(&v, &host[2], sizeof(v));
     *rescored_pairs = (int64_t)v;
   }
-  if (mode) *mode = resolved_mode(c);
+  if (mode) *mode = resolve_mode(c, c->pass1_mode, c->M);
   return 0;
 }
 
 int dsmppi_exactness_stats(dsmppi_ctx* c, int64_t* capacity_retries, int64_t* exact_fallbacks, float* guard_band,
                            float* calibration_error) {
   REQUIRE(c, "null ctx");
-  const int mode = resolved_mode(c);
-  const int slot = mode == DSMPPI_PASS1_TC_BF16 ? 1 : 0;
+  const int slot = band_slot(resolve_mode(c, c->pass1_mode, c->M));
   if (capacity_retries) *capacity_retries = c->capacity_retries;
   if (exact_fallbacks) *exact_fallbacks = c->exact_fallbacks;
   if (guard_band) *guard_band = c->guard_band > 0.f ? c->guard_band : c->band_cal[slot];
@@ -1005,33 +1014,20 @@ int dsmppi_enable_kernel_timing(dsmppi_ctx* c, int32_t on) {
 
 int dsmppi_kernel_timing_ex(dsmppi_ctx* c, int32_t* kind, double* ms_per_launch, int32_t* launches) {
   REQUIRE(c, "null ctx");
-  double tot = 0.0;
-  int n = 0;
-  for (int i = 0; i + 1 < c->ev_used; i += 2) {
-    CUDA_TRY(cudaEventSynchronize(c->ev[i + 1]));
-    float ms = 0.f;
-    CUDA_TRY(cudaEventElapsedTime(&ms, c->ev[i], c->ev[i + 1]));
-    tot += ms;
-    ++n;
-  }
+  double avg;
+  int n;
+  if (average_event_pairs(c, &avg, &n)) return 1;
   if (kind) *kind = c->ev_kind;
-  if (ms_per_launch) *ms_per_launch = n ? tot / n : 0.0;
+  if (ms_per_launch) *ms_per_launch = avg;
   if (launches) *launches = n;
   return 0;
 }
 
 int dsmppi_kernel_timing(dsmppi_ctx* c, double* pass1_ms, int32_t* pass1_n, double* exact_ms, int32_t* exact_n) {
   REQUIRE(c, "null ctx");
-  double tot = 0.0;
-  int n = 0;
-  for (int i = 0; i + 1 < c->ev_used; i += 2) {
-    CUDA_TRY(cudaEventSynchronize(c->ev[i + 1]));
-    float ms = 0.f;
-    CUDA_TRY(cudaEventElapsedTime(&ms, c->ev[i], c->ev[i + 1]));
-    tot += ms;
-    ++n;
-  }
-  const double avg = n ? tot / n : 0.0;
+  double avg;
+  int n;
+  if (average_event_pairs(c, &avg, &n)) return 1;
   if (pass1_ms) *pass1_ms = c->ev_kind == 1 ? avg : 0.0;
   if (pass1_n) *pass1_n = c->ev_kind == 1 ? n : 0;
   if (exact_ms) *exact_ms = c->ev_kind == 0 ? avg : 0.0;
@@ -1086,13 +1082,9 @@ extern "C" int dsmppi_tick(dsmppi_ctx* c, dsmppi_tick_args* t, void* stream) {
   REQUIRE(r.mod.ds_kind != DSMPPI_DS_SEDS && r.distance_provider == DSMPPI_DISTANCE_NN,
           "the graphed tick covers the linear / matrix nominal DS with the network distance");
   CUDA_TRY(cudaSetDevice(c->device));
-  {   // the prefilter path cannot be captured (it ends with a host-side verdict)
-    const int saved = c->M;
-    c->M = t->n_obs;
-    const int mode = resolved_mode(c);
-    c->M = saved;
-    REQUIRE(mode == DSMPPI_PASS1_EXACT_FP32, "the graphed tick needs the dense fp32 scoring path (few obstacles)");
-  }
+  // the prefilter path cannot be captured (it ends with a host-side verdict)
+  REQUIRE(resolve_mode(c, c->pass1_mode, t->n_obs) == DSMPPI_PASS1_EXACT_FP32,
+          "the graphed tick needs the dense fp32 scoring path (few obstacles)");
   REQUIRE(!c->timing, "kernel timing events cannot be recorded into a graph");
   cudaStream_t caller = static_cast<cudaStream_t>(stream);
   if (!c->s_tick) {

@@ -103,7 +103,6 @@ struct dsmppi_ctx {
   int obs_tables_dirty = 1;           // c->obs changed since tc_set_obstacles built the per-obstacle layer-1 table
   int pass1_hacc = 1;                 // fp16 prefilter: hidden layers accumulate in fp16 (DSMPPI_PASS1_ACC=f32: in fp32)
   int half_tiles = 1;                 // whole-horizon tensor-core rollout: 64-row tiles while one wave covers the batch
-  int table_valid = 0;                // c->enc_q holds the layer-1 table of the states the next prefilter launch scores
   int prefilter_used = 0;             // set by distance_pipeline when a call went through the tensor-core prefilter
   int64_t capacity_retries = 0;       // rollouts that were run again with a larger candidate row list
   int64_t exact_fallbacks = 0;        // rollouts that were run again with every pair scored in fp32
@@ -219,4 +218,3 @@ int launch_update_partial(dsmppi_ctx* c, const dsmppi_update_args* a, const floa
 int launch_update_finalize(dsmppi_ctx* c, const dsmppi_update_args* a, const float* packed, int* n_updated,
                            cudaStream_t st);
 int launch_kernel_candidates(dsmppi_ctx* c, const dsmppi_candidates_args* a, cudaStream_t st);
-int ensure_workspace(dsmppi_ctx* c, int n, int M);

@@ -271,10 +271,13 @@ def test_prefilter_variants_are_bitwise_the_all_pairs_rollout(factory, variant, 
         assert torch.equal(a, b)
 
 
-def test_prefilter_overflow_falls_back_to_all_pairs_fp32(factory):
+@pytest.mark.parametrize("n_obs", [294, 24], ids=["shelf", "shelf_first24"])
+def test_prefilter_overflow_falls_back_to_all_pairs_fp32(factory, n_obs):
     """A network whose hidden activations leave the fp16 range (layer 3 scaled by 1e5, layer 4 by 1e-5: the fp32
     function is an ordinary one) makes the prefilter's fp16 accumulators overflow.  The kernel reports the inf / NaN
-    outputs, the call is repeated with every pair scored in fp32, and the result is bitwise the all-pairs one."""
+    outputs, the call is repeated with every pair scored in fp32, and the result is bitwise the all-pairs one -- for
+    the rollout and for distance_repulsion_nn.  With 24 obstacles the fp32 repeat is the whole-horizon kernel.  The
+    caller's mode outlives the fallback: it is still the one reported, and the next call falls back again."""
     import optimalmodulationds_b200 as pkg
     from optimalmodulationds_b200.sdf.robot_sdf import RobotSdfCollisionNet
     c = load_npz("case_franka_shelf")
@@ -291,22 +294,58 @@ def test_prefilter_overflow_falls_back_to_all_pairs_fp32(factory):
     t = lambda x: x.cuda()  # noqa: E731
     N, H = 64, 2
     q_cur = c["q0"] + 0.2 * torch.randn(N, 7)
-    res, xs = {}, {}
+    res, xs, nn = {}, {}, {}
     for mode in ("exact", "tc_f16"):
         DS = [pkg.LinDS(t(c["qf"])), pkg.LinDS(t(c["q0"]))]
-        m = pkg.MPPI(t(c["q0"]), t(c["qf"]), t(c["dh_params"]), t(c["obs"]), float(c["dt"]), H, N, DS, t(c["dh_a"]),
-                     net, 5)
+        m = pkg.MPPI(t(c["q0"]), t(c["qf"]), t(c["dh_params"]), t(c["obs"][:n_obs]), float(c["dt"]), H, N, DS,
+                     t(c["dh_a"]), net, 5)
         m.set_pass1_mode(mode)
         m.dst_thr, m.ignored_links = 0.01, [0, 1, 2]
         m.q_cur = t(q_cur)
-        before = m.exactness_stats()["exact_fallbacks"]
+        fallbacks = [m.exactness_stats()["exact_fallbacks"]]
         res[mode] = _rollout_outputs(m)
-        xs[mode] = m.exactness_stats()["exact_fallbacks"] - before
-    print(f"exact fallbacks: {xs}")
-    assert xs["tc_f16"] >= 1 and xs["exact"] == 0
+        fallbacks.append(m.exactness_stats()["exact_fallbacks"])
+        assert m.pass1_stats()["mode"] == (1 if mode == "tc_f16" else 0)
+        again = _rollout_outputs(m)
+        fallbacks.append(m.exactness_stats()["exact_fallbacks"])
+        for a, b, name in zip(res[mode], again, ("traj", "dist", "kval", "dots", "acts", "qdot")):
+            assert torch.equal(a, b), f"{mode}: {name} differs between two calls"
+        nn[mode] = [x.clone() for x in m.distance_repulsion_nn(t(q_cur))]
+        fallbacks.append(m.exactness_stats()["exact_fallbacks"])
+        xs[mode] = [b - a for a, b in zip(fallbacks, fallbacks[1:])]
+    print(f"exact fallbacks per call (rollout, rollout, distance_repulsion_nn): {xs}")
+    assert all(x >= 1 for x in xs["tc_f16"]) and xs["exact"] == [0, 0, 0]
     for a, b, name in zip(res["exact"], res["tc_f16"], ("traj", "dist", "kval", "dots", "acts", "qdot")):
         assert torch.isfinite(a).all(), name
         assert torch.equal(a, b), f"overflowing net: {name} differs from the all-pairs fp32 rollout"
+    for a, b, name in zip(nn["exact"], nn["tc_f16"], ("distance", "gradient")):
+        assert torch.isfinite(a).all(), name
+        assert torch.equal(a, b), f"overflowing net: distance_repulsion_nn {name} differs from the all-pairs fp32 one"
+
+
+def test_debug_pass1_refuses_a_mode_without_a_kernel(factory):
+    """dsmppi_debug_pass1 runs the fp32 scoring or one of the two prefilters; AUTO (3) and unknown values return 2
+    and leave the object as it was: its next rollout equals a fresh object's bit for bit."""
+    c = load_npz("case_franka_shelf")
+    torch.manual_seed(13)
+    N, H = 64, 2
+    q_cur = c["q0"] + 0.2 * torch.randn(N, 7)
+    objs = [factory.make_mppi(c, device="cuda", N=N, H=H, q_cur=q_cur, pass1="auto", copy_policy=False)
+            for _ in range(2)]
+    for m in objs:
+        torch.manual_seed(11)
+        m.Policy.sample_policy()
+    m, fresh = objs
+    with torch.cuda.device(m._dev):
+        m._upload_obstacles()
+        q = q_cur.cuda()
+        out = torch.empty(N, c["obs"].shape[0], device="cuda")
+        for mode in (3, 7):
+            rc = m._lib.dsmppi_debug_pass1(m._ctx, q.data_ptr(), N, m._ignore_mask(), mode, out.data_ptr(), m._stream())
+            assert rc == 2 and b"bad pass-1 mode" in m._lib.dsmppi_last_error(), mode
+    got, want = _rollout_outputs(m), _rollout_outputs(fresh)
+    for a, b, name in zip(got, want, ("traj", "dist", "kval", "dots", "acts", "qdot")):
+        assert torch.equal(a, b), f"{name} differs from a fresh object's after refused debug_pass1 calls"
 
 
 def test_profiler_sees_the_reference_stage_tags(factory, score_mode):
