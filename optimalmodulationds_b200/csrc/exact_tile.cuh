@@ -19,21 +19,6 @@ constexpr int XS = 12;    // padded row stride of the raw-input scratch (nin <= 
 constexpr int WS = 8;     // k-rows of weights per pipeline stage (8 KB at WID = 256)
 constexpr int NSTAGE = 4; // ring depth
 
-__device__ __forceinline__ bool row_lookup(const RowSrc& s, int r, int n_rows, int& i, int& j) {
-  if (r >= n_rows) return false;
-  if (s.mode == ROWS_DENSE) {
-    i = r / s.M;
-    j = r - i * s.M;
-  } else if (s.mode == ROWS_SELECTED) {
-    i = r / s.K;
-    j = s.sel[r];
-  } else {
-    i = s.row_sample[r];
-    j = s.row_obs[r];
-  }
-  return true;
-}
-
 // Thread tile: rows r0 .. r0+RPT-1 and FT features: FT = 8: {fa .. fa+3} (j = 0..3) and {fa+32 .. fa+35} (j = 4..7);
 // FT = 4 / 2: {fa .. fa+FT-1}.
 template <int FT>
@@ -83,20 +68,34 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-// Packed fp32 FMA (Blackwell fma.rn.f32x2): two IEEE fused multiply-adds per issue slot, bit-identical to two
-// fmaf().  The inner loop is issue-bound with scalar FFMAs (ncu: issue 68 %, fma pipe 51 %), so halving the FFMA
-// issue count is what lets the pipe fill.
-__device__ __forceinline__ uint64_t pack2f(float lo, float hi) {
+// Packed fp32 pairs (Blackwell fma.rn.f32x2 / add / mul .f32x2): two IEEE operations per issue slot, bit-identical to
+// the scalar forms.  The inner loop of the tile below is issue-bound with scalar FFMAs (ncu: issue 68 %, fma pipe 51 %),
+// and so is the epilogue of tc_exact.cu; halving their fp32 instruction count is what lets the pipe fill.
+__device__ __forceinline__ uint64_t pk2(uint32_t lo, uint32_t hi) {
   uint64_t r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
+  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "r"(lo), "r"(hi));
   return r;
 }
-__device__ __forceinline__ void unpack2f(uint64_t v, float& lo, float& hi) {
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
+__device__ __forceinline__ uint64_t pk2f(float lo, float hi) { return pk2(__float_as_uint(lo), __float_as_uint(hi)); }
+__device__ __forceinline__ void unpk2(uint64_t v, float& lo, float& hi) {
+  uint32_t a, b;
+  asm("mov.b64 {%0, %1}, %2;" : "=r"(a), "=r"(b) : "l"(v));
+  lo = __uint_as_float(a);
+  hi = __uint_as_float(b);
 }
 __device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
   uint64_t d;
   asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
+  return d;
+}
+__device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
+  uint64_t d;
+  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
+  return d;
+}
+__device__ __forceinline__ uint64_t mul2(uint64_t a, uint64_t b) {
+  uint64_t d;
+  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
   return d;
 }
 
@@ -166,10 +165,10 @@ __device__ __forceinline__ void gemm_tile(WeightStream<WID>& ws, int& stage, int
         load_feats<FT>(wb + kk * WID, w);
         uint64_t wp[FT / 2];
 #pragma unroll
-        for (int p = 0; p < FT / 2; ++p) wp[p] = pack2f(w[2 * p], w[2 * p + 1]);
+        for (int p = 0; p < FT / 2; ++p) wp[p] = pk2f(w[2 * p], w[2 * p + 1]);
 #pragma unroll
         for (int i = 0; i < RPT; ++i) {
-          const uint64_t ad = pack2f(a[i], a[i]);
+          const uint64_t ad = pk2f(a[i], a[i]);
 #pragma unroll
           for (int p = 0; p < FT / 2; ++p) acc2[i][p] = fma2(ad, wp[p], acc2[i][p]);
         }
@@ -181,10 +180,10 @@ __device__ __forceinline__ void gemm_tile(WeightStream<WID>& ws, int& stage, int
         load_feats<FT>(wb + kk * WID, w);
         uint64_t wp[FT / 2];
 #pragma unroll
-        for (int p = 0; p < FT / 2; ++p) wp[p] = pack2f(w[2 * p], w[2 * p + 1]);
+        for (int p = 0; p < FT / 2; ++p) wp[p] = pk2f(w[2 * p], w[2 * p + 1]);
 #pragma unroll
         for (int i = 0; i < RPT; ++i) {
-          const uint64_t ad = pack2f(a[i], a[i]);
+          const uint64_t ad = pk2f(a[i], a[i]);
 #pragma unroll
           for (int p = 0; p < FT / 2; ++p) acc2[i][p] = fma2(ad, wp[p], acc2[i][p]);
         }
@@ -194,7 +193,7 @@ __device__ __forceinline__ void gemm_tile(WeightStream<WID>& ws, int& stage, int
 #pragma unroll
   for (int i = 0; i < RPT; ++i)
 #pragma unroll
-    for (int p = 0; p < FT / 2; ++p) unpack2f(acc2[i][p], acc[i][2 * p], acc[i][2 * p + 1]);
+    for (int p = 0; p < FT / 2; ++p) unpk2(acc2[i][p], acc[i][2 * p], acc[i][2 * p + 1]);
 }
 
 template <int RPT, int FT>

@@ -66,6 +66,20 @@ struct RowSrc {
   const int* row_obs;     // ROWS_LIST
   const int* out_row;     // optional: row r writes its outputs at index out_row[r] (re-scoring of flagged rows)
 };
+__device__ __forceinline__ bool row_lookup(const RowSrc& s, int r, int n_rows, int& i, int& j) {
+  if (r >= n_rows) return false;
+  if (s.mode == ROWS_DENSE) {
+    i = r / s.M;
+    j = r - i * s.M;
+  } else if (s.mode == ROWS_SELECTED) {
+    i = r / s.K;
+    j = s.sel[r];
+  } else {
+    i = s.row_sample[r];
+    j = s.row_obs[r];
+  }
+  return true;
+}
 
 struct DhTable { float v[MAXD + 1][4]; };   // rows [d, theta, a, alpha]
 

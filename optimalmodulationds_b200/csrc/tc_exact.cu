@@ -72,6 +72,7 @@
 
 namespace {
 using namespace tcx;
+using exact_tile::pk2, exact_tile::pk2f, exact_tile::unpk2, exact_tile::fma2, exact_tile::add2, exact_tile::mul2;
 
 constexpr int TROWS = 128;                 // rows per CTA per tile
 constexpr int W_MMA = 8, W_LOAD = 9;
@@ -105,35 +106,6 @@ __device__ __forceinline__ float combine(uint32_t d1, uint32_t d2, float comp) {
 
 __device__ __forceinline__ uint32_t pack_h2(float lo, float hi);
 __device__ __forceinline__ float2 unpack_h2(uint32_t p);
-// packed fp32 pairs (Blackwell fma.rn.f32x2 / add / mul .f32x2): two IEEE operations per issue slot, bit-identical to
-// the scalar forms -- the epilogue is issue-bound, so halving its fp32 instruction count is what shortens it
-__device__ __forceinline__ uint64_t pk2(uint32_t lo, uint32_t hi) {
-  uint64_t r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "r"(lo), "r"(hi));
-  return r;
-}
-__device__ __forceinline__ uint64_t pk2f(float lo, float hi) { return pk2(__float_as_uint(lo), __float_as_uint(hi)); }
-__device__ __forceinline__ void unpk2(uint64_t v, float& lo, float& hi) {
-  uint32_t a, b;
-  asm("mov.b64 {%0, %1}, %2;" : "=r"(a), "=r"(b) : "l"(v));
-  lo = __uint_as_float(a);
-  hi = __uint_as_float(b);
-}
-__device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
-  uint64_t d;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
-  return d;
-}
-__device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
-__device__ __forceinline__ uint64_t mul2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
 // D1 + D2 * 2^-11 + D1 * comp for two adjacent columns
 __device__ __forceinline__ uint64_t combine2(uint32_t d1a, uint32_t d1b, uint32_t d2a, uint32_t d2b, float comp) {
   const uint64_t a = pk2(d1a, d1b);
@@ -237,21 +209,6 @@ struct TxArgs {
 #else
 #define TCX_PROF(region, id) do { } while (0)
 #endif
-
-__device__ __forceinline__ bool row_lookup(const RowSrc& s, int r, int n_rows, int& i, int& j) {
-  if (r >= n_rows) return false;
-  if (s.mode == ROWS_DENSE) {
-    i = r / s.M;
-    j = r - i * s.M;
-  } else if (s.mode == ROWS_SELECTED) {
-    i = r / s.K;
-    j = s.sel[r];
-  } else {
-    i = s.row_sample[r];
-    j = s.row_obs[r];
-  }
-  return true;
-}
 
 __device__ __forceinline__ uint32_t pack_h2(float lo, float hi) {
   uint32_t r;
@@ -1143,7 +1100,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
       }
   } else if (warp == W_MMA) {
     // =================================== MMA issuer (leader CTA) ===================================
-    constexpr uint32_t idesc128 = make_idesc_f16(HM ? 128 : 256, 128), idesc32 = make_idesc_f16(HM ? 128 : 256, 32);
+    constexpr uint32_t idesc128 = make_idesc(0, HM ? 128 : 256, 128), idesc32 = make_idesc(0, HM ? 128 : 256, 32);
     const uint32_t a_hi = sbase + OFF_AHI, a_lo = sbase + OFF_ALO;
     uint32_t slot = 0, par = 0;                               // ring position of the next weight stage
     uint32_t acount[4] = {0, 0, 0, 0};                        // phases consumed of the four operand-quarter barriers
@@ -1257,22 +1214,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
     __syncwarp();
     tmem_free_512_2cta(tmem_base);
   }
-}
-
-uint16_t f2h(float f) {
-  __half h = __float2half_rn(f);
-  uint16_t u;
-  std::memcpy(&u, &h, 2);
-  return u;
-}
-float h2f(uint16_t u) {
-  __half h;
-  std::memcpy(&h, &u, 2);
-  return __half2float(h);
-}
-// canonical K-major no-swizzle placement of element (n, k) inside a slab of `rows` rows (see tc_ptx.cuh make_desc)
-inline size_t canon(int n, int k, int rows) {
-  return (size_t)(k / 8) * rows * 16 + (size_t)n * 16 + (size_t)(k % 8) * 2;
 }
 
 // Per-GEMM compensation of the network in hand.  Layer 1 keeps c(2) (K = 3(d+P) <= 32 whatever the width); for the

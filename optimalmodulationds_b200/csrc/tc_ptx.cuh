@@ -1,7 +1,12 @@
-// PTX wrappers shared by the tcgen05 kernels that stream their operands through shared memory (tc_exact.cu):
-// mbarriers, bulk (TMA) copies, TMEM allocation / loads, UMMA descriptors and the cta_group::2 MMA forms.
+// PTX wrappers shared by the tcgen05 kernels (the prefilter tc_pass1.cu and the scoring kernel tc_exact.cu): mbarriers,
+// bulk (TMA) copies, TMEM allocation / loads / stores, UMMA descriptors and the cta_group::2 MMA forms, plus the host
+// helpers that lay out their fp16 weight images.
 #pragma once
+#include <cuda_fp16.h>
 #include <stdint.h>
+
+#include <cstring>
+#include <utility>
 
 namespace tcx {
 
@@ -16,6 +21,9 @@ __device__ __forceinline__ void cluster_sync_all() {
 }
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
+}
+__device__ __forceinline__ void mbar_arrive_local(uint32_t bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
@@ -47,7 +55,7 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   if (mbar_try_wait(bar, parity)) return;
   const long long t0 = clock64();
   while (!mbar_try_wait(bar, parity)) {
-    if (clock64() - t0 > 2000000000LL) __trap();
+    if (clock64() - t0 > 4000000000LL) __trap();
   }
 }
 // acquire at cluster scope: the waiter goes on to hand shared memory written by the PEER CTA to the tensor core
@@ -87,6 +95,7 @@ __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.p
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tc_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 __device__ __forceinline__ void tmem_alloc_512_2cta(uint32_t dst_smem) {
   asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(dst_smem) : "memory");
@@ -114,6 +123,16 @@ __device__ __forceinline__ void mma_ss_2cta(uint32_t d_tmem, uint64_t a_desc, ui
       "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[tmem] * B[smem]^T, M = 256 over the CTA pair, issued by one thread of the leader CTA
+__device__ __forceinline__ void mma_ts_2cta(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc,
+                                            uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(d_tmem),
+      "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // completion of all MMAs issued so far by this thread -> arrive on the barrier at this offset in BOTH CTAs
 __device__ __forceinline__ void mma_commit_2cta(uint32_t bar) {
   asm volatile(
@@ -122,21 +141,40 @@ __device__ __forceinline__ void mma_commit_2cta(uint32_t bar) {
       : "memory");
 }
 
-#define TCX_R8(v, o) "=r"(v[o + 0]), "=r"(v[o + 1]), "=r"(v[o + 2]), "=r"(v[o + 3]), "=r"(v[o + 4]), "=r"(v[o + 5]), "=r"(v[o + 6]), "=r"(v[o + 7])
+#define R8(v, o) "=r"(v[o + 0]), "=r"(v[o + 1]), "=r"(v[o + 2]), "=r"(v[o + 3]), "=r"(v[o + 4]), "=r"(v[o + 5]), "=r"(v[o + 6]), "=r"(v[o + 7])
+#define W8(v, o) "r"(v[o + 0]), "r"(v[o + 1]), "r"(v[o + 2]), "r"(v[o + 3]), "r"(v[o + 4]), "r"(v[o + 5]), "r"(v[o + 6]), "r"(v[o + 7])
 // 32 / 16 consecutive accumulator columns of this thread's TMEM lane
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
       "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : TCX_R8(v, 0), TCX_R8(v, 8), TCX_R8(v, 16), TCX_R8(v, 24)
+      : R8(v, 0), R8(v, 8), R8(v, 16), R8(v, 24)
+      : "r"(taddr)
+      : "memory");
+}
+// 64 consecutive columns holding one fp16 accumulator element each (32-bit containers), two per register
+__device__ __forceinline__ void tmem_ld32p(uint32_t taddr, uint32_t (&v)[32]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x32.pack::16b.b32 "
+      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+      : R8(v, 0), R8(v, 8), R8(v, 16), R8(v, 24)
       : "r"(taddr)
       : "memory");
 }
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : TCX_R8(v, 0), TCX_R8(v, 8)
+      : R8(v, 0), R8(v, 8)
       : "r"(taddr)
+      : "memory");
+}
+template <int OFF, int N>
+__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&v)[N]) {
+  static_assert(OFF + 32 <= N, "out of range");
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%32], "
+      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31};" ::
+          W8(v, OFF + 0), W8(v, OFF + 8), W8(v, OFF + 16), W8(v, OFF + 24), "r"(taddr)
       : "memory");
 }
 
@@ -153,6 +191,23 @@ __device__ __forceinline__ uint32_t make_desc_lo(uint32_t smem_addr, uint32_t lb
   return ((smem_addr >> 4) & 0x3FFF) | (((lbo_bytes >> 4) & 0x3FFF) << 16);
 }
 constexpr uint32_t DESC_HI = (128u >> 4) | (1u << 14);
+// host: byte offset of element (n, k) of a `rows`-row slab in the layout of make_desc -- the 8-row x 16-byte core
+// matrices of a K-chunk are contiguous, so row n starts n * 16 bytes into it; K-chunks are rows * 16 bytes apart (LBO)
+inline size_t canon(int n, int k, int rows) {
+  return (size_t)(k / 8) * rows * 16 + (size_t)n * 16 + (size_t)(k % 8) * 2;
+}
+// host: fp16 conversions (round to nearest even), no device needed
+inline uint16_t f2h(float f) {
+  __half h = __float2half_rn(f);
+  uint16_t u;
+  std::memcpy(&u, &h, 2);
+  return u;
+}
+inline float h2f(uint16_t u) {
+  __half h;
+  std::memcpy(&h, &u, 2);
+  return __half2float(h);
+}
 // the issuer's form of mma_ss_2cta: descriptors assembled inside the asm block from their low words, so the compiler
 // has no 64-bit descriptor tables to precompute (and spill) ahead of the first MMA of a stage
 __device__ __forceinline__ void mma_ss_2cta_lo(uint32_t d_tmem, uint32_t a_lo, uint32_t b_lo, uint32_t idesc,
@@ -166,10 +221,35 @@ __device__ __forceinline__ void mma_ss_2cta_lo(uint32_t d_tmem, uint32_t a_lo, u
       "r"(a_lo), "r"(b_lo), "r"(idesc), "r"(accumulate), "n"(DESC_HI)
       : "memory");
 }
+// The issuer's form of mma_ts_2cta: everything that is known at compile time (TMEM column offsets, the descriptor's
+// offset from the start of shared memory, LBO, the instruction descriptor, the accumulate flag) is an immediate inside
+// the asm block, so per MMA only two adds feed the instruction and the compiler has nothing to hoist out of the
+// tile loop (a first unrolled version precomputed 240 descriptors and spilled them).
+//   sb4      = shared-memory base address >> 4
+//   DESC_IMM = (byte offset of the B slab >> 4) + (LBO >> 4 << 16), added to sb4 -> low descriptor word
+template <uint32_t D_COL, uint32_t A_COL, uint32_t DESC_IMM, uint32_t IDESC, bool ACC>
+__device__ __forceinline__ void mma_ts_2cta_imm(uint32_t tmem_base, uint32_t sb4) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t.reg .b64 bd;\n\t.reg .b32 dl, td, ta;\n\t"
+      "add.u32 td, %0, %2;\n\t"
+      "add.u32 ta, %0, %3;\n\t"
+      "add.u32 dl, %1, %4;\n\t"
+      "mov.b64 bd, {dl, %5};\n\t"
+      "setp.ne.b32 p, %7, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [td], [ta], bd, %6, p;\n\t}" ::"r"(tmem_base),
+      "r"(sb4), "n"(D_COL), "n"(A_COL), "n"(DESC_IMM), "n"(DESC_HI), "n"(IDESC), "n"(ACC ? 1 : 0)
+      : "memory");
+}
+template <uint32_t D_COL, uint32_t A_COL, uint32_t B_OFF, uint32_t LBO, uint32_t IDESC, int... KS>
+__device__ __forceinline__ void mma_group(uint32_t tmem_base, uint32_t sb4, std::integer_sequence<int, KS...>) {
+  (mma_ts_2cta_imm<D_COL, A_COL + KS * 8, (B_OFF >> 4) + ((LBO >> 4) << 16) + KS * ((2 * LBO) >> 4), IDESC,
+                   (KS > 0)>(tmem_base, sb4), ...);
+}
 
-// kind::f16 instruction descriptor: fp16 A and B (K-major), fp32 accumulate, dense
-__host__ __device__ constexpr uint32_t make_idesc_f16(int M, int N) {
-  return (1u << 4) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+// kind::f16 instruction descriptor: fp16 (fmt 0) or bf16 (fmt 1) A and B (K-major), fp32 (or fp16) accumulate, dense
+__host__ __device__ constexpr uint32_t make_idesc(int fmt, int M, int N, bool acc_f32 = true) {
+  return (acc_f32 ? (1u << 4) : 0u) | ((uint32_t)fmt << 7) | ((uint32_t)fmt << 10) | ((uint32_t)(N >> 3) << 17) |
+         ((uint32_t)(M >> 4) << 24);
 }
 
 }  // namespace tcx

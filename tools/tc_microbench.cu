@@ -42,7 +42,7 @@ mb_kernel(int mode, int iters, int nwarps, int per_wait, long long* out) {
       asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncwarp();
-    tmem_alloc_512(smem_u32((const void*)tmem_ptr_smem));
+    tmem_alloc_512_2cta(smem_u32((const void*)tmem_ptr_smem));
   }
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   tc_fence_before();
@@ -101,13 +101,13 @@ mb_kernel(int mode, int iters, int nwarps, int per_wait, long long* out) {
       for (int it = 0; it < iters; ++it) {
         if (mode == 3) {
           for (uint32_t ks = 0; ks < 16; ++ks)
-            mma_ts_2cta(tmem_base + TM_DLO, tmem_base + TM_A0 + ks * 8, make_b_desc(sbase + ks * 2 * 128 * 16, 128 * 16, 128),
+            mma_ts_2cta(tmem_base + TM_DLO, tmem_base + TM_A0 + ks * 8, make_desc(sbase + ks * 2 * 128 * 16, 128 * 16),
                         idesc256, ks > 0);
         } else {
           for (int h = 0; h < (mode == 4 ? 1 : 2); ++h)
             for (uint32_t ks = 0; ks < 16; ++ks)
               mma_ts_2cta(tmem_base + (h ? TM_DHI : TM_DLO), tmem_base + TM_A0 + ks * 8,
-                          make_b_desc(sbase + h * SZ_WHH + ks * 2 * 64 * 16, 64 * 16, 128), idesc128, ks > 0);
+                          make_desc(sbase + h * SZ_WHH + ks * 2 * 64 * 16, 64 * 16), idesc128, ks > 0);
         }
       }
       mma_commit_2cta(bar);
@@ -138,7 +138,7 @@ mb_kernel(int mode, int iters, int nwarps, int per_wait, long long* out) {
   cluster_sync_all();
   if (warp == MMA_WARP) {
     __syncwarp();
-    tmem_free_512(tmem_base);
+    tmem_free_512_2cta(tmem_base);
   }
 }
 

@@ -84,8 +84,8 @@ ss_kernel(int mode, int layers, const uint8_t* gsrc, long long* out) {
   } else if (warp == 8 && rank == 0) {
     const bool half = mode & 1;
     const bool m128 = mode & 8;           // M = 128 over the pair: 64 rows per CTA (A images with 64-row K chunks)
-    const uint32_t idesc = m128 ? (half ? make_idesc_f16(128, 128) : make_idesc_f16(128, 256))
-                                : (half ? make_idesc_f16(256, 128) : make_idesc_f16(256, 256));
+    const uint32_t idesc = m128 ? (half ? make_idesc(0, 128, 128) : make_idesc(0, 128, 256))
+                                : (half ? make_idesc(0, 256, 128) : make_idesc(0, 256, 256));
     const uint32_t a_lbo = m128 ? 1024u : 2048u;
     const uint32_t b_lbo = half ? 64 * 16 : 128 * 16;
     const uint32_t a_hi = sbase + OFF_A_HI, a_lo = sbase + OFF_A_LO;

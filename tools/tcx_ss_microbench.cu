@@ -83,7 +83,7 @@ ss_kernel(int mode, int layers, const uint8_t* gsrc, long long* out) {
       for (uint32_t k = (n >= 3 ? n - 3 : 0); k < n; ++k) mbar_wait(bar_ring + 8 * (k % 3), (k / 3) & 1);
   } else if (warp == 8 && rank == 0) {
     const bool half = mode & 1;
-    const uint32_t idesc = half ? make_idesc_f16(256, 128) : make_idesc_f16(256, 256);
+    const uint32_t idesc = half ? make_idesc(0, 256, 128) : make_idesc(0, 256, 256);
     const uint32_t b_lbo = half ? 64 * 16 : 128 * 16;
     const uint32_t a_hi = sbase + OFF_A_HI, a_lo = sbase + OFF_A_LO;
     long long c0 = 0, c1 = 0;
