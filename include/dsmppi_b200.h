@@ -198,6 +198,14 @@ int dsmppi_set_whole_horizon(dsmppi_ctx* ctx, int32_t on);
  * [x, y, r] for a network created with n_point_dim = 2. */
 int dsmppi_set_obstacles(dsmppi_ctx* ctx, const float* obs_dev, int32_t M, void* stream);
 int dsmppi_set_obstacles_host(dsmppi_ctx* ctx, const float* obs_host, int32_t M, void* stream);
+/* Constant-velocity obstacles: vel = (M, P) velocities [vx, vy, vz] (or [vx, vy] for n_point_dim = 2), device or host
+ * memory, in coordinate units per unit of the rollout's dt; radii do not change.  dsmppi_rollout then scores the state
+ * all_traj[:, t-1] of step t = 1..H against x_j + v_j * tau_t with tau_t = (float)(t - 1) * dt, computed in fp32 as one
+ * multiply and one add (no FMA contraction: torch's obs[:, :P] + vel * tau gives the same bits).  dsmppi_distance_grad,
+ * dsmppi_distance_grad_fk, dsmppi_debug_pass1 and the guard-band calibration keep scoring the current positions
+ * (tau = 0).  vel = NULL makes the obstacles static again; so does every dsmppi_set_obstacles call.  M must equal the
+ * obstacle count of the last dsmppi_set_obstacles (else 2).  dsmppi_tick refuses (2) while velocities are set. */
+int dsmppi_set_obstacle_velocities(dsmppi_ctx* ctx, const float* vel, int32_t M, void* stream);
 
 /* Parameters of a SEDS nominal DS (ds_mppi/functions/SEDS.py:9-27), already in the form its GMR uses (:36-59):
  * for Gaussian j: prior, pdf_den = sqrt(2 pi^d det_j + 1e-100) (the denominator of gaussPDF, :28-34), the input and
@@ -333,7 +341,8 @@ int dsmppi_iteration_host(dsmppi_ctx* ctx, dsmppi_iteration_host_args* args, voi
  * D2H of every output into one pinned block -- is captured once per parameter set and then costs one cudaGraphLaunch
  * and one synchronisation.  Kernel arguments are baked into a graph: it is re-captured when any scalar of `rollout`,
  * N, H or n_obs differs from the captured one.  Only for obstacle sets that take the dense fp32 scoring path (the
- * prefilter path ends with a host-side exactness verdict): returns an error otherwise, as it does on a SEDS nominal DS.
+ * prefilter path ends with a host-side exactness verdict): returns an error otherwise, as it does on a SEDS nominal DS
+ * and while obstacle velocities are set (dsmppi_set_obstacle_velocities).
  * Runs on an internal stream ordered after `stream`; synchronises before returning. */
 typedef struct {
   dsmppi_rollout_args rollout;   /* the *_dev fields are ignored; shapes and scalars are used            */

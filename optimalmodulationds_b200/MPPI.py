@@ -109,6 +109,9 @@ class MPPI:
         self.dh_params = dh_params
         self.obs = obs
         self.n_obs = obs.shape[0]
+        # (M, P) obstacle velocities per unit of dt, or None for static obstacles: rollout step t scores against
+        # obs[:, :P] + obs_vel * ((t - 1) * dt) (constant-velocity prediction over the horizon)
+        self.obs_vel = None
         self.dt = dt
         self.dt_H = dt_H
         self.N_traj = N_traj
@@ -251,6 +254,7 @@ class MPPI:
         src = self.obs
         hit = getattr(self, '_obs_uploaded', None)
         if (hit is not None and isinstance(src, torch.Tensor) and hit[0] is src and hit[1] == src._version):
+            self._upload_obstacle_velocities()
             return hit[2]
         obs = self._d(self.obs)
         if obs.dim() != 2 or obs.shape[1] != self._point_dim + 1:
@@ -258,9 +262,29 @@ class MPPI:
                              "obs must be (M, 3) = [x, y, r] for a network with n_dof + 2 inputs")
         self.n_obs = obs.shape[0]
         _capi.check(self._lib.dsmppi_set_obstacles(self._ctx, obs.data_ptr(), int(obs.shape[0]), self._stream()))
+        self._vel_uploaded = (None, None, None)        # dsmppi_set_obstacles made the obstacles static
         if isinstance(src, torch.Tensor):
             self._obs_uploaded = (src, src._version, obs)
+        self._upload_obstacle_velocities()
         return obs
+
+    def _upload_obstacle_velocities(self):
+        # same identity-and-version cache as the obstacles; called after them, so M is the uploaded obstacle count
+        src = self.obs_vel
+        hit = self._vel_uploaded
+        if hit[0] is src and (src is None or (isinstance(src, torch.Tensor) and hit[1] == src._version)):
+            return
+        M = self.n_obs
+        if src is None:
+            _capi.check(self._lib.dsmppi_set_obstacle_velocities(self._ctx, None, M, self._stream()))
+            self._vel_uploaded = (None, None, None)
+            return
+        vel = self._d(src)
+        if tuple(vel.shape) != (M, self._point_dim):
+            raise ValueError(f"obs_vel must be (M, {self._point_dim}) = one velocity per obstacle, "
+                             f"got {tuple(vel.shape)} for {M} obstacles")
+        _capi.check(self._lib.dsmppi_set_obstacle_velocities(self._ctx, vel.data_ptr(), M, self._stream()))
+        self._vel_uploaded = (src, src._version if isinstance(src, torch.Tensor) else None, vel)
 
     def _ignore_mask(self):
         mask = 0
@@ -389,6 +413,8 @@ class MPPI:
             return False
         if self._shard is not None or hasattr(self.DS, 'Mu') or getattr(self, '_timing_on', False):
             return False
+        if self.obs_vel is not None:
+            return False            # the graph replays static obstacles
         if int(self.obs.shape[0]) >= 64 or getattr(self, '_pass1_forced', 'auto') not in ('auto', 'exact'):
             return False            # the prefilter path ends with a host-side verdict: not capturable
         obs = self.obs
@@ -420,6 +446,10 @@ class MPPI:
             ta.rollout.q_cur_is_batch = 1 if probe.dim() == 2 else 0
             t = self._tick = dict(key=key, args=ta, keep=dummy)
         ta = t['args']
+        vel = getattr(self, '_vel_uploaded', (None, None, None))[2]
+        if vel is not None:         # velocities of an earlier call are still set: the graph replays static obstacles
+            _capi.check(self._lib.dsmppi_set_obstacle_velocities(self._ctx, None, int(vel.shape[0]), self._stream()))
+            self._vel_uploaded = (None, None, None)
         obs = self.obs if self.obs.is_contiguous() else self.obs.contiguous()
         q = q_cur_user if q_cur_user.is_contiguous() else q_cur_user.contiguous()
         ta.n_obs = int(obs.shape[0])
@@ -726,8 +756,10 @@ class MPPI:
             _capi.check(self._lib.dsmppi_iteration_host(self._ctx, _capi.C.byref(a), self._stream()))
         return int(a.h2d_bytes), int(a.d2h_bytes)
 
-    def update_obstacles(self, obs):
+    def update_obstacles(self, obs, obs_vel=None):
+        """New obstacle set (M, P + 1); obs_vel: their (M, P) velocities per unit of dt, or None for static ones."""
         self.obs = obs
+        self.obs_vel = obs_vel
         self.n_obs = obs.shape[0]
         return 0
 

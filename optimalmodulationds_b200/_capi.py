@@ -136,6 +136,7 @@ EXPORTS = {
     "dsmppi_set_seds": (C.c_int, [C.c_void_p, C.POINTER(Seds), C.c_void_p]),
     "dsmppi_set_obstacles": (C.c_int, [C.c_void_p, _fp, C.c_int32, C.c_void_p]),
     "dsmppi_set_obstacles_host": (C.c_int, [C.c_void_p, _fp, C.c_int32, C.c_void_p]),
+    "dsmppi_set_obstacle_velocities": (C.c_int, [C.c_void_p, _fp, C.c_int32, C.c_void_p]),
     "dsmppi_rollout": (C.c_int, [C.c_void_p, C.POINTER(RolloutArgs), C.c_void_p]),
     "dsmppi_distance_grad": (C.c_int, [C.c_void_p, _fp, C.c_int32, C.c_int32, C.c_uint32, _fp, _fp, C.c_void_p]),
     "dsmppi_distance_grad_fk": (C.c_int, [C.c_void_p, _fp, C.c_int32, C.c_int32, _fp, _fp, _fp, _fp, C.c_void_p]),

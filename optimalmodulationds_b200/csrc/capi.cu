@@ -202,7 +202,7 @@ void tick_free(dsmppi_ctx* c);
 extern "C" {
 
 const char* dsmppi_last_error(void) { return g_last_error.c_str(); }
-int dsmppi_version(void) { return 102; }   // 102: dsmppi_net.n_hidden / hidden_width
+int dsmppi_version(void) { return 103; }   // 103: dsmppi_set_obstacle_velocities
 
 void dsmppi_modulation_default(dsmppi_modulation* m) {
   if (!m) return;
@@ -323,7 +323,8 @@ int dsmppi_ctx_destroy(dsmppi_ctx* c) {
   cudaSetDevice(c->device);
   tc_free_images(c);
   tcx_free_images(c);
-  void* ptrs[] = {c->weights_blob, c->seds, c->obs, c->obs_raw, c->obs_enc, c->q_work, c->m_rows, c->mdist, c->enc_q,
+  void* ptrs[] = {c->weights_blob, c->seds, c->obs, c->obs_raw, c->obs_enc, c->vel, c->obs_step, c->obs_enc_step,
+                  c->q_work, c->m_rows, c->mdist, c->enc_q,
                   c->cand_cnt, c->row_base, c->row_sample, c->row_obs, c->counters, c->sel, c->fix_list,
                   c->sel_rows, c->row_dist, c->row_grad, c->dist_tmp, c->grad_tmp, c->upd_partials, c->stats_tmp, c->stats_part,
                   c->stats_ticket,
@@ -418,6 +419,30 @@ int dsmppi_set_obstacles(dsmppi_ctx* c, const float* obs_dev, int32_t M, void* s
   }
   c->M = M;
   c->obs_tables_dirty = 1;      // the prefilter's per-obstacle table is rebuilt by the next launch that needs it
+  c->moving = 0;                // a new obstacle set is static until its velocities are set
+  return 0;
+}
+
+int dsmppi_set_obstacle_velocities(dsmppi_ctx* c, const float* vel, int32_t M, void* stream) {
+  REQUIRE(c, "null ctx");
+  REQUIRE(M == c->M, "velocities need one row per obstacle: M differs from the obstacle count of dsmppi_set_obstacles");
+  if (!vel) {
+    c->moving = 0;
+    return 0;
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CUDA_TRY(cudaSetDevice(c->device));
+  if (M > c->vel_cap) {
+    if (c->vel) CUDA_TRY(cudaFree(c->vel));
+    c->vel = nullptr;
+    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&c->vel), (size_t)M * 4 * sizeof(float)));
+    c->vel_cap = M;
+  }
+  // the caller's (M, P) rows -> the (M, 4) layout of c->obs, the components past P zero
+  CUDA_TRY(cudaMemsetAsync(c->vel, 0, (size_t)M * 4 * sizeof(float), st));
+  CUDA_TRY(cudaMemcpy2DAsync(c->vel, 4 * sizeof(float), vel, c->P * sizeof(float), c->P * sizeof(float), M,
+                             cudaMemcpyDefault, st));
+  c->moving = 1;
   return 0;
 }
 
@@ -459,8 +484,8 @@ static int calibrate_band(dsmppi_ctx* c, const float* q, int q_stride, int n, ui
   int rc = ensure_workspace(c, nq, M, mode);
   RowSrc src{};
   src.mode = ROWS_DENSE; src.M = M; src.n_rows = nq * M;
-  if (!rc) rc = launch_exact_forward(c, dq, d, src, ignore_mask, ref, st);
-  if (!rc) rc = tc_pass1(c, dq, d, nq, ignore_mask, mode, st);
+  if (!rc) rc = launch_exact_forward(c, dq, d, c->obs, src, ignore_mask, ref, st);
+  if (!rc) rc = tc_pass1(c, dq, d, c->obs, nullptr, nq, ignore_mask, mode, st);
   if (!rc) rc = launch_max_abs_diff(c, ref, c->mdist, (long long)nq * M, err, st);
   float h = 0.f;
   if (!rc) {
@@ -478,12 +503,15 @@ static int calibrate_band(dsmppi_ctx* c, const float* q, int q_stride, int n, ui
   return 0;
 }
 
-// distance + gradient of n states q (row stride q_stride floats) against the current obstacles, scored in the
+// distance + gradient of n states q (row stride q_stride floats) against the obstacle rows obs, scored in the
 // resolved pass-1 `mode`: fills c->row_dist / c->row_grad and the ranked row indices c->sel_rows (n, K)
+// obs / obs_tab: c->obs and nullptr (the context's prefilter table), or one rollout step's positions and their table
+// (launch_obstacles_at); the guard-band calibration always runs on c->obs
 // table_ready / defer_rank: the rollout loop of the prefilter path hands the per-sample layer-1 table over from the
 // previous step and ranks inside its fused step launch (launch_rank_step)
-static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, int n, int K, uint32_t ignore_mask, int mode,
-                             cudaStream_t st, bool table_ready = false, bool defer_rank = false) {
+static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const void* obs_tab, int n,
+                             int K, uint32_t ignore_mask, int mode, cudaStream_t st, bool table_ready = false,
+                             bool defer_rank = false) {
   REQUIRE(c->M >= 1, "obstacles not set");
   REQUIRE(K >= 1 && K <= MAXK, "n_closest_obs out of range (1..8)");
   REQUIRE(K <= c->M, "n_closest_obs exceeds the number of obstacles");
@@ -503,7 +531,8 @@ static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, int n,
     src.mode = ROWS_DENSE;
     src.n_rows = n * c->M;
     if (timing_mark(c, use_tc_scoring(c) ? 3 : 0, st)) return 1;
-    if (launch_exact_fwdbwd(c, q, q_stride, src, ignore_mask, c->m_rows, c->row_dist, c->row_grad, 0, st)) return 1;
+    if (launch_exact_fwdbwd(c, q, q_stride, obs, src, ignore_mask, c->m_rows, c->row_dist, c->row_grad, 0, st))
+      return 1;
     if (timing_mark(c, use_tc_scoring(c) ? 3 : 0, st)) return 1;
     return launch_rank_dense(c, n, K, true, st);
   }
@@ -512,7 +541,7 @@ static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, int n,
     src.mode = ROWS_DENSE;
     src.n_rows = n * c->M;
     if (timing_mark(c, use_tc_scoring(c) ? 3 : 0, st)) return 1;
-    if (launch_exact_forward(c, q, q_stride, src, ignore_mask, c->m_rows, st)) return 1;
+    if (launch_exact_forward(c, q, q_stride, obs, src, ignore_mask, c->m_rows, st)) return 1;
     if (timing_mark(c, use_tc_scoring(c) ? 3 : 0, st)) return 1;
     if (launch_rank_dense(c, n, K, false, st)) return 1;
     RowSrc s2{};
@@ -521,7 +550,7 @@ static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, int n,
     s2.K = K;
     s2.n_rows = n * K;
     s2.sel = c->sel;
-    if (launch_exact_fwdbwd(c, q, q_stride, s2, ignore_mask, nullptr, c->row_dist, c->row_grad, 0, st)) return 1;
+    if (launch_exact_fwdbwd(c, q, q_stride, obs, s2, ignore_mask, nullptr, c->row_dist, c->row_grad, 0, st)) return 1;
     return launch_identity_rows(c, n, K, st);
   }
   // tensor-core prefilter -> candidate band -> one fp32 launch (ranking key + distance + gradient) -> rank
@@ -529,7 +558,7 @@ static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, int n,
   const float band = c->guard_band > 0.f ? c->guard_band : c->band_cal[band_slot(mode)];
   const size_t cap_rows = cand_list_cap(c, n);
   if (timing_mark(c, 1, st)) return 1;
-  if (tc_pass1(c, q, q_stride, n, ignore_mask, mode, st, table_ready)) return 1;
+  if (tc_pass1(c, q, q_stride, obs, obs_tab, n, ignore_mask, mode, st, table_ready)) return 1;
   if (timing_mark(c, 1, st)) return 1;
   if (launch_select_candidates(c, n, K, band, cap_rows, st)) return 1;
   src.mode = ROWS_LIST;
@@ -538,7 +567,7 @@ static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, int n,
   src.row_sample = c->row_sample;
   src.row_obs = c->row_obs;
   // the candidate count lives on the device; K + 1 per sample is what the guard band typically lets through
-  if (launch_exact_fwdbwd(c, q, q_stride, src, ignore_mask, c->m_rows, c->row_dist, c->row_grad,
+  if (launch_exact_fwdbwd(c, q, q_stride, obs, src, ignore_mask, c->m_rows, c->row_dist, c->row_grad,
                           (long long)n * (K + 1), st))
     return 1;
   if (defer_rank) return 0;
@@ -598,9 +627,24 @@ static int run_exact(dsmppi_ctx* c, int mode, int n_max, cudaStream_t st, Run&& 
   }
 }
 
+// The obstacle rows step t of a per-step path scores against: c->obs, or with moving obstacles their positions at
+// tau = (t - 1) dt, written by one launch before the step's work (with the prefilter's per-obstacle table of `mode`)
+static int step_obstacles(dsmppi_ctx* c, const dsmppi_rollout_args* a, int t, int mode, cudaStream_t st,
+                          const float** obs, const void** obs_tab) {
+  *obs = c->obs;
+  *obs_tab = nullptr;
+  if (!c->moving) return 0;
+  if (launch_obstacles_at(c, (float)(t - 1) * a->dt, mode, st)) return 1;
+  *obs = c->obs_step;
+  if (mode != DSMPPI_PASS1_EXACT_FP32) *obs_tab = c->obs_enc_step;
+  return 0;
+}
+
 // one pass over the batch (in blocks of samples) in the resolved pass-1 `mode` with the context's list budget
 static int rollout_once(dsmppi_ctx* c, const dsmppi_rollout_args* a, int mode, cudaStream_t st) {
   const int d = c->d;
+  const float* obs = nullptr;
+  const void* obs_tab = nullptr;
   const long long block = sample_block(c);
   for (long long off = 0; off < a->N; off += block) {
     dsmppi_rollout_args b = slice_samples(*a, d, off, (int)(a->N - off < block ? a->N - off : block));
@@ -612,7 +656,9 @@ static int rollout_once(dsmppi_ctx* c, const dsmppi_rollout_args* a, int mode, c
       b.n_closest = 1;
       for (int t = 1; t <= b.H; ++t) {
         const float* q = b.all_traj_dev + (size_t)(t - 1) * d;
-        if (launch_fk_distance(c, q, b.H * d, b.N, b.fk_n_pts, b.fk_span, c->row_dist, c->row_grad, d, nullptr, st))
+        if (step_obstacles(c, &b, t, DSMPPI_PASS1_EXACT_FP32, st, &obs, &obs_tab)) return 1;
+        if (launch_fk_distance(c, q, b.H * d, obs, b.N, b.fk_n_pts, b.fk_span, c->row_dist, c->row_grad, d, nullptr,
+                               st))
           return 1;
         if (launch_step(c, &b, t, st)) return 1;
       }
@@ -636,14 +682,18 @@ static int rollout_once(dsmppi_ctx* c, const dsmppi_rollout_args* a, int mode, c
       for (int t = 1; t <= b.H; ++t) {
         const float* q = b.all_traj_dev + (size_t)(t - 1) * d;        // q_prev = all_traj[:, t-1, :]
         // from step 2 on, the previous step's rank_step launch wrote the layer-1 table of these states
-        if (distance_pipeline(c, q, b.H * d, b.N, b.n_closest, b.ignored_link_mask, mode, st, t > 1, true)) return 1;
+        if (step_obstacles(c, &b, t, mode, st, &obs, &obs_tab)) return 1;
+        if (distance_pipeline(c, q, b.H * d, obs, obs_tab, b.N, b.n_closest, b.ignored_link_mask, mode, st, t > 1,
+                              true))
+          return 1;
         if (launch_rank_step(c, &b, t, mode, st)) return 1;
       }
       continue;
     }
     for (int t = 1; t <= b.H; ++t) {
       const float* q = b.all_traj_dev + (size_t)(t - 1) * d;          // q_prev = all_traj[:, t-1, :]
-      if (distance_pipeline(c, q, b.H * d, b.N, b.n_closest, b.ignored_link_mask, mode, st)) return 1;
+      if (step_obstacles(c, &b, t, mode, st, &obs, &obs_tab)) return 1;
+      if (distance_pipeline(c, q, b.H * d, obs, obs_tab, b.N, b.n_closest, b.ignored_link_mask, mode, st)) return 1;
       if (launch_step(c, &b, t, st)) return 1;
     }
   }
@@ -702,7 +752,8 @@ int dsmppi_distance_grad(dsmppi_ctx* c, const float* q_dev, int32_t n, int32_t n
     const int nb = (int)(n - off < block ? n - off : block);
     // each block is repeated on its own
     const int rc = run_exact(c, mode, nb, st, [&](int m, int) {
-      const int r = distance_pipeline(c, q_dev + off * c->d, c->d, nb, n_closest, ignored_link_mask, m, st);
+      const int r = distance_pipeline(c, q_dev + off * c->d, c->d, c->obs, nullptr, nb, n_closest, ignored_link_mask, m,
+                                      st);
       return r ? r : launch_blend(c, nb, n_closest, distance_dev + off, nn_grad_dev + off * c->d, st);
     });
     if (rc) return rc;
@@ -717,8 +768,8 @@ int dsmppi_distance_grad_fk(dsmppi_ctx* c, const float* q_dev, int32_t n, int32_
   REQUIRE(c->M >= 1, "obstacles not set");
   REQUIRE(c->P == 3, "the FK distance provider needs 3-D obstacles");
   CUDA_TRY(cudaSetDevice(c->device));
-  return launch_fk_distance(c, q_dev, c->d, n, fk_n_pts, span_host, distance_dev, grad_dev, c->d, closest_idx_dev,
-                            static_cast<cudaStream_t>(stream));
+  return launch_fk_distance(c, q_dev, c->d, c->obs, n, fk_n_pts, span_host, distance_dev, grad_dev, c->d,
+                            closest_idx_dev, static_cast<cudaStream_t>(stream));
 }
 
 int dsmppi_debug_pass1(dsmppi_ctx* c, const float* q_dev, int32_t n, uint32_t ignored_link_mask, int32_t mode,
@@ -734,11 +785,11 @@ int dsmppi_debug_pass1(dsmppi_ctx* c, const float* q_dev, int32_t n, uint32_t ig
   if (mode == DSMPPI_PASS1_EXACT_FP32) {
     RowSrc src{};
     src.mode = ROWS_DENSE; src.M = c->M; src.n_rows = n * c->M;
-    if (launch_exact_forward(c, q_dev, c->d, src, ignored_link_mask, c->m_rows, st)) return 1;
+    if (launch_exact_forward(c, q_dev, c->d, c->obs, src, ignored_link_mask, c->m_rows, st)) return 1;
     CUDA_TRY(cudaMemcpyAsync(out_dev, c->m_rows, bytes, cudaMemcpyDeviceToDevice, st));
   } else {
     REQUIRE(c->tc_blob, "tensor-core path unavailable for this network");
-    if (tc_pass1(c, q_dev, c->d, n, ignored_link_mask, mode, st)) return 1;
+    if (tc_pass1(c, q_dev, c->d, c->obs, nullptr, n, ignored_link_mask, mode, st)) return 1;
     CUDA_TRY(cudaMemcpyAsync(out_dev, c->mdist, bytes, cudaMemcpyDeviceToDevice, st));
   }
   return 0;                // the next rollout re-sizes for its own mode (ensure_workspace keys on it)
@@ -1081,6 +1132,7 @@ extern "C" int dsmppi_tick(dsmppi_ctx* c, dsmppi_tick_args* t, void* stream) {
   REQUIRE(r.n_kernels == 0 || (t->mu_tmp_host && t->sigma_tmp_host && t->alpha_tmp_host), "null policy pointer");
   REQUIRE(r.mod.ds_kind != DSMPPI_DS_SEDS && r.distance_provider == DSMPPI_DISTANCE_NN,
           "the graphed tick covers the linear / matrix nominal DS with the network distance");
+  REQUIRE(!c->moving, "the graphed tick covers static obstacles (clear the velocities, or call dsmppi_rollout)");
   CUDA_TRY(cudaSetDevice(c->device));
   // the prefilter path cannot be captured (it ends with a host-side verdict)
   REQUIRE(resolve_mode(c, c->pass1_mode, t->n_obs) == DSMPPI_PASS1_EXACT_FP32,

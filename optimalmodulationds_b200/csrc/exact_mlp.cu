@@ -58,8 +58,8 @@ exact_mlp_kernel(NetDev net, RowSrc src, const float* __restrict__ q, int q_stri
                                        (tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x);
   int stage = 0;
   for (int tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-    mlp_tile<BWD, RPT, FT, WID>(net, src, tile * R, n_rows, q, q_stride, obs, ignore_mask, out_m, out_dist, out_grad, sm, ws,
-                           stage);
+    mlp_tile<BWD, RPT, FT, WID>(net, src, tile * R, n_rows, q, q_stride, obs, nullptr, 0.f, ignore_mask, out_m, out_dist,
+                                out_grad, sm, ws, stage);
     __syncthreads();
   }
 }
@@ -72,11 +72,13 @@ exact_mlp_kernel(NetDev net, RowSrc src, const float* __restrict__ q, int q_stri
 // The weight stream simply keeps running across steps.  This is the path of the reference's own CPU-sized
 // problems (planar scripts: M = 2..4; Franka integrator tick: N = 1, H = 2) where launch latency, not FLOPs,
 // set the pace of the per-step launch sequence.
+// MOVE: constant-velocity obstacles -- step t reads obstacle j at obstacle_at(obs, vel, j, c, (t - 1) dt).  A separate
+// instantiation, so the static kernels are compiled exactly as without motion.
 // ------------------------------------------------------------------------------------------------
-template <int RPT, int FT, int WID>
+template <int RPT, int FT, int WID, bool MOVE>
 __global__ void __launch_bounds__(nthreads(FT, WID), (FT == 8 ? 3 : 2) * (HID / WID))
-rollout_fused_kernel(NetDev net, StepArgs sa, const float* __restrict__ obs, int M, uint32_t ignore_mask,
-                     float* m_rows, float* row_dist, float* row_grad, int* sel_rows) {
+rollout_fused_kernel(NetDev net, StepArgs sa, const float* __restrict__ obs, const float* __restrict__ vel, int M,
+                     uint32_t ignore_mask, float* m_rows, float* row_dist, float* row_grad, int* sel_rows) {
   constexpr int R = 4 * RPT;
   extern __shared__ __align__(16) float smem[];
   const int S = R / M;                                  // samples per CTA
@@ -96,8 +98,9 @@ rollout_fused_kernel(NetDev net, StepArgs sa, const float* __restrict__ obs, int
   const int tid = threadIdx.x;
   for (int t = 1; t <= sa.H; ++t) {
     const float* q = sa.traj + (size_t)(t - 1) * d;     // q_prev = all_traj[:, t-1, :]
-    mlp_tile<true, RPT, FT, WID>(net, src, row0, n_rows, q, sa.H * d, obs, ignore_mask, m_rows, row_dist, row_grad, sm,
-                            ws, stage);
+    const float tau = MOVE ? __fmul_rn((float)(t - 1), sa.dt) : 0.f;
+    mlp_tile<true, RPT, FT, WID>(net, src, row0, n_rows, q, sa.H * d, obs, MOVE ? vel : nullptr, tau, ignore_mask, m_rows,
+                                 row_dist, row_grad, sm, ws, stage);
     __syncthreads();                                    // the tile's rows are visible to the whole CTA
     if (tid < ns) {
       const int i = i0 + tid;
@@ -151,12 +154,12 @@ Shape pick_shape(const dsmppi_ctx* c, long long rows, int min_rows_per_tile) {
 }
 
 template <bool BWD, int RPT, int FT, int WID>
-int launch_variant(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask, float* out_m,
-                   float* out_dist, float* out_grad, cudaStream_t st) {
+int launch_variant(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src,
+                   uint32_t ignore_mask, float* out_m, float* out_dist, float* out_grad, cudaStream_t st) {
   constexpr int R = 4 * RPT;
   const long long grid = ((long long)src.n_rows + R - 1) / R;
   exact_mlp_kernel<BWD, RPT, FT, WID><<<(unsigned)grid, nthreads(FT, WID), smem_bytes(R, WID), st>>>(
-      c->net, src, q, q_stride, c->obs, ignore_mask, out_m, out_dist, out_grad);
+      c->net, src, q, q_stride, obs, ignore_mask, out_m, out_dist, out_grad);
   CUDA_TRY(cudaGetLastError());
   c->launches++;
   return 0;
@@ -180,13 +183,13 @@ int tile_width(const dsmppi_ctx* c) { return c->net.width <= 64 ? 64 : (c->net.w
   } while (0)
 
 template <bool BWD>
-int launch(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask, float* out_m,
-           float* out_dist, float* out_grad, long long rows_estimate, cudaStream_t st) {
+int launch(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src, uint32_t ignore_mask,
+           float* out_m, float* out_dist, float* out_grad, long long rows_estimate, cudaStream_t st) {
   if (src.n_rows <= 0) return 0;
   if (rows_estimate <= 0 || rows_estimate > src.n_rows) rows_estimate = src.n_rows;
   const Shape sh = pick_shape(c, rows_estimate, 1);
 #define CALL(RPT, FT, WID) \
-  launch_variant<BWD, RPT, FT, WID>(c, q, q_stride, src, ignore_mask, out_m, out_dist, out_grad, st)
+  launch_variant<BWD, RPT, FT, WID>(c, q, q_stride, obs, src, ignore_mask, out_m, out_dist, out_grad, st)
   SHAPE_DISPATCH(c, sh, CALL);
 #undef CALL
 }
@@ -197,8 +200,12 @@ int launch_fused_variant(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream
   const int S = R / c->M;
   const long long grid = ((long long)a->N + S - 1) / S;
   const StepArgs sa = make_step_args(c, a, 0);
-  rollout_fused_kernel<RPT, FT, WID><<<(unsigned)grid, nthreads(FT, WID), smem_bytes(R, WID), st>>>(
-      c->net, sa, c->obs, c->M, a->ignored_link_mask, c->m_rows, c->row_dist, c->row_grad, c->sel_rows);
+  if (c->moving)
+    rollout_fused_kernel<RPT, FT, WID, true><<<(unsigned)grid, nthreads(FT, WID), smem_bytes(R, WID), st>>>(
+        c->net, sa, c->obs, c->vel, c->M, a->ignored_link_mask, c->m_rows, c->row_dist, c->row_grad, c->sel_rows);
+  else
+    rollout_fused_kernel<RPT, FT, WID, false><<<(unsigned)grid, nthreads(FT, WID), smem_bytes(R, WID), st>>>(
+        c->net, sa, c->obs, nullptr, c->M, a->ignored_link_mask, c->m_rows, c->row_dist, c->row_grad, c->sel_rows);
   CUDA_TRY(cudaGetLastError());
   c->launches++;
   return 0;
@@ -211,7 +218,9 @@ int set_attributes_variant() {
                                 (int)smem_bytes(R, WID)));
   CUDA_TRY(cudaFuncSetAttribute(exact_mlp_kernel<false, RPT, FT, WID>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)smem_bytes(R, WID)));
-  CUDA_TRY(cudaFuncSetAttribute(rollout_fused_kernel<RPT, FT, WID>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  CUDA_TRY(cudaFuncSetAttribute(rollout_fused_kernel<RPT, FT, WID, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)smem_bytes(R, WID)));
+  CUDA_TRY(cudaFuncSetAttribute(rollout_fused_kernel<RPT, FT, WID, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)smem_bytes(R, WID)));
   return 0;
 }
@@ -246,39 +255,44 @@ int launch_rollout_fused(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream
 
 namespace {
 template <int WID>
-int launch_fixup_width(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
-                       float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st) {
+int launch_fixup_width(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src,
+                       uint32_t ignore_mask, float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st) {
   constexpr int RPT = 8, FT = 8, R = 4 * RPT;
   long long grid = ((long long)src.n_rows + R - 1) / R;
   if (grid > 4LL * c->sm_count) grid = 4LL * c->sm_count;       // usually no row is flagged: keep the launch tiny
   if (bwd)
     exact_mlp_kernel<true, RPT, FT, WID><<<(unsigned)grid, nthreads(FT, WID), smem_bytes(R, WID), st>>>(
-        c->net, src, q, q_stride, c->obs, ignore_mask, m_rows, row_dist, row_grad);
+        c->net, src, q, q_stride, obs, ignore_mask, m_rows, row_dist, row_grad);
   else
     exact_mlp_kernel<false, RPT, FT, WID><<<(unsigned)grid, nthreads(FT, WID), smem_bytes(R, WID), st>>>(
-        c->net, src, q, q_stride, c->obs, ignore_mask, m_rows, nullptr, nullptr);
+        c->net, src, q, q_stride, obs, ignore_mask, m_rows, nullptr, nullptr);
   CUDA_TRY(cudaGetLastError());
   c->launches++;
   return 0;
 }
 }  // namespace
 
-int launch_exact_fixup(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
-                       float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st) {
+int launch_exact_fixup(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src,
+                       uint32_t ignore_mask, float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st) {
+#define FIXUP(W) launch_fixup_width<W>(c, q, q_stride, obs, src, ignore_mask, m_rows, row_dist, row_grad, bwd, st)
   const int w = tile_width(c);
-  if (w == 64) return launch_fixup_width<64>(c, q, q_stride, src, ignore_mask, m_rows, row_dist, row_grad, bwd, st);
-  if (w == 128) return launch_fixup_width<128>(c, q, q_stride, src, ignore_mask, m_rows, row_dist, row_grad, bwd, st);
-  return launch_fixup_width<HID>(c, q, q_stride, src, ignore_mask, m_rows, row_dist, row_grad, bwd, st);
+  if (w == 64) return FIXUP(64);
+  if (w == 128) return FIXUP(128);
+  return FIXUP(HID);
+#undef FIXUP
 }
 
-int launch_exact_forward(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
-                         float* m_rows, cudaStream_t st) {
-  if (use_tc_scoring(c)) return launch_tc_exact(c, q, q_stride, src, ignore_mask, m_rows, nullptr, nullptr, false, st);
-  return launch<false>(c, q, q_stride, src, ignore_mask, m_rows, nullptr, nullptr, 0, st);
+int launch_exact_forward(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src,
+                         uint32_t ignore_mask, float* m_rows, cudaStream_t st) {
+  if (use_tc_scoring(c))
+    return launch_tc_exact(c, q, q_stride, obs, src, ignore_mask, m_rows, nullptr, nullptr, false, st);
+  return launch<false>(c, q, q_stride, obs, src, ignore_mask, m_rows, nullptr, nullptr, 0, st);
 }
 
-int launch_exact_fwdbwd(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
-                        float* m_rows, float* row_dist, float* row_grad, long long rows_estimate, cudaStream_t st) {
-  if (use_tc_scoring(c)) return launch_tc_exact(c, q, q_stride, src, ignore_mask, m_rows, row_dist, row_grad, true, st);
-  return launch<true>(c, q, q_stride, src, ignore_mask, m_rows, row_dist, row_grad, rows_estimate, st);
+int launch_exact_fwdbwd(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src,
+                        uint32_t ignore_mask, float* m_rows, float* row_dist, float* row_grad, long long rows_estimate,
+                        cudaStream_t st) {
+  if (use_tc_scoring(c))
+    return launch_tc_exact(c, q, q_stride, obs, src, ignore_mask, m_rows, row_dist, row_grad, true, st);
+  return launch<true>(c, q, q_stride, obs, src, ignore_mask, m_rows, row_dist, row_grad, rows_estimate, st);
 }

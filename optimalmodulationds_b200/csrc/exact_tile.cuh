@@ -248,10 +248,12 @@ __device__ __forceinline__ void stream_begin(WeightStream<WID>& ws, const NetDev
 
 // One pass of the network over the R rows [row0, row0 + R) of `src` (rows >= n_rows are padding): forward, and with
 // BWD the analytic VJP.  Called by all NT threads of the CTA; `ws` / `stage` carry the weight stream across calls.
+// The obstacle coordinates are obstacle_at(obs, vel, j, c, tau): vel == nullptr scores against obs as it is.
 template <bool BWD, int RPT, int FT, int WID = HID>
 __device__ __forceinline__ void mlp_tile(const NetDev& net, const RowSrc& src, int row0, int n_rows,
                                          const float* q, int q_stride, const float* __restrict__ obs,
-                                         uint32_t ignore_mask, float* out_m, float* out_dist, float* out_grad,
+                                         const float* __restrict__ vel, float tau, uint32_t ignore_mask,
+                                         float* out_m, float* out_dist, float* out_grad,
                                          const TileSmem<RPT, WID>& sm, WeightStream<WID>& ws, int& stage) {
   constexpr int R = 4 * RPT;
   constexpr int NT = nthreads(FT, WID);
@@ -271,7 +273,7 @@ __device__ __forceinline__ void mlp_tile(const NetDev& net, const RowSrc& src, i
     int i = 0, j = 0;
     const bool valid = row_lookup(src, row0 + r, n_rows, i, j);
     float x = 0.f;
-    if (valid) x = (c < d) ? q[(size_t)i * q_stride + c] : obs[j * 4 + (c - d)];
+    if (valid) x = (c < d) ? q[(size_t)i * q_stride + c] : obstacle_at(obs, vel, j, c - d, tau);
     xs[r * XS + c] = x;
     act[c][r] = x;
     act[nin + c][r] = sinf(x);

@@ -81,6 +81,14 @@ __device__ __forceinline__ bool row_lookup(const RowSrc& s, int r, int n_rows, i
   return true;
 }
 
+// Coordinate c (0..2) of obstacle j at time tau of a rollout with constant-velocity obstacles: x + v * tau, one fp32
+// multiply and one fp32 add without contraction, so torch's obs[:, :P] + vel * tau gives the same bits.
+// vel == nullptr: the static position (every static caller passes a literal nullptr, which folds the branch away).
+__device__ __forceinline__ float obstacle_at(const float* obs, const float* vel, int j, int c, float tau) {
+  const float x = obs[j * 4 + c];
+  return vel ? __fadd_rn(x, __fmul_rn(vel[j * 4 + c], tau)) : x;
+}
+
 struct DhTable { float v[MAXD + 1][4]; };   // rows [d, theta, a, alpha]
 
 struct dsmppi_ctx {
@@ -107,6 +115,11 @@ struct dsmppi_ctx {
   float* obs = nullptr; int obs_cap = 0;   // always (M, 4) = [x, y, z, r] on the device (z = 0 when P == 2)
   float* obs_raw = nullptr; int obs_raw_cap = 0;   // P == 2: the caller's (M, 3) rows before repacking
   void* obs_enc = nullptr; size_t obs_enc_cap = 0;   // tensor path: per-obstacle packed encodings
+  // constant-velocity obstacles (dsmppi_set_obstacle_velocities; cleared by dsmppi_set_obstacles)
+  int moving = 0;                     // 1 while velocities are set: rollout step t scores against x + v * (t - 1) dt
+  float* vel = nullptr; int vel_cap = 0;     // (M, 4) = [vx, vy, vz, 0] (vz = 0 when P == 2)
+  float* obs_step = nullptr; int obs_step_cap = 0;   // per-step paths: (M, 4) positions of the current step
+  void* obs_enc_step = nullptr; size_t obs_enc_step_cap = 0;   // ... and their per-obstacle layer-1 table (prefilter)
   // SEDS nominal DS: [priors G | pdf_den G | mu_x G*d | mu_y G*d | sigma_inv G*d*d | A G*d*d]
   float* seds = nullptr; int seds_G = 0; float seds_thr = 0.f;
   // workspace (grown on demand)
@@ -173,24 +186,26 @@ struct dsmppi_ctx {
 
 // exact_mlp.cu
 // q points at the first state; consecutive samples are q_stride floats apart
-int launch_exact_forward(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
-                         float* m_rows, cudaStream_t st);
+// obs: the (M, 4) obstacle rows to score against (c->obs, or one rollout step's positions c->obs_step)
+int launch_exact_forward(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src,
+                         uint32_t ignore_mask, float* m_rows, cudaStream_t st);
 // forward + VJP; when m_rows != nullptr also writes the pass-1 ranking key of every row
 // rows_estimate: expected row count when src.n_rows is only an upper bound (device-side counter), else 0
-int launch_exact_fwdbwd(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
-                        float* m_rows, float* row_dist, float* row_grad, long long rows_estimate, cudaStream_t st);
+int launch_exact_fwdbwd(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src,
+                        uint32_t ignore_mask, float* m_rows, float* row_dist, float* row_grad, long long rows_estimate,
+                        cudaStream_t st);
 // whole-horizon rollout in one launch (M <= 32, fp32 scoring); all_traj[:, 0] must be initialised
 int launch_rollout_fused(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream_t st);
 // the FFMA kernels over a device-counted row list with remapped outputs (grid-stride; used to re-score the rows the
 // tensor-core kernel flags as out of fp16 range)
-int launch_exact_fixup(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask,
-                       float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st);
+int launch_exact_fixup(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src,
+                       uint32_t ignore_mask, float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st);
 // tc_exact.cu: the same rows / outputs as the two launches above, on the tensor cores (split-fp16 operands)
 // (both image builders take the network embedded in the 256 x 4 frame by dsmppi_ctx_create, never the caller's)
 int tcx_build_images(dsmppi_ctx* c, const dsmppi_net* frame);
 void tcx_free_images(dsmppi_ctx* c);
-int launch_tc_exact(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask, float* m_rows,
-                    float* row_dist, float* row_grad, bool bwd, cudaStream_t st);
+int launch_tc_exact(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src,
+                    uint32_t ignore_mask, float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st);
 int launch_tc_rollout(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream_t st);
 inline bool use_tc_scoring(const dsmppi_ctx* c) { return c->tcx_blob && c->score_mode != DSMPPI_SCORE_FFMA; }
 // tc_pass1.cu
@@ -198,10 +213,15 @@ int tc_build_images(dsmppi_ctx* c, const dsmppi_net* frame);
 void tc_free_images(dsmppi_ctx* c);
 int tc_set_obstacles(dsmppi_ctx* c, cudaStream_t st);
 // table_ready: the per-sample layer-1 table (c->enc_q) of these n states has already been written
-int tc_pass1(dsmppi_ctx* c, const float* q, int q_stride, int n, uint32_t ignore_mask, int mode, cudaStream_t st,
-             bool table_ready = false);
+// obs / obs_tab: the obstacle rows and their per-obstacle layer-1 table in the format of `mode`; obs_tab == nullptr:
+// obs is c->obs and the context's table (built here when c->obs changed) is used
+int tc_pass1(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const void* obs_tab, int n,
+             uint32_t ignore_mask, int mode, cudaStream_t st, bool table_ready = false);
 int tc_reserve_sample_table(dsmppi_ctx* c, int n);
 int tc_sample_table(dsmppi_ctx* c, const float* q, int q_stride, int n, int mode, cudaStream_t st);
+// moving obstacles, per-step paths: c->obs_step = the positions at tau and, for a prefilter `mode`, c->obs_enc_step =
+// their per-obstacle layer-1 table in that mode's format -- one launch
+int launch_obstacles_at(dsmppi_ctx* c, float tau, int mode, cudaStream_t st);
 // rollout_kernels.cu
 int launch_rank_dense(dsmppi_ctx* c, int n, int K, bool rows_out, cudaStream_t st);
 int launch_identity_rows(dsmppi_ctx* c, int n, int K, cudaStream_t st);
@@ -224,8 +244,8 @@ int launch_rank_step(dsmppi_ctx* c, const dsmppi_rollout_args* a, int t, int tab
 int launch_init_traj(dsmppi_ctx* c, const dsmppi_rollout_args* a, cudaStream_t st);
 int launch_cost(dsmppi_ctx* c, const dsmppi_cost_args* a, cudaStream_t st);
 int launch_basis(dsmppi_ctx* c, const float* grad, int64_t n, float* basis, cudaStream_t st);
-int launch_fk_distance(dsmppi_ctx* c, const float* q, int q_stride, int n, int n_pts, const float* span_host,
-                       float* dist, float* grad, int grad_stride, int* idx, cudaStream_t st);
+int launch_fk_distance(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, int n, int n_pts,
+                       const float* span_host, float* dist, float* grad, int grad_stride, int* idx, cudaStream_t st);
 int launch_cost_stats(dsmppi_ctx* c, const float* cost, int N, float* stats, cudaStream_t st);
 int launch_update_partial(dsmppi_ctx* c, const dsmppi_update_args* a, const float* stats, float* packed,
                           cudaStream_t st);

@@ -931,8 +931,8 @@ int launch_cost(dsmppi_ctx* c, const dsmppi_cost_args* a, cudaStream_t st) {
   return 0;
 }
 
-int launch_fk_distance(dsmppi_ctx* c, const float* q, int q_stride, int n, int n_pts, const float* span_host,
-                       float* dist, float* grad, int grad_stride, int* idx, cudaStream_t st) {
+int launch_fk_distance(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, int n, int n_pts,
+                       const float* span_host, float* dist, float* grad, int grad_stride, int* idx, cudaStream_t st) {
   FkDistArgs a;
   if (n_pts < 1 || n_pts > FK_MAX_PTS) { dsmppi_set_error("n_pts out of range (1..32)"); return 2; }
   a.n = n; a.d = c->d; a.M = c->M; a.n_pts = n_pts;
@@ -944,7 +944,7 @@ int launch_fk_distance(dsmppi_ctx* c, const float* q, int q_stride, int n, int n
     a.span[p] = span_host ? span_host[p]
                           : (p < n_pts / 2 ? start + step * (float)p : end - step * (float)(n_pts - 1 - p));
   a.dh = c->dh;
-  a.q = q; a.q_stride = q_stride; a.obs = c->obs;
+  a.q = q; a.q_stride = q_stride; a.obs = obs;
   a.dist = dist; a.grad = grad; a.grad_stride = grad_stride; a.idx = idx;
   if (c->M >= 32) {
     const long long threads = (long long)n * 32;

@@ -180,6 +180,7 @@ struct TxArgs {
   RowSrc src;
   const float* q; int q_stride;
   const float* obs;
+  const float* vel;                          // whole-horizon kernel with MOVE: (M, 4) obstacle velocities
   uint32_t ignore_mask;
   float* out_m; float* out_dist; float* out_grad;
   int* fix_count;                            // rows appended to fix_list by this launch
@@ -282,7 +283,10 @@ __device__ __forceinline__ void store_chunk32(uint8_t* a_hi, uint8_t* a_lo, int 
 // hands over ONE 32-column chunk per N half, and K quarter 2 x + fb of the next operand is complete after 8 (not 16)
 // warp arrivals.  Everything else -- weight images, stage order, arithmetic per element -- is the same, so HM results
 // are bitwise equal to the full-tile kernel.
-template <int MODE, bool HM = false>
+//
+// MOVE (whole-horizon mode only): constant-velocity obstacles -- step t encodes and re-scores obstacle j at
+// obstacle_at(a.obs, a.vel, j, c, (t - 1) dt).  A separate instantiation: the static kernels are compiled as without it.
+template <int MODE, bool HM = false, bool MOVE = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exact_kernel(TxArgs a) {
   constexpr bool BWD = MODE >= 1;
   constexpr int RPC = HM ? 64 : TROWS;                 // rows per CTA per tile
@@ -290,6 +294,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
   constexpr uint32_t DHALF = HM ? 64 : 128;            // TMEM columns of one N = 128 accumulator half
   constexpr uint32_t D2B = HM ? 128 : 256;             // first TMEM column of D2
   static_assert(!HM || MODE == 2, "half tiles are built for the whole-horizon mode");
+  static_assert(!MOVE || MODE == 2, "the per-step launches take the step's obstacle positions in a.obs");
   extern __shared__ __align__(1024) uint8_t smem[];
   const int n_rows = MODE == 2 ? a.sa.N * a.M : (a.src.n_rows_dev ? min(*a.src.n_rows_dev, a.src.n_rows) : a.src.n_rows);
   const int n_tiles = MODE == 2 ? (a.sa.N + 2 * a.S - 1) / (2 * a.S) : (n_rows + 2 * RPC - 1) / (2 * RPC);
@@ -382,6 +387,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
     uint32_t en_range = 0;
     int en_i = 0, en_j = 0;
     bool en_valid = false;
+    float en_tau = 0.f;                                     // MOVE: time of the step being encoded
     auto enc_compute = [&](int i, int j, bool valid, const float* qsrc, int qstride) {
       en_i = i; en_j = j; en_valid = valid; en_range = 0;
       if (HM && fb != 0) return;                            // a row's encoding is written by its fb == 0 threads
@@ -414,7 +420,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
       } else {
         float xp[3];                                        // nin - d obstacle coordinates: 3, or 2 for the toy variant
 #pragma unroll
-        for (int c = 0; c < 3; ++c) xp[c] = (valid && d + c < nin) ? a.obs[j * 4 + c] : 0.f;
+        for (int c = 0; c < 3; ++c)
+          xp[c] = (valid && d + c < nin) ? obstacle_at(a.obs, MOVE ? a.vel : nullptr, j, c, en_tau) : 0.f;
 #pragma unroll
         for (int c = 0; c < 3; ++c)
           if (d + c < nin) {
@@ -478,6 +485,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
         const int ti = (tile * 2 + (int)rank) * a.S + sl;
         const bool tv = sl < a.S && ti < a.sa.N;
         grow = tv ? ti * a.M + tj : n_rows;
+        if (MOVE) en_tau = __fmul_rn((float)(t - 1), a.sa.dt);
         if (t == 1) enc_compute(ti, tj, tv, qsrc, qstride);
         else enc_compute(sl, tj, tv, stg + STG_Q, MAXD);    // ... and handed over in shared memory: no L2 round trip
       } else if (!TCX_ENC_PIPE) {
@@ -864,8 +872,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
             fs.out_row = fixl + 2 * TROWS;
             int stage = 0;
             for (int r0 = 0; r0 < nfix; r0 += 32) {
-              exact_tile::mlp_tile<true, 8, 8>(a.net, fs, r0, nfix, a.q, a.q_stride, a.obs, a.ignore_mask, a.out_m,
-                                              a.out_dist, a.out_grad, ts, ws, stage);
+              exact_tile::mlp_tile<true, 8, 8>(a.net, fs, r0, nfix, a.q, a.q_stride, a.obs, nullptr, 0.f, a.ignore_mask,
+                                              a.out_m, a.out_dist, a.out_grad, ts, ws, stage);
               exact_tile::tile_sync<exact_tile::nthreads(8)>();
             }
           }
@@ -935,8 +943,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) tc_exac
           fs.out_row = fixl + 2 * TROWS;
           int stage = 0;
           for (int r0 = 0; r0 < nfix; r0 += 32) {
-            exact_tile::mlp_tile<true, 8, 8>(a.net, fs, r0, nfix, qsrc, qstride, a.obs, a.ignore_mask, out_m, out_dist,
-                                            out_grad, ts, ws, stage);
+            exact_tile::mlp_tile<true, 8, 8>(a.net, fs, r0, nfix, qsrc, qstride, a.obs, MOVE ? a.vel : nullptr, en_tau,
+                                            a.ignore_mask, out_m, out_dist, out_grad, ts, ws, stage);
             exact_tile::tile_sync<exact_tile::nthreads(8)>();
           }
         }
@@ -1301,6 +1309,8 @@ int tcx_build_images(dsmppi_ctx* c, const dsmppi_net* net) {
   CUDA_TRY(cudaFuncSetAttribute(tc_exact_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
   CUDA_TRY(cudaFuncSetAttribute(tc_exact_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
   CUDA_TRY(cudaFuncSetAttribute(tc_exact_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+  CUDA_TRY(cudaFuncSetAttribute(tc_exact_kernel<2, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+  CUDA_TRY(cudaFuncSetAttribute(tc_exact_kernel<2, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
   return 0;
 }
 
@@ -1312,8 +1322,8 @@ void tcx_free_images(dsmppi_ctx* c) {
   c->tcx_blob = nullptr;
 }
 
-int launch_tc_exact(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& src, uint32_t ignore_mask, float* m_rows,
-                    float* row_dist, float* row_grad, bool bwd, cudaStream_t st) {
+int launch_tc_exact(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const RowSrc& src, uint32_t ignore_mask,
+                    float* m_rows, float* row_dist, float* row_grad, bool bwd, cudaStream_t st) {
   REQUIRE(c->tcx_blob, "split weight images not built");
   if (src.n_rows <= 0) return 0;
   TxImages* t = static_cast<TxImages*>(c->tcx_blob);
@@ -1324,7 +1334,8 @@ int launch_tc_exact(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& s
   a.src = src;
   a.q = q;
   a.q_stride = q_stride;
-  a.obs = c->obs;
+  a.obs = obs;
+  a.vel = nullptr;
   a.ignore_mask = ignore_mask;
   a.out_m = m_rows;
   a.out_dist = row_dist;
@@ -1389,7 +1400,7 @@ int launch_tc_exact(dsmppi_ctx* c, const float* q, int q_stride, const RowSrc& s
   fix.row_sample = c->fix_list;
   fix.row_obs = c->fix_list + c->fix_cap;
   fix.out_row = c->fix_list + 2 * c->fix_cap;
-  return launch_exact_fixup(c, q, q_stride, fix, ignore_mask, m_rows, row_dist, row_grad, bwd, st);
+  return launch_exact_fixup(c, q, q_stride, obs, fix, ignore_mask, m_rows, row_dist, row_grad, bwd, st);
 }
 
 // whole-horizon rollout in one launch on the tensor cores; the caller has checked M <= 128 / 1 and initialised
@@ -1403,6 +1414,7 @@ int launch_tc_rollout(dsmppi_ctx* c, const dsmppi_rollout_args* ra, cudaStream_t
   a.img1 = t->dev + IMG_BYTES;
   a.net = c->net;
   a.obs = c->obs;
+  a.vel = c->moving ? c->vel : nullptr;
   a.ignore_mask = ra->ignored_link_mask;
   a.sa = make_step_args(c, ra, 0);
   a.M = c->M;
@@ -1442,8 +1454,14 @@ int launch_tc_rollout(dsmppi_ctx* c, const dsmppi_rollout_args* ra, cudaStream_t
   long long pairs = c->sm_count / 2;
   if (pairs > tiles) pairs = tiles;
   if (pairs < 1) pairs = 1;
-  if (half_tiles) tc_exact_kernel<2, true><<<dim3((unsigned)(2 * pairs)), NTHREADS, SMEM_BYTES, st>>>(a);
-  else tc_exact_kernel<2><<<dim3((unsigned)(2 * pairs)), NTHREADS, SMEM_BYTES, st>>>(a);
+  const dim3 grid((unsigned)(2 * pairs));
+  if (c->moving) {
+    if (half_tiles) tc_exact_kernel<2, true, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(a);
+    else tc_exact_kernel<2, false, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(a);
+  } else {
+    if (half_tiles) tc_exact_kernel<2, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(a);
+    else tc_exact_kernel<2><<<grid, NTHREADS, SMEM_BYTES, st>>>(a);
+  }
   CUDA_TRY(cudaGetLastError());
   c->launches++;
 #ifdef DSMPPI_TCX_PROF

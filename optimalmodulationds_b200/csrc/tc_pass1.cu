@@ -139,6 +139,35 @@ __global__ void __launch_bounds__(HID) l1_table_kernel(const float* __restrict__
   (void)n;
 }
 
+// Moving obstacles, one launch per rollout step of the per-step paths: obstacle j's position at tau (obstacle_at) into
+// pos, and with tab != nullptr also its row of the per-obstacle table B in one format -- the l1_table_kernel<BF16> row
+// of that position, computed the same way, so the prefilter sees the table tc_set_obstacles would build for it.
+// With a table: one CTA of 256 threads per obstacle; without: one thread per obstacle.
+__global__ void __launch_bounds__(HID) obstacles_at_kernel(const float* __restrict__ obs, const float* __restrict__ vel,
+                                                           int M, float tau, float* __restrict__ pos, int ncomp,
+                                                           int comp0, int nin, const float* __restrict__ Wf0, int bf16,
+                                                           uint16_t* __restrict__ tab) {
+  if (!tab) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= M) return;
+    for (int c = 0; c < 3; ++c) pos[j * 4 + c] = obstacle_at(obs, vel, j, c, tau);
+    pos[j * 4 + 3] = obs[j * 4 + 3];
+    return;
+  }
+  const int j = blockIdx.x, k = threadIdx.x;
+  __shared__ float xs[3 * MAXD];
+  if (k < 4) pos[j * 4 + k] = k < 3 ? obstacle_at(obs, vel, j, k, tau) : obs[j * 4 + 3];
+  if (k < ncomp) {
+    const float v = obstacle_at(obs, vel, j, k, tau);
+    float sn, cs;
+    sincosf(v, &sn, &cs);
+    xs[3 * k] = v; xs[3 * k + 1] = sn; xs[3 * k + 2] = cs;
+  }
+  __syncthreads();
+  const float acc = l1_feature(Wf0, nullptr, k, xs, ncomp, comp0, nin);
+  tab[((size_t)(k >> 3) * M + j) * 8 + (k & 7)] = l1_to_half_bits(acc, bf16 != 0);
+}
+
 // ------------------------------------------------------------------------------------------------
 // The prefilter kernel
 // ------------------------------------------------------------------------------------------------
@@ -830,12 +859,40 @@ int tc_sample_table(dsmppi_ctx* c, const float* q, int q_stride, int n, int mode
   return 0;
 }
 
-int tc_pass1(dsmppi_ctx* c, const float* q, int q_stride, int n, uint32_t ignore_mask, int mode, cudaStream_t st,
-             bool table_ready) {
+int launch_obstacles_at(dsmppi_ctx* c, float tau, int mode, cudaStream_t st) {
+  const int M = c->M;
+  if (M > c->obs_step_cap) {
+    if (c->obs_step) CUDA_TRY(cudaFree(c->obs_step));
+    c->obs_step = nullptr;
+    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&c->obs_step), (size_t)M * 4 * sizeof(float)));
+    c->obs_step_cap = M;
+  }
+  if (mode == DSMPPI_PASS1_EXACT_FP32) {
+    obstacles_at_kernel<<<(M + 127) / 128, 128, 0, st>>>(c->obs, c->vel, M, tau, c->obs_step, 0, 0, 0, nullptr, 0,
+                                                         nullptr);
+  } else {
+    const size_t need = (size_t)M * HID * 2;
+    if (need > c->obs_enc_step_cap) {
+      if (c->obs_enc_step) CUDA_TRY(cudaFree(c->obs_enc_step));
+      c->obs_enc_step = nullptr;
+      CUDA_TRY(cudaMalloc(&c->obs_enc_step, need));
+      c->obs_enc_step_cap = need;
+    }
+    obstacles_at_kernel<<<M, HID, 0, st>>>(c->obs, c->vel, M, tau, c->obs_step, c->P, c->d, c->nin, c->net.Wf[0],
+                                           mode == DSMPPI_PASS1_TC_BF16 ? 1 : 0,
+                                           static_cast<uint16_t*>(c->obs_enc_step));
+  }
+  CUDA_TRY(cudaGetLastError());
+  c->launches++;
+  return 0;
+}
+
+int tc_pass1(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, const void* obs_tab, int n,
+             uint32_t ignore_mask, int mode, cudaStream_t st, bool table_ready) {
   REQUIRE(c->tc_blob, "tensor-core images not built");
   TcImages* t = static_cast<TcImages*>(c->tc_blob);
   const bool bf16 = mode == DSMPPI_PASS1_TC_BF16;
-  if (c->obs_tables_dirty) {              // (small obstacle sets never get here: they are scored densely in fp32)
+  if (!obs_tab && c->obs_tables_dirty) {  // (small obstacle sets never get here: they are scored densely in fp32)
     if (tc_set_obstacles(c, st)) return 1;
     c->obs_tables_dirty = 0;
   }
@@ -846,8 +903,9 @@ int tc_pass1(dsmppi_ctx* c, const float* q, int q_stride, int n, uint32_t ignore
   a.img0 = base;
   a.img1 = base + IMG_BYTES;
   a.tabA = reinterpret_cast<const uint4*>(c->enc_q);
-  a.tabB = reinterpret_cast<const uint4*>(static_cast<uint16_t*>(c->obs_enc) + (bf16 ? (size_t)c->M * HID : 0));
-  a.obs = c->obs;
+  a.tabB = obs_tab ? static_cast<const uint4*>(obs_tab)
+                   : reinterpret_cast<const uint4*>(static_cast<uint16_t*>(c->obs_enc) + (bf16 ? (size_t)c->M * HID : 0));
+  a.obs = obs;
   a.mdist = c->mdist;
   a.n_rows = (long long)n * c->M;
   a.n = n;

@@ -251,7 +251,7 @@ int main(int argc, char** argv) {
   cudaEventCreate(&e0); cudaEventCreate(&e1);
   for (int rep = 0; rep < 3; ++rep) {
     cudaEventRecord(e0);
-    if (tc_pass1(&c, dq, 7, n, 0x7, DSMPPI_PASS1_TC_F16, 0)) return 1;
+    if (tc_pass1(&c, dq, 7, c.obs, nullptr, n, 0x7, DSMPPI_PASS1_TC_F16, 0)) return 1;
     cudaEventRecord(e1);
     cudaError_t e = cudaDeviceSynchronize();
     if (e != cudaSuccess) { printf("tc_pass1: %s\n", cudaGetErrorString(e)); return 1; }
