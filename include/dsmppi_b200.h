@@ -380,6 +380,19 @@ int dsmppi_pass1_stats(dsmppi_ctx* ctx, int64_t* rescored_pairs, int64_t* band_o
  * over 256 random joint vectors + the first states of the calling batch x every obstacle. */
 int dsmppi_exactness_stats(dsmppi_ctx* ctx, int64_t* capacity_retries, int64_t* exact_fallbacks, float* guard_band,
                            float* calibration_error);
+/* Dead-feature skip of the prefilter.  The guard-band calibration also takes a census (fp32, over its joint vectors x
+ * every obstacle) of the features of hidden layers 2..4 that are never active; they are moved last in the prefilter's
+ * feature order (an exact transform of the network) and whole K = 16 steps of them are left out of the tensor-core
+ * GEMMs that read them.  Every prefiltered row proves its skip: when a skipped feature was active in a row, the call is
+ * repeated without the skip and the next call takes the census again.  `skipped_ksteps[3]`: K-steps (of 16) left out
+ * of the layer 3, layer 4 and output GEMMs; `repeated_calls`: calls repeated without the skip since ctx creation. */
+int dsmppi_prefilter_skip_stats(dsmppi_ctx* ctx, int32_t* skipped_ksteps, int64_t* repeated_calls);
+/* The transform the skip applies (host only, no device needed): layers 2..5 of a network of four hidden layers of
+ * width 256 (W: three 256 x 256 blocks then n_out x 256, b: three 256 then n_out; torch orientation, concatenated)
+ * with feature f of hidden layer 2 + l taken from feature perm[l * 256 + f] of the input (perm: 3 x 256).  Returns 2
+ * when perm is not a permutation. */
+int dsmppi_permute_hidden(int32_t n_out, const float* W, const float* b, const int32_t* perm, float* W_out,
+                          float* b_out);
 /* Scoring arithmetic in effect (DSMPPI_SCORE_FFMA / _TC_SPLIT) and, for the tensor-core path, how many rows left the
  * fp16 range of its split operands and were re-scored by the FFMA kernel since the context was created
  * (`dropped_rows` > 0 means the re-scoring list overflowed: results of those rows are saturated, not exact). */

@@ -775,6 +775,13 @@ class MPPI:
                                                      _capi.C.byref(e)))
         return dict(capacity_retries=r.value, exact_fallbacks=f.value, guard_band=g.value, calibration_error=e.value)
 
+    def prefilter_skip_stats(self):
+        """Dead-feature skip of the prefilter (dsmppi_prefilter_skip_stats): K-steps (of 16) left out of the layer 3,
+        layer 4 and output GEMMs, and how many calls were repeated without the skip."""
+        k, r = (_capi.C.c_int32 * 3)(), _capi.C.c_int64()
+        _capi.check(self._lib.dsmppi_prefilter_skip_stats(self._ctx, k, _capi.C.byref(r)))
+        return dict(skipped_ksteps=tuple(k), repeated_calls=r.value)
+
     def pass1_stats(self):
         a, b, m = _capi.C.c_int64(), _capi.C.c_int64(), _capi.C.c_int32()
         _capi.check(self._lib.dsmppi_pass1_stats(self._ctx, _capi.C.byref(a), _capi.C.byref(b), _capi.C.byref(m),

@@ -155,6 +155,8 @@ EXPORTS = {
                                      C.c_void_p]),
     "dsmppi_exactness_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_float),
                                          C.POINTER(C.c_float)]),
+    "dsmppi_prefilter_skip_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_int64)]),
+    "dsmppi_permute_hidden": (C.c_int, [C.c_int32, _fp, _fp, _fp, _fp, _fp]),
     "dsmppi_score_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_int64),
                                      C.c_void_p]),
     "dsmppi_enable_kernel_timing": (C.c_int, [C.c_void_p, C.c_int32]),

@@ -459,11 +459,14 @@ int dsmppi_set_obstacles_host(dsmppi_ctx* c, const float* obs_host, int32_t M, v
 // joint vectors in [-pi, pi]^d plus the first states of the calling batch, against every current obstacle, fp32
 // scoring kernel vs prefilter; band = CAL_SAFETY x the largest difference.  One-off (re-run when the obstacle count
 // changes); costs two launches and one host synchronisation.  dsmppi_set_pass1_mode(.., band > 0) overrides it.
+// With `census`, the same states first take the dead-feature census (tc_census), so that the band is measured on the
+// reordered, skipping kernel that will run; a new feature order voids the band of the other format too.  Should a
+// calibration row itself prove a skipped feature active, the skip is dropped and the band measured again without it.
 constexpr int CAL_Q = 256;
 constexpr float CAL_SAFETY = 3.f;
 
 static int calibrate_band(dsmppi_ctx* c, const float* q, int q_stride, int n, uint32_t ignore_mask, int mode,
-                          cudaStream_t st) {
+                          cudaStream_t st, bool census) {
   const int slot = band_slot(mode);
   const int d = c->d, M = c->M;
   const int n_act = n < CAL_Q ? n : CAL_Q;
@@ -482,18 +485,34 @@ static int calibrate_band(dsmppi_ctx* c, const float* q, int q_stride, int n, ui
   CUDA_TRY(cudaMemcpy2DAsync(dq + (size_t)CAL_Q * d, d * sizeof(float), q, (size_t)q_stride * sizeof(float),
                              d * sizeof(float), n_act, cudaMemcpyDeviceToDevice, st));
   int rc = ensure_workspace(c, nq, M, mode);
+  bool reordered = false;
+  if (!rc && census) rc = tc_census(c, dq, nq, st, &reordered);
+  if (reordered) c->band_cal[0] = c->band_cal[1] = 0.f;
+  const bool measure = c->guard_band <= 0.f && (c->band_cal[slot] <= 0.f || c->band_cal_M[slot] != M);
   RowSrc src{};
   src.mode = ROWS_DENSE; src.M = M; src.n_rows = nq * M;
-  if (!rc) rc = launch_exact_forward(c, dq, d, c->obs, src, ignore_mask, ref, st);
-  if (!rc) rc = tc_pass1(c, dq, d, c->obs, nullptr, nq, ignore_mask, mode, st);
-  if (!rc) rc = launch_max_abs_diff(c, ref, c->mdist, (long long)nq * M, err, st);
+  if (!rc && measure) rc = launch_exact_forward(c, dq, d, c->obs, src, ignore_mask, ref, st);
+  auto ck = [](cudaError_t e) {
+    if (e == cudaSuccess) return 0;
+    dsmppi_set_error(std::string("guard-band calibration: ") + cudaGetErrorString(e));
+    return 1;
+  };
   float h = 0.f;
-  if (!rc) {
-    CUDA_TRY(cudaMemcpyAsync(&h, err, sizeof(float), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
+  for (int pass = 0; !rc && measure && pass < 2; ++pass) {
+    int fired = 0;                         // counter 10 of this measurement alone, cleared for the call that follows
+    rc = ck(cudaMemsetAsync(c->counters + 10, 0, sizeof(int), st));
+    if (!rc) rc = tc_pass1(c, dq, d, c->obs, nullptr, nq, ignore_mask, mode, st);
+    if (!rc) rc = launch_max_abs_diff(c, ref, c->mdist, (long long)nq * M, err, st);
+    if (!rc) rc = ck(cudaMemcpyAsync(&h, err, sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (!rc) rc = ck(cudaMemcpyAsync(&fired, c->counters + 10, sizeof(int), cudaMemcpyDeviceToHost, st));
+    if (!rc) rc = ck(cudaMemsetAsync(c->counters + 10, 0, sizeof(int), st));
+    if (!rc) rc = ck(cudaStreamSynchronize(st));
+    if (rc || fired == 0) break;
+    for (int l = 0; l < 3; ++l) c->pass1_skip[l] = 0;
   }
   cudaFree(dq); cudaFree(ref); cudaFree(err);
   if (rc) return rc;
+  if (!measure) return 0;
   c->band_cal_err[slot] = h;
   float band = CAL_SAFETY * h;
   const float floor_band = (c->O == 9 ? 1e-3f : 1e-2f);      // never below 1 mm (cm-scaled net) / 1 cm
@@ -515,10 +534,13 @@ static int distance_pipeline(dsmppi_ctx* c, const float* q, int q_stride, const 
   REQUIRE(c->M >= 1, "obstacles not set");
   REQUIRE(K >= 1 && K <= MAXK, "n_closest_obs out of range (1..8)");
   REQUIRE(K <= c->M, "n_closest_obs exceeds the number of obstacles");
-  if (mode != DSMPPI_PASS1_EXACT_FP32 && c->guard_band <= 0.f) {
+  if (mode != DSMPPI_PASS1_EXACT_FP32) {
     const int slot = band_slot(mode);
-    if (c->band_cal[slot] <= 0.f || c->band_cal_M[slot] != c->M) {
-      if (calibrate_band(c, q, q_stride, n, ignore_mask, mode, st)) return 1;
+    const bool band_due = c->guard_band <= 0.f && (c->band_cal[slot] <= 0.f || c->band_cal_M[slot] != c->M);
+    // (not while a call is repeated without the skip: the census is taken again by the next call)
+    const bool census_due = !c->pass1_noskip && (c->census_M != c->M || c->census_stale);
+    if (band_due || census_due) {
+      if (calibrate_band(c, q, q_stride, n, ignore_mask, mode, st, census_due)) return 1;
       table_ready = false;                 // the calibration wrote ITS states' table over the one handed in
     }
   }
@@ -593,6 +615,13 @@ static int prefilter_verdict(dsmppi_ctx* c, int n_max, cudaStream_t st, int* ver
     c->exact_fallbacks++;
     return 0;
   }
+  if (h[10] != 0) {      // a row proved a skipped dead feature active: the same prefilter without the skip
+    *verdict = 1;
+    c->pass1_noskip = 1;
+    c->census_stale = 1;
+    c->skip_repeats++;
+    return 0;
+  }
   const size_t high = (size_t)(unsigned)h[8];
   if (high <= cand_list_cap(c, n_max)) return 0;
   *verdict = 1;
@@ -610,14 +639,15 @@ static int prefilter_verdict(dsmppi_ctx* c, int n_max, cudaStream_t st, int* ver
 
 // The prefilter path is exact by construction: a call whose candidates did not all fit the row list is detected after
 // it ran (high-water mark, prefilter_verdict) and run again with a list that holds them -- or, past 2^27 rows or on
-// prefilter outputs beyond fp16, once more with every pair scored in fp32.  The repeat recomputes from the same inputs.
+// prefilter outputs beyond fp16, once more with every pair scored in fp32 -- or, when a row proved a skipped dead feature
+// active (counter 10), once more with the same prefilter and no skip.  The repeat recomputes from the same inputs.
 // run(mode, attempt) does the work of one call in the resolved pass-1 `mode`; attempt is 0, 1, .. for the runs the
 // verdict checks and -1 for the fp32 fallback.
 template <typename Run>
-static int run_exact(dsmppi_ctx* c, int mode, int n_max, cudaStream_t st, Run&& run) {
+static int run_exact_attempts(dsmppi_ctx* c, int mode, int n_max, cudaStream_t st, Run&& run) {
   for (int attempt = 0;; ++attempt) {
     c->prefilter_used = 0;
-    CUDA_TRY(cudaMemsetAsync(c->counters + 8, 0, 2 * sizeof(int), st));
+    CUDA_TRY(cudaMemsetAsync(c->counters + 8, 0, 3 * sizeof(int), st));
     if (const int rc = run(mode, attempt)) return rc;
     int verdict = 0, exact = 0;
     if (const int rc = prefilter_verdict(c, n_max, st, &verdict, &exact)) return rc;
@@ -625,6 +655,14 @@ static int run_exact(dsmppi_ctx* c, int mode, int n_max, cudaStream_t st, Run&& 
     REQUIRE(attempt < 4, "candidate row list still too small after four attempts");
     if (exact) return run(DSMPPI_PASS1_EXACT_FP32, -1);
   }
+}
+// (a repeat without the dead-feature skip lasts for the rest of this call only)
+template <typename Run>
+static int run_exact(dsmppi_ctx* c, int mode, int n_max, cudaStream_t st, Run&& run) {
+  c->pass1_noskip = 0;
+  const int rc = run_exact_attempts(c, mode, n_max, st, run);
+  c->pass1_noskip = 0;
+  return rc;
 }
 
 // The obstacle rows step t of a per-step path scores against: c->obs, or with moving obstacles their positions at
@@ -1031,6 +1069,14 @@ int dsmppi_pass1_stats(dsmppi_ctx* c, int64_t* rescored_pairs, int64_t* band_ove
     *rescored_pairs = (int64_t)v;
   }
   if (mode) *mode = resolve_mode(c, c->pass1_mode, c->M);
+  return 0;
+}
+
+int dsmppi_prefilter_skip_stats(dsmppi_ctx* c, int32_t* skipped_ksteps, int64_t* repeated_calls) {
+  REQUIRE(c, "null argument");
+  if (skipped_ksteps)
+    for (int l = 0; l < 3; ++l) skipped_ksteps[l] = c->pass1_skip[l];
+  if (repeated_calls) *repeated_calls = c->skip_repeats;
   return 0;
 }
 

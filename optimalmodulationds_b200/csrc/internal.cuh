@@ -129,6 +129,12 @@ struct dsmppi_ctx {
   int* counters_host = nullptr;       // pinned mirror of `counters` for the end-of-rollout exactness check
   int obs_tables_dirty = 1;           // c->obs changed since tc_set_obstacles built the per-obstacle layer-1 table
   int pass1_hacc = 1;                 // fp16 prefilter: hidden layers accumulate in fp16 (DSMPPI_PASS1_ACC=f32: in fp32)
+  // dead-feature skip of the prefilter (tc_pass1.cu: tc_census)
+  int pass1_skip[3] = {0, 0, 0};      // K-steps not issued by the layer 3, layer 4 and output GEMMs
+  int census_M = 0;                   // obstacle count of the last census (0: none yet)
+  int census_stale = 0;               // a row proved a skipped feature active: census again on the next call
+  int pass1_noskip = 0;               // 1 while a call is repeated without the skip
+  int64_t skip_repeats = 0;           // calls repeated without the skip
   int half_tiles = 1;                 // whole-horizon tensor-core rollout: 64-row tiles while one wave covers the batch
   int prefilter_used = 0;             // set by distance_pipeline when a call went through the tensor-core prefilter
   int64_t capacity_retries = 0;       // rollouts that were run again with a larger candidate row list
@@ -147,7 +153,9 @@ struct dsmppi_ctx {
                                       // range-fixup row counts (ping-pong), [6] rows re-scored in FFMA so far, [7] rows
                                       // that did not fit the range-fixup list, [8] largest [0] of any step of this
                                       // rollout (> capacity: the rollout is repeated with a larger list), [9] prefilter
-                                      // outputs that were inf / NaN (> 0: the call is repeated with all pairs in fp32)
+                                      // outputs that were inf / NaN (> 0: the call is repeated with all pairs in fp32),
+                                      // [10] prefiltered rows in which a skipped dead feature was active (> 0: the
+                                      // call is repeated without the skip)
   int* sel = nullptr;                 // (n, K) selected obstacle indices (two-launch fp32 path)
   int* sel_rows = nullptr;            // (n, K) rows of row_dist / row_grad holding the K closest, ranked
   float* row_dist = nullptr;          // pass-2 distance of every differentiated row
@@ -212,6 +220,9 @@ inline bool use_tc_scoring(const dsmppi_ctx* c) { return c->tcx_blob && c->score
 int tc_build_images(dsmppi_ctx* c, const dsmppi_net* frame);
 void tc_free_images(dsmppi_ctx* c);
 int tc_set_obstacles(dsmppi_ctx* c, cudaStream_t st);
+// dead-feature census over n states q (row stride d) x the current obstacles; reorders the images and sets
+// c->pass1_skip (*changed: the images' feature order changed).  Synchronises the stream.
+int tc_census(dsmppi_ctx* c, const float* q, int n, cudaStream_t st, bool* changed);
 // table_ready: the per-sample layer-1 table (c->enc_q) of these n states has already been written
 // obs / obs_tab: the obstacle rows and their per-obstacle layer-1 table in the format of `mode`; obs_tab == nullptr:
 // obs is c->obs and the context's table (built here when c->obs changed) is used

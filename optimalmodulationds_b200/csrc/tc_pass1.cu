@@ -85,6 +85,11 @@ constexpr uint32_t TM_A0 = 0, TM_A1 = 128, TM_DLO = 256, TM_DHI = 384;
 
 struct TcImages {
   uint8_t* img[2];        // device images, one per CTA rank
+  // layers 2..5 of the network in the 256 x 4 frame, laid out as dsmppi_permute_hidden takes them: the images are
+  // rebuilt from them whenever the census reorders the hidden features
+  std::vector<float> W, b;
+  int32_t perm[NHID * HID];            // the order of the images in effect
+  uint32_t alive[NHID][HID / 32] = {}; // census: features of hidden layers 2..4 seen active since the last fresh one
 };
 
 template <bool BF16>
@@ -168,6 +173,67 @@ __global__ void __launch_bounds__(HID) obstacles_at_kernel(const float* __restri
   tab[((size_t)(k >> 3) * M + j) * 8 + (k & 7)] = l1_to_half_bits(acc, bf16 != 0);
 }
 
+// Census of the dead-feature skip (tc_census): which features of hidden layers 2..4 have a positive pre-activation
+// for any of the n x M pairs of states q (row stride d) and obstacles obs, in fp32 from the fp32 weights.  One CTA
+// of 256 threads (one feature each) per CEN_R pair-rows; alive[l][w]: bit f % 32 of word f / 32 for feature f.
+constexpr int CEN_R = 32;
+__global__ void __launch_bounds__(HID) census_kernel(const NetDev net, const float* __restrict__ q, int n,
+                                                     const float* __restrict__ obs, int M,
+                                                     uint32_t* __restrict__ alive) {
+  __shared__ __align__(16) float h[HID][CEN_R];
+  __shared__ float xq[CEN_R][3 * MAXD], xp[CEN_R][9];
+  const int k = threadIdx.x, P = net.nin - net.d;
+  const long long nrows = (long long)n * M, r0 = (long long)blockIdx.x * CEN_R;
+  for (int e = k; e < CEN_R * (MAXD + 3); e += HID) {
+    const int r = e / (MAXD + 3), cc = e % (MAXD + 3);
+    const long long row = min(r0 + r, nrows - 1);
+    float v = 0.f;
+    if (cc < net.d) v = q[(row / M) * net.d + cc];
+    else if (cc >= MAXD && cc - MAXD < P) v = obs[(row % M) * 4 + cc - MAXD];
+    else continue;
+    float sn, cs;
+    sincosf(v, &sn, &cs);
+    float* x = cc < MAXD ? &xq[r][3 * cc] : &xp[r][3 * (cc - MAXD)];
+    x[0] = v; x[1] = sn; x[2] = cs;
+  }
+  __syncthreads();
+  float acc[CEN_R];
+#pragma unroll 1
+  for (int r = 0; r < CEN_R; ++r)
+    h[k][r] = fmaxf(l1_feature(net.Wf[0], net.b[0], k, xq[r], net.d, 0, net.nin) +
+                        l1_feature(net.Wf[0], nullptr, k, xp[r], P, net.d, net.nin), 0.f);
+  __syncthreads();
+#pragma unroll 1
+  for (int l = 1; l <= NHID; ++l) {
+#pragma unroll
+    for (int r = 0; r < CEN_R; ++r) acc[r] = net.b[l][k];
+    const float* w = net.Wf[l] + k;
+#pragma unroll 4
+    for (int i = 0; i < HID; ++i) {
+      const float wi = w[(size_t)i * HID];
+      const float4* hv = reinterpret_cast<const float4*>(h[i]);
+#pragma unroll
+      for (int r4 = 0; r4 < CEN_R / 4; ++r4) {
+        const float4 x = hv[r4];
+        acc[4 * r4 + 0] = fmaf(wi, x.x, acc[4 * r4 + 0]);
+        acc[4 * r4 + 1] = fmaf(wi, x.y, acc[4 * r4 + 1]);
+        acc[4 * r4 + 2] = fmaf(wi, x.z, acc[4 * r4 + 2]);
+        acc[4 * r4 + 3] = fmaf(wi, x.w, acc[4 * r4 + 3]);
+      }
+    }
+    __syncthreads();
+    bool any = false;
+#pragma unroll
+    for (int r = 0; r < CEN_R; ++r) {
+      any = any || (r0 + r < nrows && acc[r] > 0.f);
+      h[k][r] = fmaxf(acc[r], 0.f);
+    }
+    const uint32_t bits = __ballot_sync(0xffffffffu, any);
+    if ((k & 31) == 0 && bits) atomicOr(alive + (l - 1) * (HID / 32) + (k >> 5), bits);
+    __syncthreads();
+  }
+}
+
 // ------------------------------------------------------------------------------------------------
 // The prefilter kernel
 // ------------------------------------------------------------------------------------------------
@@ -184,6 +250,11 @@ struct TcArgs {
   int use_writers;                             // 1: warps 9 / 10 store the distances (0: the row warps do, see there)
   long long* prof;                             // DSMPPI_TC_PROF builds only: [block][warp][8] cycle counters
   int* nonfinite;                              // counts pair-rows whose prefilter output is inf / NaN (see the epilogue)
+  // Dead-feature skip: skip[l] of the last K-steps of the GEMM that reads hidden GEMM l's output (network layer 3, 4,
+  // output) are not issued (0..8: only features 128..255, the D_hi half, are ever skipped).  Their input features
+  // were never active in the calibration's census and come last in the images' feature order (tc_census).
+  int skip[NHID];
+  int* dead_fired;                             // counts valid pair-rows in which a skipped feature was not +0
 };
 
 // Per-phase cycle accounting of the kernel's own pipeline (tools/tc_microbench.cu builds with
@@ -240,6 +311,25 @@ __device__ __forceinline__ void load_bias16(const uint4* __restrict__ src, uint4
   for (int k = 0; k < 16; ++k)      // volatile: the compiler would sink plain loads back to their uses, behind the wait
     asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];"
                  : "=r"(b[k].x), "=r"(b[k].y), "=r"(b[k].z), "=r"(b[k].w) : "r"(sa + 16u * k));
+}
+
+// OR of the packed activations (D_hi half, features 128..255, two per word) that the next GEMM does not read when
+// its last `s` K-steps (8 words each) are skipped: 0 certifies that every skipped product was an exact zero
+__device__ __forceinline__ uint32_t dead_or(const uint32_t (&pk)[64], int s) {
+  // straight-line code: a switch over s became indirect branches inside the epilogue and cost spills around them
+  uint32_t r = 0;
+#pragma unroll
+  for (int g = 0; g < 8; ++g)            // words 8g..8g+7 feed K-step 8 + g, skipped when 8 + g >= 16 - s
+    if (g >= 8 - s) r |= (pk[8 * g] | pk[8 * g + 1] | pk[8 * g + 2]) | (pk[8 * g + 3] | pk[8 * g + 4] | pk[8 * g + 5]) |
+                         (pk[8 * g + 6] | pk[8 * g + 7]);
+  return r;
+}
+
+// A skipped feature that was active in a valid row: that row's distance lacks its products.  Counted once the
+// tile's three hidden epilogues are done (not at the output, where one more live register spilled); the host repeats
+// the call without the skip (prefilter_verdict).
+__device__ __forceinline__ void dead_count(const TcArgs& a, uint32_t dead, int i) {
+  if (dead != 0u && i < a.n) atomicAdd(a.dead_fired, 1);
 }
 
 // relu(a + b) on two packed half-precision values: the first hidden activation from the layer-1 tables
@@ -456,6 +546,7 @@ tc_pass1_kernel(const __grid_constant__ TcArgs a) {
       int i_next = min(i_cur + di, a.n), j_next = j_cur + dj;
       if (j_next >= a.M) { j_next -= a.M; i_next = min(i_next + 1, a.n); }
       uint32_t tile_dep = 0;
+      uint32_t dead = 0;                     // dead_or over this tile's three hidden epilogues
       // fp16-accumulator build: one hidden layer's epilogue
       auto hacc_layer = [&](auto L) {
         constexpr int l = decltype(L)::value;
@@ -490,9 +581,13 @@ tc_pass1_kernel(const __grid_constant__ TcArgs a) {
         relu_h2_32<32, 8>(raw[1], bq, pk);
         tmem_st32<0>(tA + 64, pk);
         tmem_st32<32>(tA + 96, pk);
+        dead |= dead_or(pk, a.skip[l]);      // under the store's latency
         tc_wait_st();
         signal(bar_aready);
-        if (l == NHID - 1) tile_dep = (pk[7] | pk[23] | pk[39] | pk[63]) & a.zero;
+        if (l == NHID - 1) {
+          tile_dep = (pk[7] | pk[23] | pk[39] | pk[63]) & a.zero;
+          dead_count(a, dead, i_cur);
+        }
         PROF_ADD(5);
       };
       if constexpr (HACC) {
@@ -542,9 +637,13 @@ tc_pass1_kernel(const __grid_constant__ TcArgs a) {
         relu_pack32<BF16, 48>(raw[3], bl + 224, pk);
         tmem_st32<0>(tA + 64, pk);
         tmem_st32<32>(tA + 96, pk);
+        dead |= dead_or(pk, a.skip[l]);
         tc_wait_st();
         signal(bar_aready);                                         // next layer's A operand is in TMEM
-        if (l == NHID - 1) tile_dep = (pk[7] | pk[23] | pk[39] | pk[63]) & a.zero;
+        if (l == NHID - 1) {
+          tile_dep = (pk[7] | pk[23] | pk[39] | pk[63]) & a.zero;
+          dead_count(a, dead, i_cur);
+        }
         PROF_ADD(5);
       }
       }
@@ -659,8 +758,11 @@ tc_pass1_kernel(const __grid_constant__ TcArgs a) {
       constexpr int ksteps = HID / 16;
       constexpr uint32_t idesc = l < NHID ? idesc128 : idesc32;
       constexpr uint32_t dcol = h ? TM_DHI : TM_DLO, acol = s ? TM_A1 : TM_A0;
+      // K-steps 8..15 of the GEMMs after layer 2 may be skipped (their features come last, see TcArgs::skip)
+      constexpr int fixed = l == 0 ? ksteps : ksteps / 2;
+      const uint32_t nk = l == 0 ? ksteps : ksteps - a.skip[l > 0 ? l - 1 : 0];
       if (elect_one()) {
-        mma_group<dcol, acol, boff, lbo, idesc>(tmem_base, sb4, std::make_integer_sequence<int, ksteps>{});
+        mma_group<dcol, acol, boff, lbo, idesc, fixed>(tmem_base, sb4, nk, std::make_integer_sequence<int, ksteps>{});
         mma_commit_2cta(BAR(BAR_DFULL00 + s * 2 + h));
       }
       __syncwarp();
@@ -755,19 +857,40 @@ uint16_t f2bf(float f) {
 
 }  // namespace
 
-int tc_build_images(dsmppi_ctx* c, const dsmppi_net* net) {
-  c->tc_blob = nullptr;
-  if (c->O > 16) return 0;                          // output N is fixed at 16 links; fall back to fp32
-  const char* dis = std::getenv("DSMPPI_DISABLE_TC");
-  if (dis && dis[0] == '1') return 0;
-  TcImages* t = new TcImages();
-  // two formats x two CTA ranks
-  uint8_t* dev = nullptr;
-  if (cudaMalloc(reinterpret_cast<void**>(&dev), (size_t)4 * IMG_BYTES) != cudaSuccess) {
-    dsmppi_set_error("cudaMalloc(tc images) failed");
-    delete t;
-    return 1;
+// Layers 2..5 of a network in the 256 x 4 frame (W: three 256 x 256 then O x 256, b: three 256 then O; torch
+// orientation, concatenated) with the hidden features of layers 2..4 reordered: feature f of hidden layer 2 + l
+// becomes the network's feature perm[l * 256 + f].  An exact transform of the network: the rows and biases of the
+// layer 2..4 GEMMs and the matching input columns of the layer 3, layer 4 and output GEMMs move together (layer 1
+// keeps its order).
+int dsmppi_permute_hidden(int32_t n_out, const float* W, const float* b, const int32_t* perm, float* W_out,
+                          float* b_out) {
+  REQUIRE(W && b && perm && W_out && b_out, "null argument");
+  REQUIRE(n_out >= 1 && n_out <= MAXO, "n_out out of range (1..16)");
+  for (int l = 0; l < NHID; ++l) {
+    std::vector<int> seen(HID, 0);
+    for (int f = 0; f < HID; ++f) {
+      REQUIRE(perm[l * HID + f] >= 0 && perm[l * HID + f] < HID && !seen[perm[l * HID + f]], "perm is not a permutation");
+      seen[perm[l * HID + f]] = 1;
+    }
   }
+  auto in_feat = [&](int l, int k) { return l == 0 ? k : perm[(l - 1) * HID + k]; };
+  for (int l = 0; l <= NHID; ++l) {
+    const size_t wo = (size_t)l * HID * HID, bo = (size_t)l * HID;
+    const int rows = l < NHID ? HID : n_out;
+    for (int o = 0; o < rows; ++o) {
+      const int src = l < NHID ? perm[l * HID + o] : o;
+      for (int k = 0; k < HID; ++k) W_out[wo + (size_t)o * HID + k] = W[wo + (size_t)src * HID + in_feat(l, k)];
+      b_out[bo + o] = b[bo + src];
+    }
+  }
+  return 0;
+}
+
+namespace {
+
+// The four weight images (fp16 / bf16 x CTA rank) of layers 2..5 of the network, W / b as dsmppi_permute_hidden
+// lays them out
+std::vector<uint8_t> image_bytes(const std::vector<float>& W, const std::vector<float>& b, int O) {
   std::vector<uint8_t> host((size_t)4 * IMG_BYTES, 0);
   for (int fmt = 0; fmt < 2; ++fmt)
     for (int rank = 0; rank < 2; ++rank) {
@@ -781,19 +904,49 @@ int tc_build_images(dsmppi_ctx* c, const dsmppi_net* net) {
           const int feat = 128 * h + 64 * rank + n;        // output feature held by this CTA in half h
           for (int l = 0; l < NHID; ++l)                   // network layers 2..4 (layer 1 comes from the tables)
             for (int k = 0; k < HID; ++k)
-              put(OFF_WH + (l * 2 + h) * SZ_WHH + canon(n, k, 64), net->W_host[l + 1][(size_t)feat * HID + k]);
+              put(OFF_WH + (l * 2 + h) * SZ_WHH + canon(n, k, 64), W[(size_t)l * HID * HID + (size_t)feat * HID + k]);
         }
       for (int n = 0; n < 16; ++n) {
         const int o = 16 * rank + n;                       // N = 32 over the pair: links 0..15 | 16..31 (padding)
         for (int k = 0; k < HID; ++k)
-          put(OFF_W5 + canon(n, k, 16), o < c->O ? net->W_host[4][(size_t)o * HID + k] : 0.f);
+          put(OFF_W5 + canon(n, k, 16), o < O ? W[(size_t)NHID * HID * HID + (size_t)o * HID + k] : 0.f);
       }
       float* bias = reinterpret_cast<float*>(img + OFF_BIAS);
-      for (int l = 0; l < NHID; ++l)
-        for (int k = 0; k < HID; ++k) bias[l * HID + k] = net->b_host[l + 1][k];
-      for (int o = 0; o < 16; ++o) bias[NHID * HID + o] = o < c->O ? net->b_host[4][o] : 0.f;
+      for (int k = 0; k < NHID * HID; ++k) bias[k] = b[k];
+      for (int o = 0; o < 16; ++o) bias[NHID * HID + o] = o < O ? b[NHID * HID + o] : 0.f;
     }
-  CUDA_TRY(cudaMemcpy(dev, host.data(), host.size(), cudaMemcpyHostToDevice));
+  return host;
+}
+
+}  // namespace
+
+int tc_build_images(dsmppi_ctx* c, const dsmppi_net* net) {
+  c->tc_blob = nullptr;
+  if (c->O > 16) return 0;                          // output N is fixed at 16 links; fall back to fp32
+  const char* dis = std::getenv("DSMPPI_DISABLE_TC");
+  if (dis && dis[0] == '1') return 0;
+  TcImages* t = new TcImages();
+  for (int l = 1; l <= 4; ++l) {
+    const int rows = l < 4 ? HID : c->O;
+    t->W.insert(t->W.end(), net->W_host[l], net->W_host[l] + (size_t)rows * HID);
+    t->b.insert(t->b.end(), net->b_host[l], net->b_host[l] + rows);
+  }
+  for (int l = 0; l < NHID; ++l)
+    for (int f = 0; f < HID; ++f) t->perm[l * HID + f] = f;
+  // two formats x two CTA ranks
+  uint8_t* dev = nullptr;
+  if (cudaMalloc(reinterpret_cast<void**>(&dev), (size_t)4 * IMG_BYTES) != cudaSuccess) {
+    dsmppi_set_error("cudaMalloc(tc images) failed");
+    delete t;
+    return 1;
+  }
+  const std::vector<uint8_t> host = image_bytes(t->W, t->b, c->O);
+  if (cudaMemcpy(dev, host.data(), host.size(), cudaMemcpyHostToDevice) != cudaSuccess) {
+    dsmppi_set_error("cudaMemcpy(tc images) failed");
+    cudaFree(dev);
+    delete t;
+    return 1;
+  }
   t->img[0] = dev;
   t->img[1] = nullptr;
   c->tc_blob = t;
@@ -816,6 +969,68 @@ void tc_free_images(dsmppi_ctx* c) {
   if (t->img[0]) cudaFree(t->img[0]);
   delete t;
   c->tc_blob = nullptr;
+}
+
+// Census of the dead-feature skip, over the n states q (row stride d) x every current obstacle: features of hidden
+// layers 2..4 that never had a positive pre-activation go last in the images' order, and whole K = 16 steps of them
+// are not issued by the GEMM that reads them (c->pass1_skip; at most 8 per GEMM, the D_hi half).  Each prefiltered row
+// proves its skip (the kernel's dead_or): a row in which a skipped feature was active makes the host repeat the call
+// without the skip and mark the census stale.  A census at the same obstacle count adds to the features seen active
+// before; one that finds nothing new after such a repeat turns the skip off until the next fresh census (the active
+// feature is then one the census rows do not reach).  *changed: the images' order changed.
+int tc_census(dsmppi_ctx* c, const float* q, int n, cudaStream_t st, bool* changed) {
+  TcImages* t = static_cast<TcImages*>(c->tc_blob);
+  *changed = false;
+  uint32_t* dev = nullptr;
+  uint32_t alive[NHID][HID / 32];
+  CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&dev), sizeof(alive)));
+  cudaError_t e = cudaMemsetAsync(dev, 0, sizeof(alive), st);
+  const long long rows = (long long)n * c->M;
+  if (e == cudaSuccess) {
+    census_kernel<<<(unsigned)((rows + CEN_R - 1) / CEN_R), HID, 0, st>>>(c->net, q, n, c->obs, c->M, dev);
+    c->launches++;
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaMemcpyAsync(alive, dev, sizeof(alive), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  cudaFree(dev);
+  CUDA_TRY(e);
+  const bool fresh = c->census_M != c->M;
+  bool woke = false;
+  for (int l = 0; l < NHID; ++l)
+    for (int w = 0; w < HID / 32; ++w) {
+      if (!fresh) {
+        woke = woke || (alive[l][w] & ~t->alive[l][w]) != 0;
+        alive[l][w] |= t->alive[l][w];
+      }
+      t->alive[l][w] = alive[l][w];
+    }
+  // active features first, each group in the network's order
+  int32_t perm[NHID * HID];
+  for (int l = 0; l < NHID; ++l) {
+    int p = 0;
+    for (int pass = 0; pass < 2; ++pass)
+      for (int f = 0; f < HID; ++f)
+        if (((alive[l][f >> 5] >> (f & 31)) & 1u) == (pass == 0 ? 1u : 0u)) perm[l * HID + p++] = f;
+  }
+  for (int l = 0; l < NHID; ++l) {
+    int n_alive = 0;
+    for (int w = 0; w < HID / 32; ++w) n_alive += __builtin_popcount(alive[l][w]);
+    const int s = (HID - n_alive) / 16;
+    c->pass1_skip[l] = (fresh || woke) ? (s < 8 ? s : 8) : 0;
+  }
+  c->census_M = c->M;
+  c->census_stale = 0;
+  if (std::memcmp(perm, t->perm, sizeof(perm)) != 0) {
+    std::vector<float> W(t->W.size()), b(t->b.size());
+    if (const int rc = dsmppi_permute_hidden(c->O, t->W.data(), t->b.data(), perm, W.data(), b.data())) return rc;
+    const std::vector<uint8_t> host = image_bytes(W, b, c->O);
+    CUDA_TRY(cudaMemcpyAsync(t->img[0], host.data(), host.size(), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    std::memcpy(t->perm, perm, sizeof(perm));
+    *changed = true;
+  }
+  return 0;
 }
 
 int tc_set_obstacles(dsmppi_ctx* c, cudaStream_t st) {
@@ -916,6 +1131,8 @@ int tc_pass1(dsmppi_ctx* c, const float* q, int q_stride, const float* obs, cons
   a.zero = 0u;
   a.use_writers = 1;
   a.nonfinite = c->counters + 9;
+  a.dead_fired = c->counters + 10;
+  for (int l = 0; l < NHID; ++l) a.skip[l] = c->pass1_noskip ? 0 : c->pass1_skip[l];
   a.prof = nullptr;
 #ifdef DSMPPI_TC_PROF
   a.prof = reinterpret_cast<long long*>(c->stage);   // the micro-benchmark parks its counter buffer here

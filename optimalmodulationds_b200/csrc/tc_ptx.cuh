@@ -240,10 +240,32 @@ __device__ __forceinline__ void mma_ts_2cta_imm(uint32_t tmem_base, uint32_t sb4
       "r"(sb4), "n"(D_COL), "n"(A_COL), "n"(DESC_IMM), "n"(DESC_HI), "n"(IDESC), "n"(ACC ? 1 : 0)
       : "memory");
 }
-template <uint32_t D_COL, uint32_t A_COL, uint32_t B_OFF, uint32_t LBO, uint32_t IDESC, int... KS>
-__device__ __forceinline__ void mma_group(uint32_t tmem_base, uint32_t sb4, std::integer_sequence<int, KS...>) {
-  (mma_ts_2cta_imm<D_COL, A_COL + KS * 8, (B_OFF >> 4) + ((LBO >> 4) << 16) + KS * ((2 * LBO) >> 4), IDESC,
-                   (KS > 0)>(tmem_base, sb4), ...);
+// The same MMA, issued only when KS < nk (one warp-uniform compare per K-step; nk is a kernel argument)
+template <uint32_t D_COL, uint32_t A_COL, uint32_t DESC_IMM, uint32_t IDESC, uint32_t KS>
+__device__ __forceinline__ void mma_ts_2cta_imm_if(uint32_t tmem_base, uint32_t sb4, uint32_t nk) {
+  asm volatile(
+      "{\n\t.reg .pred q;\n\t.reg .b64 bd;\n\t.reg .b32 dl, td, ta;\n\t"
+      "setp.lt.u32 q, %7, %8;\n\t"
+      "add.u32 td, %0, %2;\n\t"
+      "add.u32 ta, %0, %3;\n\t"
+      "add.u32 dl, %1, %4;\n\t"
+      "mov.b64 bd, {dl, %5};\n\t"
+      "@q tcgen05.mma.cta_group::2.kind::f16 [td], [ta], bd, %6, 1;\n\t}" ::"r"(tmem_base),
+      "r"(sb4), "n"(D_COL), "n"(A_COL), "n"(DESC_IMM), "n"(DESC_HI), "n"(IDESC), "n"(KS), "r"(nk)
+      : "memory");
+}
+// The K-steps KS of one accumulator group.  K-steps from FIXED on are issued only while KS < nk: the last 16 - nk
+// K-steps multiply input features that the calibration found never active (tc_pass1.cu, dead-feature skip).
+template <uint32_t D_COL, uint32_t A_COL, uint32_t B_OFF, uint32_t LBO, uint32_t IDESC, int FIXED, int... KS>
+__device__ __forceinline__ void mma_group(uint32_t tmem_base, uint32_t sb4, uint32_t nk,
+                                          std::integer_sequence<int, KS...>) {
+  auto one = [&](auto K) {
+    constexpr int k = decltype(K)::value;
+    constexpr uint32_t desc = (B_OFF >> 4) + ((LBO >> 4) << 16) + k * ((2 * LBO) >> 4);
+    if constexpr (k < FIXED) mma_ts_2cta_imm<D_COL, A_COL + k * 8, desc, IDESC, (k > 0)>(tmem_base, sb4);
+    else mma_ts_2cta_imm_if<D_COL, A_COL + k * 8, desc, IDESC, k>(tmem_base, sb4, nk);
+  };
+  (one(std::integral_constant<int, KS>{}), ...);
 }
 
 // kind::f16 instruction descriptor: fp16 (fmt 0) or bf16 (fmt 1) A and B (K-major), fp32 (or fp16) accumulate, dense
