@@ -693,25 +693,32 @@ tc_pass1_kernel(const __grid_constant__ TcArgs a) {
       // (one branch holds the whole life of the 128-register operand: split into two `if (more)` blocks around the
       // wait, the compiler kept it conditionally live through the hidden-layer epilogues and spilled 3 KB per thread)
       if (more) {
-        // (the output-layer MMA sits behind the other tile's layer in the issuer's order and completes late: draining
-        // it BEFORE the table loads are consumed -- to release D_lo sooner -- put that wait in front of the next
-        // tile's operand and cost 5 %)
+        // D_lo is released as soon as the output layer has completed, with the next tile's table loads in flight and
+        // before they are consumed: the other slot's next layer waits for D_lo (profiles/tc_pass1_schedule_ab.txt)
         uint32_t nxt[128];
         if constexpr (ASM) {
           TableLoads t;
           first_layer_issue(a, i_next, j_next, tile_dep, lane, t);
+          PROF_ADD(6);
+          mbar_wait(bar_full_lo, 1u);                               // fourth use of D_lo in this tile
+          tc_fence_after();
+          PROF_ADD(0);
+          tmem_ld16(tDlo, v);
+          tc_wait_ld();
+          signal(BAR(BAR_DFREE0));
           first_layer_finish<BF16>(a, i_next, t, abuf, lane, nxt);
+          store_operand(tA, nxt);               // the output-layer MMA has retired: A may be overwritten
         } else {
           first_layer<BF16>(a, i_next, j_next, tile_dep, nxt);
+          PROF_ADD(6);
+          mbar_wait(bar_full_lo, 1u);
+          tc_fence_after();
+          PROF_ADD(0);
+          tmem_ld16(tDlo, v);
+          store_operand(tA, nxt);
+          tc_wait_ld();
+          signal(BAR(BAR_DFREE0));
         }
-        PROF_ADD(6);
-        mbar_wait(bar_full_lo, 1u);                                 // fourth use of D_lo in this tile
-        tc_fence_after();
-        PROF_ADD(0);
-        tmem_ld16(tDlo, v);
-        store_operand(tA, nxt);                 // the output-layer MMA has retired: A may be overwritten
-        tc_wait_ld();
-        signal(BAR(BAR_DFREE0));
         tc_wait_st();
         signal(bar_aready);
         finish_tile(v);

@@ -6,6 +6,10 @@
 //      warps and of the MMA issuer on a Franka-shelf-sized problem.
 // Build:  nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo -DDSMPPI_TC_PROF \
 //              -I include -I optimalmodulationds_b200/csrc tools/tc_microbench.cu -o tools/tc_microbench
+// Run:    tc_microbench [n [M]]        all of the above, random-init net, random obstacles
+//         tc_microbench power           the bare MMA loop at full power (fp32 / fp16 accumulators)
+//         tc_microbench phase FILE [n]  only 4., on the net and obstacles of FILE (tools/tc_phase_inputs.py writes it),
+//                                       after the dead-feature census of the library (tc_census) on 128 of the states
 #include <cstdio>
 #include <random>
 #include <string>
@@ -180,9 +184,38 @@ void run_mb(const char* name, int mode, int iters, int nwarps, int per_wait, lon
 
 }  // namespace
 
+// FILE of `phase`: int32 M, then float32 W0 (256 x 30), b0, W1..W3 (256 x 256 each), b1..b3, W4 (9 x 256), b4 in
+// torch orientation, then the (M, 4) obstacles
+bool read_phase_inputs(const char* path, std::vector<float> (&W)[5], std::vector<float> (&b)[5], std::vector<float>& obs,
+                       int& M) {
+  FILE* f = fopen(path, "rb");
+  if (!f) return false;
+  const int in_dim[5] = {30, 256, 256, 256, 256}, out_dim[5] = {256, 256, 256, 256, 9};
+  bool ok = fread(&M, 4, 1, f) == 1 && M > 0;
+  for (int l = 0; ok && l < 5; ++l) {
+    W[l].resize((size_t)in_dim[l] * out_dim[l]);
+    b[l].resize(out_dim[l]);
+    ok = fread(W[l].data(), 4, W[l].size(), f) == W[l].size() && fread(b[l].data(), 4, b[l].size(), f) == b[l].size();
+  }
+  if (ok) {
+    obs.resize((size_t)M * 4);
+    ok = fread(obs.data(), 4, obs.size(), f) == obs.size();
+  }
+  fclose(f);
+  return ok;
+}
+
+float* upload(const std::vector<float>& h) {
+  float* d = nullptr;
+  cudaMalloc(&d, h.size() * 4);
+  cudaMemcpy(d, h.data(), h.size() * 4, cudaMemcpyHostToDevice);
+  return d;
+}
+
 int main(int argc, char** argv) {
-  const int n = argc > 1 ? atoi(argv[1]) : 4096;
-  const int M = argc > 2 ? atoi(argv[2]) : 2064;
+  const bool phase = argc > 2 && std::string(argv[1]) == "phase";
+  const int n = phase ? (argc > 3 ? atoi(argv[3]) : 4096) : argc > 1 ? atoi(argv[1]) : 4096;
+  int M = phase ? 0 : argc > 2 ? atoi(argv[2]) : 2064;
   cudaFuncSetAttribute(mb_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MB_SMEM);
   long long* dout;
   cudaMalloc(&dout, 2 * 148 * 9 * sizeof(long long));
@@ -193,12 +226,17 @@ int main(int argc, char** argv) {
     }
     return 0;
   }
-  for (int nw : {4, 8})
-    for (int pw : {1, 2, 4}) run_mb("tcgen05.ld 32x32b.x32", 0, 2000, nw, pw, dout, 0);
-  for (int nw : {4, 8}) run_mb("tcgen05.st 32x32b.x32", 1, 2000, nw, 4, dout, 0);
-  run_mb("tcgen05.mma cg2 ts M256 N128 K16 (2 halves)", 2, 200, 0, 0, dout, 0);
-  run_mb("tcgen05.mma cg2 ts M256 N256 K16", 3, 200, 0, 0, dout, 0);
-  run_mb("tcgen05.mma N128 + 4 warps draining D_hi", 4, 400, 0, 0, dout, 0);
+  std::vector<float> W[5], b[5], obs;
+  if (phase) {
+    if (!read_phase_inputs(argv[2], W, b, obs, M)) { fprintf(stderr, "cannot read %s\n", argv[2]); return 1; }
+  } else {
+    for (int nw : {4, 8})
+      for (int pw : {1, 2, 4}) run_mb("tcgen05.ld 32x32b.x32", 0, 2000, nw, pw, dout, 0);
+    for (int nw : {4, 8}) run_mb("tcgen05.st 32x32b.x32", 1, 2000, nw, 4, dout, 0);
+    run_mb("tcgen05.mma cg2 ts M256 N128 K16 (2 halves)", 2, 200, 0, 0, dout, 0);
+    run_mb("tcgen05.mma cg2 ts M256 N256 K16", 3, 200, 0, 0, dout, 0);
+    run_mb("tcgen05.mma N128 + 4 warps draining D_hi", 4, 400, 0, 0, dout, 0);
+  }
 
   // ---- the production kernel with phase accounting
   dsmppi_ctx c;
@@ -208,34 +246,38 @@ int main(int argc, char** argv) {
   c.sm_count = prop.multiProcessorCount;
   std::mt19937 rng(0);
   std::normal_distribution<float> nd(0.f, 1.f);
-  std::vector<float> W[5], b[5];
   const int in_dim[5] = {30, 256, 256, 256, 256}, out_dim[5] = {256, 256, 256, 256, 9};
   dsmppi_net net;
   net.n_dof = 7; net.n_out = 9;
   for (int l = 0; l < 5; ++l) {
-    W[l].resize((size_t)in_dim[l] * out_dim[l]);
-    b[l].resize(out_dim[l]);
-    for (auto& x : W[l]) x = nd(rng) / sqrtf((float)in_dim[l]);
-    for (auto& x : b[l]) x = 0.1f * nd(rng);
+    if (!phase) {
+      W[l].resize((size_t)in_dim[l] * out_dim[l]);
+      b[l].resize(out_dim[l]);
+      for (auto& x : W[l]) x = nd(rng) / sqrtf((float)in_dim[l]);
+      for (auto& x : b[l]) x = 0.1f * nd(rng);
+    }
     net.W_host[l] = W[l].data();
     net.b_host[l] = b[l].data();
   }
   if (tc_build_images(&c, &net)) return 1;
-  // the layer-1 tables are computed from the fp32 weights (W1^T, [3 nin][256]) and the layer-1 bias on the device
-  {
-    std::vector<float> wf0((size_t)30 * 256);
+  // the layer-1 tables are computed from the fp32 weights (W1^T, [3 nin][256]) and the layer-1 bias on the device;
+  // the census reads layers 2..4 the same way (forward orientation [in][256])
+  for (int l = 0; l < 4; ++l) {
+    std::vector<float> wf((size_t)in_dim[l] * 256);
     for (int o = 0; o < 256; ++o)
-      for (int k = 0; k < 30; ++k) wf0[(size_t)k * 256 + o] = W[0][(size_t)o * 30 + k];
-    float *dwf = nullptr, *db0 = nullptr;
-    cudaMalloc(&dwf, wf0.size() * 4);
-    cudaMemcpy(dwf, wf0.data(), wf0.size() * 4, cudaMemcpyHostToDevice);
-    cudaMalloc(&db0, 256 * 4);
-    cudaMemcpy(db0, b[0].data(), 256 * 4, cudaMemcpyHostToDevice);
-    c.net.Wf[0] = dwf; c.net.b[0] = db0; c.P = 3;
+      for (int k = 0; k < in_dim[l]; ++k) wf[(size_t)k * 256 + o] = W[l][(size_t)o * in_dim[l] + k];
+    c.net.Wf[l] = upload(wf);
+    c.net.b[l] = upload(b[l]);
   }
-  std::vector<float> obs((size_t)M * 4), q((size_t)n * 7);
-  for (auto& x : obs) x = 0.5f * nd(rng);
-  for (auto& x : q) x = nd(rng);
+  c.net.d = 7; c.net.nin = 10; c.net.nenc = 30; c.net.O = 9; c.P = 3;
+  std::vector<float> q((size_t)n * 7);
+  if (!phase) {
+    obs.resize((size_t)M * 4);
+    for (auto& x : obs) x = 0.5f * nd(rng);
+  }
+  // joint vectors uniform in [-pi, pi]^7 (tools/dead_feature_study.py: the census features stay dead on them)
+  std::uniform_real_distribution<float> ud(-3.14159265f, 3.14159265f);
+  for (auto& x : q) x = phase ? ud(rng) : nd(rng);
   cudaMalloc(&c.obs, obs.size() * 4);
   cudaMemcpy(c.obs, obs.data(), obs.size() * 4, cudaMemcpyHostToDevice);
   float* dq;
@@ -244,6 +286,12 @@ int main(int argc, char** argv) {
   cudaMalloc(&c.mdist, (size_t)n * M * 4);
   cudaMalloc(reinterpret_cast<void**>(&c.counters), N_COUNTERS * sizeof(int));   // (the kernel counts non-finite outputs)
   cudaMemset(c.counters, 0, N_COUNTERS * sizeof(int));
+  if (phase) {
+    bool reordered = false;
+    if (tc_census(&c, dq, n < 128 ? n : 128, 0, &reordered)) return 1;
+    printf("census: %d / %d / %d K-steps skipped in the layer 3 / layer 4 / output GEMMs\n", c.pass1_skip[0],
+           c.pass1_skip[1], c.pass1_skip[2]);
+  }
   const size_t prof_n = (size_t)c.sm_count * 9 * 8;
   cudaMalloc(reinterpret_cast<void**>(&c.stage), prof_n * sizeof(long long));
   cudaMemset(c.stage, 0, prof_n * sizeof(long long));
@@ -260,6 +308,9 @@ int main(int argc, char** argv) {
     const double fl = (double)n * M * 2.0 * (30 * 256 + 3 * 256 * 256 + 256 * 9);
     printf("tc_pass1 (PROF build) n=%d M=%d: %.3f ms  %.1f TFLOP/s algorithmic\n", n, M, ms, fl / ms * 1e-9);
   }
+  int counters[N_COUNTERS];
+  cudaMemcpy(counters, c.counters, sizeof(counters), cudaMemcpyDeviceToHost);
+  printf("rows with a skipped feature active: %d, non-finite rows: %d\n", counters[10], counters[9]);
   std::vector<long long> prof(prof_n);
   cudaMemcpy(prof.data(), c.stage, prof_n * sizeof(long long), cudaMemcpyDeviceToHost);
   const char* row_names[8] = {"wait D_lo full", "drain D_lo (ld+pack 64)", "pack lo 64..127", "wait D_hi full",
